@@ -7,7 +7,10 @@ A "step" is ONE query round over one synthetic pool (SURVEY.md 8d): gather 25x25
 |P(class1)-0.5| -> top-k (the 'entropy' answer, k=100) AND uncertainty pre-filter to B=10,000 -> factored FI of the
 last two FC layers -> greedy selection of k=100 (the 'fi' answer) -> both index sets on the host.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
+
+`--dump-outputs DIR` also writes what the timed path computed in its last step as DIR/<name>.npy (float32 / float64;
+indices as float64): the inputs are seeded, so two builds can be compared array by array.
 
 Prints ONE JSON line (rank 0).  `value` = whole-job samples/s with volumes, weights and pool indices resident in
 HBM; `e2e` = the same round through the reference-facing API (nnal_b200.PW_NNAL.CNN_query(..., 'entropy+fi') with
@@ -123,6 +126,41 @@ def make_model():
     return model
 
 
+DUMP_MAX_BYTES = 64 * 10 ** 6      # all files of one --dump-outputs together
+NPY_HEADER_BYTES = 1024            # allowance per file for the .npy header (128 bytes for these shapes)
+
+
+def _dump_float(a):
+    a = np.asarray(a)
+    return a if a.dtype == np.float32 else a.astype(np.float64)
+
+
+def dump_outputs(out_dir, arrays, posteriors=None, posteriors_name='pool_posteriors', lo=0):
+    """Writes each array as out_dir/<name>.npy: float32 stays float32, everything else (indices included) becomes float64.
+    ``posteriors`` [..., n] (one column per pool sample, global positions lo..lo+n-1) is written as ``posteriors_name``
+    next to ``pool_positions``: all n columns, or a fixed seeded sample of as many as the byte budget leaves after the
+    other arrays and the file headers (each sampled column costs its posterior rows plus one float64 position)."""
+    conv = {name: _dump_float(a) for name, a in arrays.items()}
+    if posteriors is not None:
+        post = _dump_float(posteriors)
+        n = post.shape[-1]
+        per_col = 8 + post.dtype.itemsize * int(np.prod(post.shape[:-1]))
+        left = DUMP_MAX_BYTES - sum(a.nbytes for a in conv.values()) - NPY_HEADER_BYTES * (len(conv) + 2)
+        m = max(0, min(n, left // per_col))
+        cols = np.arange(n) if m == n else np.sort(np.random.RandomState(0).choice(n, m, replace=False))
+        conv['pool_positions'] = (cols + lo).astype(np.float64)
+        conv[posteriors_name] = np.ascontiguousarray(post[..., cols])
+    if sum(a.nbytes for a in conv.values()) + NPY_HEADER_BYTES * len(conv) > DUMP_MAX_BYTES:
+        raise ValueError('outputs do not fit the %d-byte dump budget' % DUMP_MAX_BYTES)
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, a in conv.items():
+        path = os.path.join(out_dir, name + '.npy')
+        np.save(path, a)
+        total += os.path.getsize(path)
+    sys.stderr.write('bench.py: wrote %d arrays (%d bytes) to %s\n' % (len(conv), total, out_dir))
+
+
 def digest(*arrays):
     h = hashlib.sha1()
     for a in arrays:
@@ -222,7 +260,8 @@ def cpu_reference_round(sample, fi_B, threads=None):
     D = O.last_layers_dim(2, U.shape[0], A.shape[0])
     S, _ = O.greedy_fi_rank1(Kt, D, FI_DELTA, min(K_QUERY, fi_B))
     t2 = time.perf_counter()
-    return t2 - t0, sample, threads, {'entropy_half_s': t1 - t0, 'fi_half_s': t2 - t1, 'q_ent': q_ent, 'q_fi': sel[S]}
+    return t2 - t0, sample, threads, {'entropy_half_s': t1 - t0, 'fi_half_s': t2 - t1, 'q_ent': q_ent, 'q_fi': sel[S],
+                                      'posts': posts}
 
 
 def _cpu_desc(sample, fi_B, pool):
@@ -239,9 +278,12 @@ def run_reference(args, rank, world):
     times = []
     threads = os.cpu_count()
     for i in range(args.warmup + args.steps):
-        dt, n, threads, _ = cpu_reference_round(sample, fi_B)
+        dt, n, threads, det = cpu_reference_round(sample, fi_B)
         if i >= args.warmup:
             times.append(dt)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {'entropy_query': det['q_ent'], 'fi_query': det['q_fi']}, det['posts'],
+                     'pool_posteriors_class1')
     total = sum(times)
     value = sample * len(times) / total
     line = {'impl': 'reference', 'metric': METRIC, 'value': value, 'unit': UNIT, 'n_gpus': args.gpus,
@@ -314,7 +356,7 @@ def run_ours(args, rank, world):
         chosen, obj, red = fimod.greedy_select(eng, min(k, len(sel)), FI_DELTA, np.nonzero(own)[0].astype(np.int64))
         if mark:
             mark(3)
-        return q_ent, sel[chosen], red
+        return q_ent, sel[chosen], red, obj
 
     # The interpreter's cyclic collector walks every tracked object of the process (torch, NumPy, this harness: millions) whenever
     # a generation-2 collection triggers -- 20-80 ms pauses at random steps of the host-timed e2e leg.  Objects alive now are
@@ -373,6 +415,11 @@ def run_ours(args, rank, world):
         t, c = eng.profile_read(cid)
         classes[name] = {'ms': t, 'launches': c, 'macs_per_sample': 0, 'tc': 0, 'type': -1}
     eng.profile(False)
+    if args.dump_outputs and rank == 0:
+        # the last timed step's answers and its pool posteriors (still in the pool buffers: the e2e leg below reuses them);
+        # with several ranks, the posteriors are rank 0's shard
+        dump_outputs(args.dump_outputs, {'entropy_query': q_res[0], 'fi_query': q_res[1], 'fi_reduced_objective': q_res[2],
+                                         'fi_objective': q_res[3]}, eng.pool_posteriors(), 'pool_posteriors', lo)
     if world > 1:
         tms = torch.tensor([dev_ms] + list(stage_acc), dtype=torch.float64, device='cuda')
         torch.distributed.all_reduce(tms, op=torch.distributed.ReduceOp.MAX)
@@ -854,7 +901,10 @@ def main():
     ap.add_argument('--mc-T', type=int, default=10, help='MC-dropout passes of the extra MC-entropy round (0: skip)')
     ap.add_argument('--config4-slices', type=int, default=180, help='slices of the config-4 full-volume gather at 1 GPU (0: skip)')
     ap.add_argument('--strong-pool', type=int, default=1000000, help='fixed pool of the config-3 strong-scaling leg (0: skip)')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the last timed step\'s outputs as DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
     rank = int(os.environ.get('RANK', '0'))
     world = int(os.environ.get('WORLD_SIZE', '1'))
     if args.impl == 'reference':

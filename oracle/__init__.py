@@ -7,8 +7,8 @@ reference`` legs may import it, and there only as the checker / CPU baseline.
 
 Parity status
 -------------
-``oracle/check_against_reference.py`` (run in the dev container, where
-/root/reference exists) imports the UNMODIFIED reference in place, missing
+``oracle/check_against_reference.py`` (run with $NNAL_REFERENCE set to the
+original sources) imports the UNMODIFIED reference in place, missing
 third-party modules stubbed, compares on seeded inputs and writes the golden
 vectors in ``tests/golden/``:
 

@@ -1,12 +1,12 @@
 """Pin the oracle against the reference's own pure-NumPy functions and write the
-golden vectors in tests/golden/ (run in the dev container only).
+golden vectors in tests/golden/.
 
-The reference (read-only at /root/reference) is imported IN PLACE under
-``sys.modules`` stubs for its missing third-party imports (SURVEY.md §4); only its
-NumPy-only helpers are executed, unchanged.  This script is the generator of every
-file in tests/golden/; the GPU box never needs /root/reference.
+The reference (the original nn-active-learning sources, read-only, at $NNAL_REFERENCE) is
+imported IN PLACE under ``sys.modules`` stubs for its missing third-party imports
+(SURVEY.md §4); only its NumPy-only helpers are executed, unchanged.  This script is the
+generator of every file in tests/golden/; the tests need only those files.
 
-    python oracle/check_against_reference.py            # check + (re)write goldens
+    NNAL_REFERENCE=<tree> python oracle/check_against_reference.py     # check + (re)write goldens
 """
 import os
 import sys
@@ -15,13 +15,15 @@ from unittest.mock import MagicMock
 
 import numpy as np
 
-REF = os.environ.get('NNAL_REFERENCE', '/root/reference')
+REF = os.environ.get('NNAL_REFERENCE')
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 GOLD = os.environ.get('NNAL_GOLD_OUT', os.path.join(ROOT, 'tests', 'golden'))   # NNAL_GOLD_OUT: check only, write elsewhere
 
 
 def import_reference():
+    if not REF or not os.path.isdir(REF):
+        sys.exit('set NNAL_REFERENCE to the directory of the original nn-active-learning sources')
     for m in ['tensorflow', 'tensorflow.examples', 'tensorflow.examples.tutorials',
               'tensorflow.examples.tutorials.mnist', 'tensorflow.python',
               'tensorflow.python.ops', 'tensorflow.python.framework', 'nrrd', 'cvxopt',
