@@ -248,6 +248,18 @@ int nnal_fi_step_pack(nnal_ctx* ctx, int64_t step, void* d_msg);
 int nnal_fi_step_apply_gathered(nnal_ctx* ctx, int64_t step, const void* d_msgs, int world, int rank);
 int nnal_fi_result(nnal_ctx* ctx, int64_t k, int64_t* gids_out, double* red_out);
 
+/* Greedy FI selection for multi-class models (2 <= c <= 32), last FC layer only, in block form (csrc/fi_block.cu):
+ * F_i = A(pi_i) (x) [u_i;1][u_i;1]^T with A(pi) = diag pi - pi pi^T = L_i L_i^T (closed-form c x (c-1) factor of the
+ * float64-renormalised posteriors), block kernel K_ij = (L_i^T L_j)(u_i.u_j + 1), D = c(d+1), r = c-1.  Same objective
+ * f(S) = tr((sum_{i in S} F_i/|S| + delta I)^-1) = (D - |S| r)/delta + red(S), red(S) = tr((delta I + K_SS/|S|)^-1), and
+ * the same conventions as nnal_fi_set_candidates / nnal_fi_set_factors / nnal_fi_greedy (ties: lowest candidate index;
+ * fewer than k candidates: only n_cand entries written).  k (c-1) <= 4096.
+ * Candidates from the current pool pass (keep >= 1; NULL = every pool sample), or from host factors:
+ * post[c][n] posteriors, U[n][d] feature-layer activations (input of the last FC). */
+int nnal_fi_block_set_candidates(nnal_ctx* ctx, const int64_t* cand, int64_t n_cand);
+int nnal_fi_block_set_factors(nnal_ctx* ctx, int64_t n, int c, int d, const float* post, const float* U);
+int nnal_fi_block_greedy(nnal_ctx* ctx, int64_t k, double delta, int64_t* sel_out, double* obj_out, double* red_out);
+
 /* All-gather of the per-step messages over NVLink peer memory instead of NCCL (csrc/p2p.cu): 100 dependent steps of one small
  * message each are latency bound, and one kernel that stores into the peers' buffers and spins on their flags costs a third of
  * an NCCL call.  The reference has no distributed code; the contract is SURVEY.md 8e, collective 3.

@@ -94,7 +94,10 @@ SIGNATURES = {
     'nnal_fi_step_pack': (C.c_int, [c_vp, C.c_int64, c_vp]),
     'nnal_fi_step_apply_gathered': (C.c_int, [c_vp, C.c_int64, c_vp, C.c_int, C.c_int]),
     'nnal_fi_result': (C.c_int, [c_vp, C.c_int64, c_vp, c_vp]),
-    'nnal_p2p_alloc': (C.c_int, [c_vp, C.c_int, C.c_int, C.c_int64, c_vp]),
+    'nnal_fi_block_set_candidates': (C.c_int, [c_vp, c_vp, C.c_int64]),
+    'nnal_fi_block_set_factors': (C.c_int, [c_vp, C.c_int64, C.c_int, C.c_int, c_vp, c_vp]),
+    'nnal_fi_block_greedy': (C.c_int, [c_vp, C.c_int64, C.c_double, c_vp, c_vp, c_vp]),
+    'nnal_p2p_alloc':(C.c_int, [c_vp, C.c_int, C.c_int, C.c_int64, c_vp]),
     'nnal_p2p_open': (C.c_int, [c_vp, c_vp]),
     'nnal_p2p_allgather': (C.c_int, [c_vp, c_vp, C.c_int64, C.c_uint64, c_vp]),
     'nnal_p2p_base': (C.c_int, [c_vp, c_vp]),

@@ -6,7 +6,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 OUT = os.path.join(HERE, 'libnnal_b200.so')
-SOURCES = ['capi.cu', 'volume.cu', 'forward.cu', 'forward_simt.cu', 'score.cu', 'gemm_tc.cu', 'conv_tc.cu', 'conv_wt.cu', 'fi.cu', 'sims.cu', 'shrunk.cu', 'sdp.cu', 'influence.cu', 'p2p.cu']
+SOURCES = ['capi.cu', 'volume.cu', 'forward.cu', 'forward_simt.cu', 'score.cu', 'gemm_tc.cu', 'conv_tc.cu', 'conv_wt.cu', 'fi.cu', 'fi_block.cu', 'sims.cu', 'shrunk.cu', 'sdp.cu', 'influence.cu', 'p2p.cu']
 NVCC = os.environ.get('NVCC', '/usr/local/cuda/bin/nvcc')
 FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-O3', '-lineinfo', '-std=c++17',
          '-Xcompiler', '-fPIC', '-Xcompiler', '-pthread']

@@ -184,6 +184,7 @@ extern "C" int nnal_volume_clear(nnal_ctx* ctx) {
 }
 
 int nnal_fi_release(nnal_ctx* ctx);
+int nnal_fi_block_release(nnal_ctx* ctx);
 int nnal_sims_release(nnal_ctx* ctx);
 
 extern "C" int nnal_ctx_destroy(nnal_ctx* ctx) {
@@ -194,6 +195,7 @@ extern "C" int nnal_ctx_destroy(nnal_ctx* ctx) {
   free_layers(ctx);
   free_pool(ctx);
   nnal_fi_release(ctx);
+  nnal_fi_block_release(ctx);
   nnal_sims_release(ctx);
   nnal_bw_release(ctx);
   nnal_sdp_release(ctx);

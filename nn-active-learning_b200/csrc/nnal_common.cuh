@@ -194,6 +194,7 @@ struct nnal_ctx {
   void* tc_state = nullptr;              // tensor-map cache etc. (gemm_tc.cu)
   void* sims_state = nullptr;            // representativeness queries (sims.cu)
   void* fi_state = nullptr;              // Fisher-information candidate set / greedy state (fi.cu)
+  void* fi_block_state = nullptr;        // multi-class block-form FI candidates / greedy state (fi_block.cu)
   unsigned long long weights_version = 0; // bumped by nnal_model_set / nnal_model_set_weights: derived weight copies (shrunk.cu) are rebuilt
   void* bw_state = nullptr;              // shrunk class-score gradients: kept activations and gradient buffers (shrunk.cu)
   void* sdp_state = nullptr;             // query-distribution solver workspaces (sdp.cu)
@@ -255,6 +256,9 @@ static inline void prof_end(nnal_ctx* ctx) {
 #define NNAL_PROF_FI_GRAM 111
 #define NNAL_PROF_FI_GREEDY 112
 #define NNAL_PROF_FI_SOLVE 113
+#define NNAL_PROF_FIB_SYSTEM 114         // fi_block.cu: K_SS row, alpha I + K_SS, inversion, Z, tr C
+#define NNAL_PROF_FIB_EVAL 115           // fi_block.cu: per-candidate losses + arg-min
+#define NNAL_PROF_FIB_COLUMN 116         // fi_block.cu: the winner's column s_{., w}
 #define NNAL_PROF_BW_FORWARD 120
 #define NNAL_PROF_BW_BACKWARD 121
 

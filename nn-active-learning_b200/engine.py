@@ -509,6 +509,43 @@ class Engine(object):
         self._chk(self.lib.nnal_fi_greedy(self.h, k, float(delta), _ptr(sel), _ptr(obj), _ptr(red)))
         return sel, obj, red
 
+    def fi_block_set_candidates(self, cand=None):
+        """Multi-class block-form FI (last FC layer): candidates = pool positions ``cand`` (None: every pool sample) of
+        the current pool pass, which must have kept the feature layer."""
+        if cand is None:
+            self._chk(self.lib.nnal_fi_block_set_candidates(self.h, None, 0))
+            self._fi_block_n = self._pool_n
+        else:
+            cand = np.ascontiguousarray(cand, dtype=np.int64).ravel()
+            self.h2d_bytes += cand.nbytes
+            self._chk(self.lib.nnal_fi_block_set_candidates(self.h, _ptr(cand) if cand.size else None, cand.size))
+            self._fi_block_n = cand.size
+
+    def fi_block_set_factors(self, post, U):
+        """Multi-class block-form FI candidates from host factors: ``post`` [c,n] posteriors, ``U`` [n,d] features."""
+        post = np.ascontiguousarray(post, dtype=np.float32)
+        U = np.ascontiguousarray(U, dtype=np.float32)
+        if post.ndim != 2 or U.ndim != 2 or post.shape[1] != U.shape[0]:
+            raise ValueError('post must be [c,n] and U [n,d] for the same n')
+        c, n = post.shape
+        self.h2d_bytes += post.nbytes + U.nbytes
+        self._chk(self.lib.nnal_fi_block_set_factors(self.h, n, c, U.shape[1], _ptr(post), _ptr(U)))
+        self._fi_block_n = n
+
+    def fi_block_greedy(self, k, delta):
+        """Block-form greedy FI selection.  Returns (candidate indices in selection order, objective per step, reduced
+        objective ``tr((delta I + K_SS/s)^-1)`` per step)."""
+        k = int(k)
+        n = getattr(self, '_fi_block_n', None)
+        if n is not None:
+            k = min(k, n)
+        sel = np.empty(max(k, 1), dtype=np.int64)
+        obj = np.empty(max(k, 1), dtype=np.float64)
+        red = np.empty(max(k, 1), dtype=np.float64)
+        self.d2h_bytes += 16 * k
+        self._chk(self.lib.nnal_fi_block_greedy(self.h, k, float(delta), _ptr(sel), _ptr(obj), _ptr(red)))
+        return sel[:k], obj[:k], red[:k]
+
     # ------------------------------------------------------------------
     # the reference's shrunk FI coordinates + SDP query distribution
     # ------------------------------------------------------------------

@@ -590,3 +590,47 @@ def query_whole(model, expr, pool_inds, session):
     gids = np.nonzero(own)[0].astype(np.int64)
     chosen, _, _ = greedy_select(eng, min(k, len(sel_inds)), delta, gids)
     return sel_inds[chosen]
+
+
+def query_whole_block(model, expr, pool_inds, session, return_objective=False):
+    """``NNAL.CNN_query(..., 'fi')`` with ``expr.pars['fi_mode'] = 'block-greedy'``: greedy minimisation of the last-layer
+    FI objective ``tr((sum_{i in S} F_i/|S| + delta I)^-1)`` for any number of classes c >= 2 (c <= 32, k (c-1) <= 4096),
+    ``F_i = (diag pi_i - pi_i pi_i^T) (x) [u_i;1][u_i;1]^T`` (NN.LLFC_hess, NN.py:891-901), in the block form of
+    csrc/fi_block.cu.  Entropy pre-filter to B exactly as ``query_whole``, then the greedy over ``min(k, B)`` steps.
+    Keys read: ``k``, ``B``, ``fi_diag_load`` (default 1e-5); ``fi_layers`` is ignored (last FC layer only, as in
+    ``query_whole``).  Returns positions into ``pool_inds`` in selection order (and, with ``return_objective``, the
+    objective and its kernel-dependent part per step).
+
+    Several ranks: every rank reads its own candidates' posteriors and feature rows, the B candidates are all-gathered and
+    put in pre-filter order on every rank, and every rank runs the same deterministic greedy on them."""
+    from .NNAL import _posteriors_on_device
+    k, B = int(expr.pars['k']), int(expr.pars['B'])
+    delta = float(expr.pars.get('fi_diag_load', 1e-5))
+    pool_inds = np.asarray(pool_inds)
+    n = len(pool_inds)
+    eng, lo, hi = _posteriors_on_device(model, expr, pool_inds, session, keep=1)
+    if B < n:
+        eng.pool_score(L.SCORE_NEG_ENTROPY, 1e-8)
+        sel_inds, _ = dist.topk_global(eng, B, lo, n)
+    else:
+        sel_inds = np.arange(n, dtype=np.int64)
+    if not dist.is_dist():
+        eng.fi_block_set_candidates(sel_inds - lo)
+    else:
+        own = (sel_inds >= lo) & (sel_inds < hi)
+        rows = sel_inds[own] - lo
+        c = eng.n_class
+        post = eng.pool_posteriors()[:, rows] if len(rows) else np.zeros((c, 0), dtype=np.float32)
+        F = eng.pool_feature_rows(rows)
+        d = F.shape[1]
+        gpos = dist.allgather_concat(sel_inds[own].astype(np.int64))
+        P = dist.allgather_concat(np.ascontiguousarray(post.T, dtype=np.float32).ravel()).reshape(-1, c)
+        Fg = dist.allgather_concat(np.ascontiguousarray(F, dtype=np.float32).ravel()).reshape(-1, d)
+        order = np.argsort(gpos, kind='stable')
+        perm = order[np.searchsorted(gpos[order], sel_inds)]          # gathered row of every candidate, pre-filter order
+        eng.fi_block_set_factors(P[perm].T, Fg[perm])
+    chosen, obj, red = eng.fi_block_greedy(min(k, len(sel_inds)), delta)
+    q = sel_inds[chosen]
+    if return_objective == 'reduced':
+        return q, obj, red
+    return (q, obj) if return_objective else q
