@@ -298,6 +298,9 @@ extern "C" int nnal_model_set(nnal_ctx* ctx, const nnal_layer_spec* specs, int n
       L.kh = L.kw = specs[i].kh;
       L.in_h = H; L.in_w = W; L.in_c = C;
       L.out_h = (H + L.kh - 1) / L.kh; L.out_w = (W + L.kw - 1) / L.kw; L.out_c = C;
+      // tf.nn.max_pool SAME: the pad_total = out*s - in missing cells are split, the smaller half BEFORE the first
+      // row / column (nonzero only when s >= 3 leaves two or more cells over)
+      L.pad_t = (L.out_h * L.kh - H) / 2; L.pad_l = (L.out_w * L.kw - W) / 2;
       H = L.out_h; W = L.out_w;
     } else if (L.type == NNAL_LAYER_FC) {
       if (specs[i].out <= 0) NNAL_FAIL(ctx, NNAL_ERR_INVALID, "fc layer needs out > 0");

@@ -120,10 +120,11 @@ int nnal_k_conv_simt_split(nnal_ctx* ctx, const Layer& L, const float* in, nnal_
 }
 
 // ------------------------------------------------------------------------------------------
-// max-pool SAME, window == stride (NN.py:1473-1477): output ceil(n/s), padding after, never wins
+// max-pool SAME, window == stride (NN.py:1473-1477): output ceil(n/s); window (yo, xo) starts at (yo*s - pt, xo*s - pl)
+// with TF's padding before (pt, pl; 0 for s = 2), and padded cells never win
 // ------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) pool_kernel(const float* __restrict__ in, float* __restrict__ out, int64_t total,
-                                                    int H, int Wd, int C, int Ho, int Wo, int s) {
+                                                    int H, int Wd, int C, int Ho, int Wo, int s, int pt, int pl) {
   for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
     int c = e % C;
     int64_t t = e / C;
@@ -131,12 +132,10 @@ __global__ void __launch_bounds__(256) pool_kernel(const float* __restrict__ in,
     int yo = t % Ho;
     int64_t smp = t / Ho;
     float m = -INFINITY;
-    for (int dy = 0; dy < s; ++dy) {
-      int y = yo * s + dy;
-      if (y >= H) break;
-      for (int dx = 0; dx < s; ++dx) {
-        int x = xo * s + dx;
-        if (x >= Wd) break;
+    const int y0 = yo * s - pt, x0 = xo * s - pl;
+    const int y1 = min(y0 + s, H), x1 = min(x0 + s, Wd);
+    for (int y = max(y0, 0); y < y1; ++y) {
+      for (int x = max(x0, 0); x < x1; ++x) {
         m = fmaxf(m, in[((smp * H + y) * Wd + x) * (int64_t)C + c]);
       }
     }
@@ -157,7 +156,8 @@ __device__ __forceinline__ void pool8_update(const uint4& h, const uint4& l, flo
 }
 __global__ void __launch_bounds__(256) pool_split_kernel(const nnal_h* __restrict__ in_hi, const nnal_h* __restrict__ in_lo,
                                                           nnal_h* __restrict__ out_hi, nnal_h* __restrict__ out_lo,
-                                                          int64_t total8, int H, int Wd, int C, int Ho, int Wo, int s) {
+                                                          int64_t total8, int H, int Wd, int C, int Ho, int Wo, int s,
+                                                          int pt, int pl) {
   const int C8 = C / 8;
   for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total8; e += (int64_t)gridDim.x * blockDim.x) {
     int c8 = e % C8;
@@ -169,12 +169,10 @@ __global__ void __launch_bounds__(256) pool_split_kernel(const nnal_h* __restric
     uint32_t bh[8], bl[8];
 #pragma unroll
     for (int k = 0; k < 8; ++k) { m[k] = -INFINITY; bh[k] = 0; bl[k] = 0; }
-    for (int dy = 0; dy < s; ++dy) {
-      int y = yo * s + dy;
-      if (y >= H) break;
-      for (int dx = 0; dx < s; ++dx) {
-        int x = xo * s + dx;
-        if (x >= Wd) break;
+    const int y0 = yo * s - pt, x0 = xo * s - pl;
+    const int y1 = min(y0 + s, H), x1 = min(x0 + s, Wd);
+    for (int y = max(y0, 0); y < y1; ++y) {
+      for (int x = max(x0, 0); x < x1; ++x) {
         int64_t idx = ((smp * H + y) * Wd + x) * (int64_t)C + c8 * 8;
         uint4 h = *reinterpret_cast<const uint4*>(in_hi + idx);
         uint4 l = *reinterpret_cast<const uint4*>(in_lo + idx);
@@ -190,7 +188,8 @@ __global__ void __launch_bounds__(256) pool_split_kernel(const nnal_h* __restric
 // scalar variant for channel counts that are not a multiple of 8
 __global__ void __launch_bounds__(256) pool_split_scalar_kernel(const nnal_h* __restrict__ in_hi, const nnal_h* __restrict__ in_lo,
                                                                  nnal_h* __restrict__ out_hi, nnal_h* __restrict__ out_lo,
-                                                                 int64_t total, int H, int Wd, int C, int Ho, int Wo, int s) {
+                                                                 int64_t total, int H, int Wd, int C, int Ho, int Wo, int s,
+                                                                 int pt, int pl) {
   for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
     int c = e % C;
     int64_t t = e / C;
@@ -199,12 +198,10 @@ __global__ void __launch_bounds__(256) pool_split_scalar_kernel(const nnal_h* __
     int64_t smp = t / Ho;
     float m = -INFINITY;
     nnal_h bh = __float2half_rn(0.f), bl = bh;
-    for (int dy = 0; dy < s; ++dy) {
-      int y = yo * s + dy;
-      if (y >= H) break;
-      for (int dx = 0; dx < s; ++dx) {
-        int x = xo * s + dx;
-        if (x >= Wd) break;
+    const int y0 = yo * s - pt, x0 = xo * s - pl;
+    const int y1 = min(y0 + s, H), x1 = min(x0 + s, Wd);
+    for (int y = max(y0, 0); y < y1; ++y) {
+      for (int x = max(x0, 0); x < x1; ++x) {
         int64_t idx = ((smp * H + y) * Wd + x) * (int64_t)C + c;
         nnal_h h = in_hi[idx], l = in_lo[idx];
         float v = nnal_merge(h, l);
@@ -223,10 +220,12 @@ int nnal_k_pool_split(nnal_ctx* ctx, const Layer& L, const nnal_h* in_hi, const 
   if (L.out_c % 8 == 0) {
     int64_t total8 = total / 8;
     int grid = (int)((total8 + 255) / 256 < (int64_t)ctx->sm_count * 32 ? (total8 + 255) / 256 : (int64_t)ctx->sm_count * 32);
-    pool_split_kernel<<<grid, 256, 0, ctx->stream>>>(in_hi, in_lo, out_hi, out_lo, total8, L.in_h, L.in_w, L.in_c, L.out_h, L.out_w, L.kh);
+    pool_split_kernel<<<grid, 256, 0, ctx->stream>>>(in_hi, in_lo, out_hi, out_lo, total8, L.in_h, L.in_w, L.in_c, L.out_h, L.out_w, L.kh,
+        L.pad_t, L.pad_l);
   } else {
     int grid = (int)((total + 255) / 256 < (int64_t)ctx->sm_count * 16 ? (total + 255) / 256 : (int64_t)ctx->sm_count * 16);
-    pool_split_scalar_kernel<<<grid, 256, 0, ctx->stream>>>(in_hi, in_lo, out_hi, out_lo, total, L.in_h, L.in_w, L.in_c, L.out_h, L.out_w, L.kh);
+    pool_split_scalar_kernel<<<grid, 256, 0, ctx->stream>>>(in_hi, in_lo, out_hi, out_lo, total, L.in_h, L.in_w, L.in_c, L.out_h, L.out_w, L.kh,
+        L.pad_t, L.pad_l);
   }
   ctx->launches++;
   CUDA_TRY(ctx, cudaGetLastError());
@@ -237,7 +236,7 @@ int nnal_k_pool(nnal_ctx* ctx, const Layer& L, const float* in, float* out, int6
   int64_t total = n * L.out_h * L.out_w * L.out_c;
   if (total == 0) return NNAL_OK;
   int grid = (int)((total + 255) / 256 < (int64_t)ctx->sm_count * 16 ? (total + 255) / 256 : (int64_t)ctx->sm_count * 16);
-  pool_kernel<<<grid, 256, 0, ctx->stream>>>(in, out, total, L.in_h, L.in_w, L.in_c, L.out_h, L.out_w, L.kh);
+  pool_kernel<<<grid, 256, 0, ctx->stream>>>(in, out, total, L.in_h, L.in_w, L.in_c, L.out_h, L.out_w, L.kh, L.pad_t, L.pad_l);
   ctx->launches++;
   CUDA_TRY(ctx, cudaGetLastError());
   return NNAL_OK;

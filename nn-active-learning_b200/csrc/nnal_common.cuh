@@ -89,6 +89,7 @@ struct Layer {
   int kh = 0, kw = 0;
   int in_h = 0, in_w = 0, in_c = 0;      // conv/pool input geometry (NHWC)
   int out_h = 0, out_w = 0, out_c = 0;   // conv/pool output geometry
+  int pad_t = 0, pad_l = 0;              // pool: TF SAME padding before the first row / column (0 for 2x2)
   int in_dim = 0, out_dim = 0;           // fc
   int relu = 0;
   bool has_weights = false;

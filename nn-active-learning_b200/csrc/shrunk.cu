@@ -68,8 +68,9 @@ __global__ void relu_mask_kernel(float* __restrict__ d, const float* __restrict_
 }
 
 // ---- max-pool SAME, window == stride: every input cell asks whether it is the FIRST maximum of its window ----------
+// (window (yo, xo) starts at (yo*s - pt, xo*s - pl): TF's SAME padding before, as in forward_simt.cu)
 __global__ void pool_bwd_kernel(const float* __restrict__ d_out, const float* __restrict__ in, float* __restrict__ d_in,
-                                int64_t total_in, int H, int Wd, int C, int Ho, int Wo, int s) {
+                                int64_t total_in, int H, int Wd, int C, int Ho, int Wo, int s, int pt, int pl) {
   const int per = H * Wd * C;                      // one sample: 32-bit index arithmetic below
   for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total_in; e += (int64_t)gridDim.x * blockDim.x) {
     const int64_t smp = e / per;
@@ -77,16 +78,14 @@ __global__ void pool_bwd_kernel(const float* __restrict__ d_out, const float* __
     const int c = r % C;
     const int t = r / C;
     const int x = t % Wd, y = t / Wd;
-    const int yo = y / s, xo = x / s;
+    const int yo = (y + pt) / s, xo = (x + pl) / s;
     const float* base = in + smp * per;
     float m = -INFINITY;
     int wy = -1, wx = -1;
-    for (int dy = 0; dy < s; ++dy) {
-      const int y2 = yo * s + dy;
-      if (y2 >= H) break;
-      for (int dx = 0; dx < s; ++dx) {
-        const int x2 = xo * s + dx;
-        if (x2 >= Wd) break;
+    const int y0 = yo * s - pt, x0 = xo * s - pl;
+    const int y1 = min(y0 + s, H), x1 = min(x0 + s, Wd);
+    for (int y2 = max(y0, 0); y2 < y1; ++y2) {
+      for (int x2 = max(x0, 0); x2 < x1; ++x2) {
         const float v = base[(y2 * Wd + x2) * C + c];
         if (v > m) { m = v; wy = y2; wx = x2; }
       }
@@ -97,7 +96,7 @@ __global__ void pool_bwd_kernel(const float* __restrict__ d_out, const float* __
 
 // four channels per thread (C % 4 == 0): 16-byte loads, four independent comparisons in flight
 __global__ void pool_bwd_vec4_kernel(const float* __restrict__ d_out, const float* __restrict__ in, float* __restrict__ d_in,
-                                     int64_t total4, int H, int Wd, int C, int Ho, int Wo, int s) {
+                                     int64_t total4, int H, int Wd, int C, int Ho, int Wo, int s, int pt, int pl) {
   const int C4 = C / 4, per4 = H * Wd * C4;
   for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total4; e += (int64_t)gridDim.x * blockDim.x) {
     const int64_t smp = e / per4;
@@ -105,16 +104,14 @@ __global__ void pool_bwd_vec4_kernel(const float* __restrict__ d_out, const floa
     const int c4 = r % C4;
     const int t = r / C4;
     const int x = t % Wd, y = t / Wd;
-    const int yo = y / s, xo = x / s;
+    const int yo = (y + pt) / s, xo = (x + pl) / s;
     const float* base = in + smp * (int64_t)per4 * 4 + 4 * c4;
     float m[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
     int win[4] = {-1, -1, -1, -1};
-    for (int dy = 0; dy < s; ++dy) {
-      const int y2 = yo * s + dy;
-      if (y2 >= H) break;
-      for (int dx = 0; dx < s; ++dx) {
-        const int x2 = xo * s + dx;
-        if (x2 >= Wd) break;
+    const int y0 = yo * s - pt, x0 = xo * s - pl;
+    const int y1 = min(y0 + s, H), x1 = min(x0 + s, Wd);
+    for (int y2 = max(y0, 0); y2 < y1; ++y2) {
+      for (int x2 = max(x0, 0); x2 < x1; ++x2) {
         const float4 v = *reinterpret_cast<const float4*>(base + (int64_t)(y2 * Wd + x2) * C);
         const float vv[4] = {v.x, v.y, v.z, v.w};
         const int id = y2 * Wd + x2;
@@ -733,10 +730,11 @@ int shrunk_chunk(nnal_ctx* ctx, BwState* st, int64_t nb, int64_t n_total, int64_
         const int64_t total_in = nb * L.in_h * L.in_w * L.in_c;
         if (L.in_c % 4 == 0)
           pool_bwd_vec4_kernel<<<grid_for(ctx, total_in / 4, 16), 256, 0, ctx->stream>>>(d, in_of(i), other, total_in / 4, L.in_h,
-                                                                                         L.in_w, L.in_c, L.out_h, L.out_w, L.kh);
+                                                                                         L.in_w, L.in_c, L.out_h, L.out_w, L.kh,
+                                                                                         L.pad_t, L.pad_l);
         else
           pool_bwd_kernel<<<grid_for(ctx, total_in, 16), 256, 0, ctx->stream>>>(d, in_of(i), other, total_in, L.in_h, L.in_w,
-                                                                                L.in_c, L.out_h, L.out_w, L.kh);
+                                                                                L.in_c, L.out_h, L.out_w, L.kh, L.pad_t, L.pad_l);
         ctx->launches++;
         d = other; pp ^= 1;
         continue;

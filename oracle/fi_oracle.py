@@ -18,7 +18,7 @@ which is exactly the SDP objective of NNAL_tools.py:589-602 evaluated at
 q = uniform(S).
 """
 import numpy as np
-from .nnal_oracle import forward, stable_topk, batch_eval, get_patches, normalize_batch_eval
+from .nnal_oracle import forward, stable_topk, batch_eval, get_patches, normalize_batch_eval, pool_same_pads
 
 __all__ = [
     'class_score_factors', 'explicit_class_gradients', 'shrink_gradient',
@@ -68,12 +68,13 @@ def _backward(layers, weights, acts, dlogits):
                 x = rec['in']
                 _, H, Wd, C = x.shape
                 Ho, Wo = nhwc.shape[1], nhwc.shape[2]
-                am = rec['argmax']                       # [N,Ho,Wo,C] index in s*s window
+                am = rec['argmax']                       # [N,Ho,Wo,C] index in s*s window of the padded input
                 dxp = np.zeros((N, Ho, Wo, C, s * s))
                 np.put_along_axis(dxp, am[..., None], d[..., None], axis=-1)
                 dxp = dxp.reshape(N, Ho, Wo, C, s, s).transpose(0, 1, 4, 2, 5, 3)
                 dxp = dxp.reshape(N, Ho * s, Wo * s, C)
-                d = dxp[:, :H, :Wd, :]
+                pt, pl = pool_same_pads(H, s)[0], pool_same_pads(Wd, s)[0]
+                d = dxp[:, pt:pt + H, pl:pl + Wd, :]
             elif spec[1] == 'conv':
                 W = weights[name][0].astype(np.float64)
                 kh, kw, cin, cout = W.shape

@@ -9,7 +9,7 @@ import numpy as np
 __all__ = [
     'pw1_layers', 'he_init_weights', 'layer_shapes',
     'get_patches', 'get_patches_multimg', 'global2local_inds',
-    'normalize_batch_eval', 'conv2d_same', 'max_pool_same', 'flatten_tf',
+    'normalize_batch_eval', 'conv2d_same', 'pool_same_pads', 'max_pool_same', 'flatten_tf',
     'forward', 'batch_eval', 'compute_entropy', 'uncertainty_filtering',
     'binary_uncertainty_filter', 'stable_topk', 'bin_uncertainty_filter_multimg',
     'pixelwise_entropy', 'query_entropy_single', 'query_entropy_multimg',
@@ -181,13 +181,25 @@ def conv2d_same(x, W, b):
     return out + b.reshape(1, 1, 1, cout)
 
 
+def pool_same_pads(n, s):
+    """TF SAME padding of a window-s, stride-s pool along an axis of length n:
+    out = ceil(n/s), pad_total = out*s - n, (pad_before, pad_after) =
+    (pad_total // 2, pad_total - pad_total // 2)."""
+    tot = -(-n // s) * s - n
+    return tot // 2, tot - tot // 2
+
+
 def max_pool_same(x, s=2, return_argmax=False):
     """tf.nn.max_pool(ksize=s, strides=s, 'SAME') (NN.py:1473-1477): output
-    ceil(n/s); padding goes AFTER and never wins."""
+    ceil(n/s); the pad_total = out*s - n padded cells are split with the
+    smaller half BEFORE the first row/column (``pool_same_pads``; nothing before
+    for s = 2) and never win.  ``return_argmax`` indexes the s*s window of the
+    PADDED input."""
     N, H, W, C = x.shape
     Ho, Wo = -(-H // s), -(-W // s)
+    pt, pl = pool_same_pads(H, s)[0], pool_same_pads(W, s)[0]
     xp = np.full((N, Ho * s, Wo * s, C), -np.inf, dtype=x.dtype)
-    xp[:, :H, :W, :] = x
+    xp[:, pt:pt + H, pl:pl + W, :] = x
     xr = xp.reshape(N, Ho, s, Wo, s, C).transpose(0, 1, 3, 5, 2, 4).reshape(N, Ho, Wo, C, s * s)
     out = xr.max(axis=-1)
     if return_argmax:

@@ -1,7 +1,7 @@
 """Float32 torch-CPU restatement of the forward pass (TEST ORACLE / CPU BASELINE ONLY).
 
 Same TF semantics as ``oracle.nnal_oracle.forward`` (conv SAME stride 1 + bias + ReLU, max-pool
-SAME = ceil_mode, flatten row = c*(W*H)+w*H+h, column-batch FC, softmax over classes; NN.py:184-188,
+SAME with TF's split of the padding (``pool_same_pads``), flatten row = c*(W*H)+w*H+h, column-batch FC, softmax over classes; NN.py:184-188,
 258-340, 1473-1477) but in float32 on all host cores, which is the closest stand-in for the
 reference's TensorFlow-CPU execution that can run here (TensorFlow 1.x is not installable;
 BASELINE.md §4).  Used by bench.py's ``cpu_baseline`` / ``--impl reference`` legs and by tests as
@@ -9,6 +9,8 @@ a fast second opinion."""
 import numpy as np
 import torch
 import torch.nn.functional as F
+
+from .nnal_oracle import pool_same_pads
 
 
 class TorchForward(object):
@@ -42,7 +44,12 @@ class TorchForward(object):
                 W, b = self.params[name]
                 h = F.relu(F.conv2d(h, W, b, padding=(W.shape[2] // 2, W.shape[3] // 2)))
             elif spec[1] == 'pool':
-                h = F.max_pool2d(h, spec[0][0], spec[0][0], ceil_mode=True)
+                s = spec[0][0]
+                (pt, pb), (pl, pr) = pool_same_pads(h.shape[2], s), pool_same_pads(h.shape[3], s)
+                if pt or pl:
+                    h = F.max_pool2d(F.pad(h, (pl, pr, pt, pb), value=-float('inf')), s, s)
+                else:                 # padding after only (always for s = 2): ceil mode is the same window set
+                    h = F.max_pool2d(h, s, s, ceil_mode=True)
             else:
                 if not flat:
                     h = h.permute(1, 3, 2, 0).reshape(-1, h.shape[0])     # [C,W,H,N] -> [C*W*H, N]
