@@ -100,7 +100,7 @@ int nnal_model_set(nnal_ctx* ctx, const nnal_layer_spec* specs, int n_layers, in
 int nnal_model_set_weights(nnal_ctx* ctx, int layer, const float* W, const float* b);
 int nnal_model_info(nnal_ctx* ctx, int* n_class, int* feat_dim, int* prev_dim);
 /* multiply-accumulates per sample of layer `layer` and the kernel family it runs on: 0 FP32 CUDA cores, 1 tcgen05
- * (conv_tc_kernel / fc_tc_kernel), 2 tcgen05 weight-stationary conv (conv_wt_kernel) */
+ * (conv_tc_kernel / fc_tc_pair_kernel), 2 tcgen05 weight-stationary conv (conv_wt_kernel) */
 int nnal_model_layer_info(nnal_ctx* ctx, int layer, int* type, long long* macs_per_sample, int* uses_tc);
 
 /* ---- volumes: the padded multi-modality images the query functions receive ----------------- */

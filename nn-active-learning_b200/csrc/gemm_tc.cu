@@ -11,12 +11,17 @@
 // into FP32 TMEM accumulators (chunks of 8 k-blocks, summed with round-to-nearest in registers: the tensor core accumulates
 // with round-toward-zero): 1.1e-5 ... 2.3e-5 max posterior error measured on PW1.
 //
-// Structure (one persistent CTA per SM, 384 threads):
-//   warp 0    : TMA producer  -- cp.async.bulk.tensor 2-D tiles (SWIZZLE_128B) of A_hi, A_lo, W_hi, W_lo
-//   warp 1    : MMA issuer    -- one elected lane issues tcgen05.mma.cta_group::1.kind::f16, M=128 N=256 K=16
-//   warp 2    : TMEM allocator (512 columns = two 128x256 FP32 accumulators)
-//   warps 4-11: epilogue      -- tcgen05.ld -> FP32 register sums -> +bias, ReLU -> global (fp32 / fp16 hi,lo)
-// smem ring: 2 stages x (2 x 16 KB A + 2 x 32 KB W) = 192 KB, mbarrier full/empty pairs.
+// Structure: persistent CTA pairs (clusters of 2, one pair per two SMs), 384 threads per CTA.  A pair computes a
+// 256 (M) x 256 (N) tile with the 2-SM MMA: each CTA holds its own 128 rows of A and half (128) of the 256 W rows, so a
+// CTA reads 64 KB per 64-wide k-block for the MMA work that needed 96 KB with one CTA per 128x256 tile.
+//   warp 0    : TMA producer (both CTAs) -- cp.async.bulk.tensor 2-D tiles (SWIZZLE_128B) of A_hi, A_lo, W_hi, W_lo; the
+//               loads of both CTAs complete on the leader CTA's full barrier
+//   warp 1    : MMA issuer (leader CTA only) -- one elected lane issues tcgen05.mma.cta_group::2.kind::f16, M=256 N=256 K=16;
+//               tcgen05.commit ... multicast frees the stage in both CTAs and signals both accumulator-full barriers
+//   warp 2    : TMEM allocator (cta_group::2, 512 columns per CTA = two 128x256 FP32 accumulators)
+//   warps 4-11: epilogue (both CTAs, own 128 rows) -- tcgen05.ld -> FP32 register sums -> +bias, ReLU -> global (fp32 / fp16
+//               hi,lo); the 16 epilogue warps of the pair release an accumulator on the leader's empty barrier
+// smem ring per CTA: 3 stages x (2 x 16 KB A + 2 x 16 KB W) = 192 KB, mbarrier full/empty pairs.
 //
 // Chunked accumulation.  The tensor core adds into its FP32 accumulator with round-toward-zero
 // (measured on B200: signed bias -1.1e-5 of the output rms at K=4704, shrinking linearly with the
@@ -28,10 +33,11 @@
 
 namespace tc {
 
-constexpr int BM = 128, BN = 256, BK = 64, STAGES = 2;
+constexpr int BM = 128, BN = 256, BK = 64, STAGES = 3;  // BM: rows per CTA; a pair tile is 2 BM x BN
+constexpr int PAIR_M = 2 * BM;
 constexpr int A_BYTES = BM * BK * 2;                  // 16 KB
-constexpr int B_BYTES = BN * BK * 2;                  // 32 KB
-constexpr int STAGE_BYTES = 2 * A_BYTES + 2 * B_BYTES;   // 96 KB
+constexpr int B_BYTES = (BN / 2) * BK * 2;            // 16 KB: this CTA's half of the W rows
+constexpr int STAGE_BYTES = 2 * A_BYTES + 2 * B_BYTES;   // 64 KB per CTA; the leader's full barrier expects both CTAs' bytes
 constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + 1024 /*align slack*/ + 256 /*barriers*/;
 constexpr int NUM_THREADS = 384;
 constexpr int CHUNK_KB = 8;                           // k-blocks (of 64) accumulated inside the tensor core
@@ -43,9 +49,6 @@ __device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
 }
 __device__ __forceinline__ void mbar_arrive_expect_tx(uint32_t bar, uint32_t bytes) {
   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
 }
 // Bounded wait: a protocol bug must surface as a CUDA error (trap), never as a hung GPU.
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
@@ -68,9 +71,34 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
   }
 }
 
+// Arrive on the barrier at the same offset in CTA `rank` of the cluster (the pair's leader for the accumulator-empty barrier).
+__device__ __forceinline__ void mbar_arrive_cluster(uint32_t bar, uint32_t rank) {
+  asm volatile(
+      "{\n\t.reg .b32 ra;\n\t"
+      "mapa.shared::cluster.u32 ra, %0, %1;\n\t"
+      "mbarrier.arrive.release.cluster.shared::cluster.b64 _, [ra];\n\t}"
+      ::"r"(bar), "r"(rank)
+      : "memory");
+}
+__device__ __forceinline__ uint32_t map_to_rank(uint32_t addr, uint32_t rank) {
+  uint32_t r;
+  asm("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank));
+  return r;
+}
+__device__ __forceinline__ uint32_t cluster_ctarank() {
+  uint32_t r;
+  asm("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
+  return r;
+}
+__device__ __forceinline__ void cluster_sync() {
+  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
+}
+
+// 2-SM form: lands in this CTA's shared memory and completes on `bar`, which may be the peer (leader) CTA's barrier
+// (a shared::cluster address from map_to_rank).
 __device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* tmap, uint32_t bar, int c0, int c1) {
   asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
+      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
       ::"r"(dst), "l"(tmap), "r"(bar), "r"(c0), "r"(c1)
       : "memory");
 }
@@ -97,12 +125,14 @@ __device__ __forceinline__ void umma_bf16(uint32_t d_tmem, uint64_t adesc, uint6
   asm volatile(
       "{\n\t.reg .pred p;\n\t"
       "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
+      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
       ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
+// arrives on the barrier at this offset in both CTAs of the pair once the leader's issued MMAs retire
+__device__ __forceinline__ void umma_commit_pair(uint32_t bar) {
+  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
+               ::"r"(bar), "h"((uint16_t)0x3) : "memory");
 }
 __device__ __forceinline__ bool elect_one_sync() {
   uint32_t pred;
@@ -157,13 +187,15 @@ struct FcParams {
   DropSpec drop;             // tf.nn.dropout on the activated output (thresh == 0: off)
 };
 
-__global__ void __launch_bounds__(NUM_THREADS, 1)
-fc_tc_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__ CUtensorMap tmAl,
-             const __grid_constant__ CUtensorMap tmBh, const __grid_constant__ CUtensorMap tmBl, FcParams p) {
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1)
+fc_tc_pair_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__ CUtensorMap tmAl,
+                  const __grid_constant__ CUtensorMap tmBh, const __grid_constant__ CUtensorMap tmBl, FcParams p) {
   extern __shared__ uint8_t smem_raw[];
   const uint32_t raw = smem_u32(smem_raw);
   const uint32_t base = (raw + 1023u) & ~1023u;            // SWIZZLE_128B tiles need 1024-B alignment
   uint8_t* base_ptr = smem_raw + (base - raw);
+  // Both CTAs of a pair use the same offsets: the leader's MMA descriptors and commits address the peer's stages and barriers
+  // at the offsets of its own.
   const uint32_t bar0 = base + STAGES * STAGE_BYTES;
   auto full_bar = [&](int s) { return bar0 + 8u * s; };
   auto empty_bar = [&](int s) { return bar0 + 8u * (STAGES + s); };
@@ -172,13 +204,16 @@ fc_tc_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__ C
   volatile uint32_t* tmem_slot = reinterpret_cast<volatile uint32_t*>(base_ptr + STAGES * STAGE_BYTES + 8 * (2 * STAGES + 4));
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int mblocks = (p.M + BM - 1) / BM, nblocks = (p.N + BN - 1) / BN;
+  const uint32_t rank = cluster_ctarank();                 // 0: leader (issues the MMAs), 1: peer
+  const int pair = blockIdx.x >> 1, npairs = gridDim.x >> 1;
+  const int mblocks = (p.M + PAIR_M - 1) / PAIR_M, nblocks = (p.N + BN - 1) / BN;
   const int ntiles = mblocks * nblocks;
-  // Tile order: N is cut into bands of NBAND column blocks and a band is finished (all row blocks) before the next starts.  With
-  // the plain row-major order the 148 tiles in flight touch EVERY column block: fc1's weight planes (77 MB) went through the L2
-  // once per wave and were re-read from HBM 14 times per launch (1.42 GB read against 0.39 GB algorithmic, profiles/r2_traffic.json);
-  // with bands, fc1 reads 1.22 GB and fc2 0.99 GB (was 1.22) and both run 2-3 % faster.  (The band's planes still do not survive from
-  // one wave to the next -- L2 evict_last / evict_first hints on the TMA loads changed nothing for fc1 and cost fc2 20 % more reads.)
+  // Tile order (in pair tiles): N is cut into bands of NBAND column blocks and a band is finished (all row blocks) before the next
+  // starts.  With the plain row-major order the tiles in flight touch EVERY column block: fc1's weight planes (77 MB) went through
+  // the L2 once per wave and were re-read from HBM 14 times per launch (1.42 GB read against 0.39 GB algorithmic,
+  // profiles/r2_traffic.json); with bands, fc1 reads 1.22 GB and fc2 0.99 GB (was 1.22) and both run 2-3 % faster.  (The band's
+  // planes still do not survive from one wave to the next -- L2 evict_last / evict_first hints on the TMA loads changed nothing
+  // for fc1 and cost fc2 20 % more reads.)
   constexpr int NBAND = 8;
   auto tile_blocks = [&](int t, int& m_blk, int& n_blk) {
     const int full = mblocks * NBAND;
@@ -199,23 +234,26 @@ fc_tc_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__ C
   }
   if (warp == 1 && lane == 0) {
     for (int s = 0; s < STAGES; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
-    for (int a = 0; a < 2; ++a) { mbar_init(tfull_bar(a), 1); mbar_init(tempty_bar(a), 8); }
+    // accumulator-empty: released by the 8 epilogue warps of each CTA (only the leader's barrier is used)
+    for (int a = 0; a < 2; ++a) { mbar_init(tfull_bar(a), 1); mbar_init(tempty_bar(a), 16); }
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   if (warp == 2) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32((const void*)tmem_slot)), "r"(512));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
+    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32((const void*)tmem_slot)), "r"(512));
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;");
   }
+  // the peer's TMA and epilogue signal the leader's barriers: both CTAs' barriers must be initialised first
   tc_fence_before();
-  __syncthreads();
+  cluster_sync();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
 
   if (warp == 0) {
-    // ===== TMA producer =====
+    // ===== TMA producer (both CTAs): own 128 rows of A, own 128 of the tile's 256 W rows =====
     if (lane == 0) {
       uint32_t it = 0;
-      for (int t = blockIdx.x; t < ntiles; t += gridDim.x) {
+      const int a_row = (int)rank * BM, b_row = (int)rank * (BN / 2);
+      for (int t = pair; t < ntiles; t += npairs) {
         int n_blk, m_blk;
         tile_blocks(t, m_blk, n_blk);
         for (int kb = 0; kb < p.num_kb; ++kb, ++it) {
@@ -223,19 +261,20 @@ fc_tc_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__ C
           const uint32_t ph = (it / STAGES) & 1;
           mbar_wait(empty_bar(s), ph ^ 1);
           const uint32_t sa = base + s * STAGE_BYTES;
-          mbar_arrive_expect_tx(full_bar(s), STAGE_BYTES);
-          tma_load_2d(sa, &tmAh, full_bar(s), kb * BK, m_blk * BM);
-          tma_load_2d(sa + A_BYTES, &tmAl, full_bar(s), kb * BK, m_blk * BM);
-          tma_load_2d(sa + 2 * A_BYTES, &tmBh, full_bar(s), kb * BK, n_blk * BN);
-          tma_load_2d(sa + 2 * A_BYTES + B_BYTES, &tmBl, full_bar(s), kb * BK, n_blk * BN);
+          const uint32_t fb = map_to_rank(full_bar(s), 0);
+          if (rank == 0) mbar_arrive_expect_tx(full_bar(s), 2 * STAGE_BYTES);
+          tma_load_2d(sa, &tmAh, fb, kb * BK, m_blk * PAIR_M + a_row);
+          tma_load_2d(sa + A_BYTES, &tmAl, fb, kb * BK, m_blk * PAIR_M + a_row);
+          tma_load_2d(sa + 2 * A_BYTES, &tmBh, fb, kb * BK, n_blk * BN + b_row);
+          tma_load_2d(sa + 2 * A_BYTES + B_BYTES, &tmBl, fb, kb * BK, n_blk * BN + b_row);
         }
       }
     }
-  } else if (warp == 1) {
-    // ===== MMA issuer: warp-uniform control flow, one elected lane issues =====
-    const uint32_t idesc = make_idesc_bf16(BM, BN);
+  } else if (warp == 1 && rank == 0) {
+    // ===== MMA issuer (leader): warp-uniform control flow, one elected lane issues =====
+    const uint32_t idesc = make_idesc_bf16(PAIR_M, BN);
     uint32_t it = 0, cc = 0;                                     // smem-stage counter, accumulation-chunk counter
-    for (int t = blockIdx.x; t < ntiles; t += gridDim.x) {
+    for (int t = pair; t < ntiles; t += npairs) {
       for (int kb0 = 0; kb0 < p.num_kb; kb0 += CHUNK_KB, ++cc) {
         const int acc = cc & 1;
         const uint32_t acc_ph = (cc >> 1) & 1;
@@ -259,8 +298,8 @@ fc_tc_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__ C
               umma_bf16(d_tmem, dAh + adv, dBl + adv, idesc, 1);
               umma_bf16(d_tmem, dAh + adv, dBh + adv, idesc, 1);
             }
-            umma_commit(empty_bar(s));                           // frees the smem stage when the MMAs retire
-            if (kb == kb1 - 1) umma_commit(tfull_bar(acc));      // chunk complete -> epilogue
+            umma_commit_pair(empty_bar(s));                      // frees the smem stage of both CTAs when the MMAs retire
+            if (kb == kb1 - 1) umma_commit_pair(tfull_bar(acc)); // chunk complete -> both epilogues
           }
           __syncwarp();
         }
@@ -271,7 +310,7 @@ fc_tc_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__ C
     const int q = warp & 3;                                      // TMEM lane quarter owned by this warp
     const int half = (warp - 4) >> 2;                            // which 128 of the 256 accumulator columns
     uint32_t cc = 0;
-    for (int t = blockIdx.x; t < ntiles; t += gridDim.x) {
+    for (int t = pair; t < ntiles; t += npairs) {
       int n_blk, m_blk;
       tile_blocks(t, m_blk, n_blk);
       float sum[128];
@@ -292,9 +331,9 @@ fc_tc_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__ C
         }
         tc_fence_before();
         __syncwarp();
-        if (lane == 0) mbar_arrive(tempty_bar(acc));
+        if (lane == 0) mbar_arrive_cluster(tempty_bar(acc), 0);
       }
-      const int row = m_blk * BM + q * 32 + lane;
+      const int row = m_blk * PAIR_M + (int)rank * BM + q * 32 + lane;
       if (row < p.M) {
 #pragma unroll
         for (int c = 0; c < 128; c += 16) {
@@ -377,11 +416,13 @@ fc_tc_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__ C
     }
   }
 
+  // Neither CTA leaves while the other may still signal its barriers or (leader MMAs) use its shared and tensor memory.
+  __syncwarp();
   tc_fence_before();
-  __syncthreads();
+  cluster_sync();
   if (warp == 2) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512));
+    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512));
   }
 }
 
@@ -408,7 +449,7 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
 
 struct TcState {
   EncodeTiledFn encode = nullptr;
-  bool attr_set = false;
+  int max_pairs = 0;         // co-resident CTA pairs of fc_tc_pair_kernel (0: not queried yet)
 };
 
 static int get_state(nnal_ctx* ctx, TcState** out) {
@@ -485,20 +526,33 @@ int nnal_tc_gemm_planes(nnal_ctx* ctx, const nnal_h* Ah, const nnal_h* Al, int64
   CUtensorMap tmAh, tmAl, tmBh, tmBl;
   NNAL_TRY(tc::make_tmap(ctx, st, &tmAh, Ah, (uint64_t)K, (uint64_t)M, (uint64_t)lda, tc::BM));
   NNAL_TRY(tc::make_tmap(ctx, st, &tmAl, Al, (uint64_t)K, (uint64_t)M, (uint64_t)lda, tc::BM));
-  NNAL_TRY(tc::make_tmap(ctx, st, &tmBh, Bh, (uint64_t)K, (uint64_t)N, (uint64_t)ldb, tc::BN));
-  NNAL_TRY(tc::make_tmap(ctx, st, &tmBl, Bl, (uint64_t)K, (uint64_t)N, (uint64_t)ldb, tc::BN));
-  if (!st->attr_set) {
-    CUDA_TRY(ctx, cudaFuncSetAttribute(tc::fc_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_BYTES));
-    st->attr_set = true;
+  NNAL_TRY(tc::make_tmap(ctx, st, &tmBh, Bh, (uint64_t)K, (uint64_t)N, (uint64_t)ldb, tc::BN / 2));
+  NNAL_TRY(tc::make_tmap(ctx, st, &tmBl, Bl, (uint64_t)K, (uint64_t)N, (uint64_t)ldb, tc::BN / 2));
+  if (!st->max_pairs) {
+    CUDA_TRY(ctx, cudaFuncSetAttribute(tc::fc_tc_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_BYTES));
+    cudaLaunchConfig_t cfg = {};
+    cudaLaunchAttribute attr;
+    attr.id = cudaLaunchAttributeClusterDimension;
+    attr.val.clusterDim.x = 2; attr.val.clusterDim.y = 1; attr.val.clusterDim.z = 1;
+    cfg.gridDim = dim3(2 * ctx->sm_count);
+    cfg.blockDim = dim3(tc::NUM_THREADS);
+    cfg.dynamicSmemBytes = tc::SMEM_BYTES;
+    cfg.stream = ctx->stream;
+    cfg.attrs = &attr;
+    cfg.numAttrs = 1;
+    int n = 0;
+    CUDA_TRY(ctx, cudaOccupancyMaxActiveClusters(&n, (void*)tc::fc_tc_pair_kernel, &cfg));
+    if (n < 1) NNAL_FAIL(ctx, NNAL_ERR_CUDA, "fc_tc_pair_kernel: no CTA pair fits on the device");
+    st->max_pairs = n;
   }
   tc::FcParams p;
   p.bias = bias; p.out = out; p.out_hi = out_hi; p.out_lo = out_lo; p.ld_split = ld_split;
   p.M = (int)M; p.N = N; p.num_kb = (int)((K + tc::BK - 1) / tc::BK); p.relu = relu; p.ldo = ldo; p.w_scale_inv = scale;
   p.accum = accum;
   p.drop = drop ? *drop : DropSpec();
-  const int ntiles = cdiv(M, tc::BM) * cdiv(N, tc::BN);
-  const int grid = ntiles < ctx->sm_count ? ntiles : ctx->sm_count;
-  tc::fc_tc_kernel<<<grid, tc::NUM_THREADS, tc::SMEM_BYTES, ctx->stream>>>(tmAh, tmAl, tmBh, tmBl, p);
+  const int ntiles = cdiv(M, tc::PAIR_M) * cdiv(N, tc::BN);
+  const int pairs = ntiles < st->max_pairs ? ntiles : st->max_pairs;
+  tc::fc_tc_pair_kernel<<<2 * pairs, tc::NUM_THREADS, tc::SMEM_BYTES, ctx->stream>>>(tmAh, tmAl, tmBh, tmBl, p);
   ctx->launches++;
   CUDA_TRY(ctx, cudaGetLastError());
   return NNAL_OK;

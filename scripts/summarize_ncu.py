@@ -85,7 +85,7 @@ def traffic(path, samples_per_launch):
             re.search(r'Cfg<(\d+), \d+, (\d+), (\d+)', name)
         if ('conv_tc_kernel' in name or 'conv_wt_kernel' in name) and m:
             cls = {('25', '3'): 'conv1', ('25', '16'): 'conv1', ('25', '24'): 'conv2', ('13', '32'): 'conv3', ('13', '48'): 'conv4'}.get((m.group(1), m.group(2)))
-        elif 'fc_tc_kernel' in name:
+        elif 'fc_tc_kernel' in name or 'fc_tc_pair_kernel' in name:
             nfc += 1
             cls = 'fc%d' % nfc if nfc <= 2 else None
         elif 'gather_split_kernel' in name:
