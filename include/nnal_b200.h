@@ -248,7 +248,7 @@ int nnal_fi_step_pack(nnal_ctx* ctx, int64_t step, void* d_msg);
 int nnal_fi_step_apply_gathered(nnal_ctx* ctx, int64_t step, const void* d_msgs, int world, int rank);
 int nnal_fi_result(nnal_ctx* ctx, int64_t k, int64_t* gids_out, double* red_out);
 
-/* Greedy FI selection for multi-class models (2 <= c <= 32), last FC layer only, in block form (csrc/fi_block.cu):
+/* Greedy FI selection for multi-class models (2 <= c <= 32), last FC layer (or the last two, below), in block form (csrc/fi_block.cu):
  * F_i = A(pi_i) (x) [u_i;1][u_i;1]^T with A(pi) = diag pi - pi pi^T = L_i L_i^T (closed-form c x (c-1) factor of the
  * float64-renormalised posteriors), block kernel K_ij = (L_i^T L_j)(u_i.u_j + 1), D = c(d+1), r = c-1.  Same objective
  * f(S) = tr((sum_{i in S} F_i/|S| + delta I)^-1) = (D - |S| r)/delta + red(S), red(S) = tr((delta I + K_SS/|S|)^-1), and
@@ -258,6 +258,16 @@ int nnal_fi_result(nnal_ctx* ctx, int64_t k, int64_t* gids_out, double* red_out)
  * post[c][n] posteriors, U[n][d] feature-layer activations (input of the last FC). */
 int nnal_fi_block_set_candidates(nnal_ctx* ctx, const int64_t* cand, int64_t n_cand);
 int nnal_fi_block_set_factors(nnal_ctx* ctx, int64_t n, int c, int d, const float* post, const float* U);
+/* The same over the last TWO FC layers (n_layers = 2; n_layers = 1 is the pair above): the previous FC's weights and bias are
+ * added, g_y = [(e_y - pi) (x) [u;1] ; (M W3^T (e_y - pi)) (x) [a;1]], M = diag 1[u > 0], W3 the last FC's [c][d] weights,
+ * a the input of the feature layer's FC (prev_dim); the block kernel becomes K_ij = L_i^T (s_ij I + s'_ij W3 diag(m_i o m_j) W3^T) L_j,
+ * s'_ij = a_i.a_j + 1, and D = c(d+1) + d(d_prev+1).  At c = 2 it is the binary n_layers = 2 kernel of nnal_fi_*.
+ * In place: the pool pass must have kept the previous FC output (keep >= 2, else NNAL_ERR_STATE); W3 is the model's.
+ * Host factors: A_prev[n][d_prev] and w_last[c][d], both NULL (one layer) or both given.  The greedy keeps k(c-1)-many
+ * columns of c(c+1)/2 + 2 doubles per candidate; a size the device cannot hold returns NNAL_ERR_UNSUPPORTED. */
+int nnal_fi_block_set_candidates_nl(nnal_ctx* ctx, const int64_t* cand, int64_t n_cand, int n_layers);
+int nnal_fi_block_set_factors_nl(nnal_ctx* ctx, int64_t n, int c, int d, int d_prev, const float* post, const float* U,
+                                 const float* A_prev, const float* w_last);
 int nnal_fi_block_greedy(nnal_ctx* ctx, int64_t k, double delta, int64_t* sel_out, double* obj_out, double* red_out);
 
 /* All-gather of the per-step messages over NVLink peer memory instead of NCCL (csrc/p2p.cu): 100 dependent steps of one small
@@ -352,6 +362,8 @@ int nnal_cs_step_apply_gathered(nnal_ctx* ctx, int64_t step, const void* d_msgs,
 int nnal_cs_greedy(nnal_ctx* ctx, int64_t k, int64_t* sel_out, double* val_out);
 /* feature rows of the given pool positions as [n][d] float32 on the host (row-major) */
 int nnal_pool_feature_rows(nnal_ctx* ctx, const int64_t* pos, int64_t n, float* out);
+/* Rows `pos` of the previous FC layer's output (input of the feature layer's FC, prev_dim) kept by a pool pass with keep >= 2. */
+int nnal_pool_prev_rows(nnal_ctx* ctx, const int64_t* pos, int64_t n, float* out);
 
 /* ---- test hooks --------------------------------------------------------------------------- */
 /* Kernel-selection switches for TESTS (there are no environment variables): "chunk" / "bw_chunk" (samples per chunk of the

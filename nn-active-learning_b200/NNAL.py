@@ -34,7 +34,8 @@ def CNN_query(model, expr, pool_inds, method_name, session, col=True, extra_feed
     ``entropy``: posteriors ``[c,n]`` -> compute_entropy (zeros -> 1e-7) -> argsort(-H)[:k]
     (NNAL.py:298-310).  ``fi``: see ``nnal_b200.fi.query_whole``; ``expr.pars['fi_mode'] = 'sdp'`` runs the reference's
     own multiclass A-matrix + SDP + sampling pipeline (``nnal_b200.fi.query_whole_sdp``); ``'block-greedy'`` runs the greedy
-    last-layer FI selection for any number of classes (``nnal_b200.fi.query_whole_block``)."""
+    FI selection for any number of classes (``nnal_b200.fi.query_whole_block``) over the last FC layer, or over the last two
+    with ``expr.pars['fi_layers'] = 2``."""
     k = expr.pars['k']
     if method_name == 'random':
         return np.random.permutation(len(pool_inds))[:k]

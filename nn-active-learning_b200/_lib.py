@@ -77,6 +77,7 @@ SIGNATURES = {
     'nnal_cs_step_apply_gathered': (C.c_int, [c_vp, C.c_int64, c_vp, C.c_int, C.c_int]),
     'nnal_cs_greedy': (C.c_int, [c_vp, C.c_int64, c_vp, c_vp]),
     'nnal_pool_feature_rows': (C.c_int, [c_vp, c_vp, C.c_int64, c_vp]),
+    'nnal_pool_prev_rows': (C.c_int, [c_vp, c_vp, C.c_int64, c_vp]),
     'nnal_fi_set_candidates': (C.c_int, [c_vp, c_vp, C.c_int64, C.c_int]),
     'nnal_fi_set_factors': (C.c_int, [c_vp, C.c_int64, C.c_int, C.c_int, c_vp, c_vp, c_vp, c_vp]),
     'nnal_fi_info': (C.c_int, [c_vp, c_i64p, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int), c_f64p]),
@@ -97,6 +98,8 @@ SIGNATURES = {
     'nnal_fi_block_set_candidates': (C.c_int, [c_vp, c_vp, C.c_int64]),
     'nnal_fi_block_set_factors': (C.c_int, [c_vp, C.c_int64, C.c_int, C.c_int, c_vp, c_vp]),
     'nnal_fi_block_greedy': (C.c_int, [c_vp, C.c_int64, C.c_double, c_vp, c_vp, c_vp]),
+    'nnal_fi_block_set_candidates_nl': (C.c_int, [c_vp, c_vp, C.c_int64, C.c_int]),
+    'nnal_fi_block_set_factors_nl': (C.c_int, [c_vp, C.c_int64, C.c_int, C.c_int, C.c_int, c_vp, c_vp, c_vp, c_vp]),
     'nnal_p2p_alloc':(C.c_int, [c_vp, C.c_int, C.c_int, C.c_int64, c_vp]),
     'nnal_p2p_open': (C.c_int, [c_vp, c_vp]),
     'nnal_p2p_allgather': (C.c_int, [c_vp, c_vp, C.c_int64, C.c_uint64, c_vp]),

@@ -859,25 +859,37 @@ __global__ void gather_rows_f32_kernel(const float* __restrict__ src, const int6
   }
 }
 
-extern "C" int nnal_pool_feature_rows(nnal_ctx* ctx, const int64_t* pos, int64_t n, float* out) {
-  if (!ctx || n < 0) return NNAL_ERR_INVALID;
-  if (!ctx->pool_feat || ctx->keep < 1) NNAL_FAIL(ctx, NNAL_ERR_STATE, "pool pass did not keep features");
+// rows `pos` of a kept pool matrix src [pool_n][d] -> out [n][d] (host)
+static int gather_pool_rows(nnal_ctx* ctx, const float* src, int d, const int64_t* pos, int64_t n, float* out) {
   if (n == 0) return NNAL_OK;
   if (!pos || !out) return NNAL_ERR_INVALID;
   for (int64_t i = 0; i < n; ++i)
     if (pos[i] < 0 || pos[i] >= ctx->pool_n) NNAL_FAIL(ctx, NNAL_ERR_INVALID, "feature row position outside the pool");
   CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-  const int d = ctx->feat_dim;
   NNAL_TRY(devbuf_reserve(ctx, ctx->act[0], (size_t)n * d * sizeof(float)));
   NNAL_TRY(devbuf_reserve(ctx, ctx->inds, (size_t)n * 8));
   CUDA_TRY(ctx, cudaMemcpyAsync(ctx->inds.p, pos, (size_t)n * 8, cudaMemcpyHostToDevice, ctx->stream));
-  gather_rows_f32_kernel<<<std::min(cdiv(n * d, 256), ctx->sm_count * 16), 256, 0, ctx->stream>>>(ctx->pool_feat, (const int64_t*)ctx->inds.p, n, d,
+  gather_rows_f32_kernel<<<std::min(cdiv(n * d, 256), ctx->sm_count * 16), 256, 0, ctx->stream>>>(src, (const int64_t*)ctx->inds.p, n, d,
                                                                                                  (float*)ctx->act[0].p);
   ctx->launches++;
   CUDA_TRY(ctx, cudaGetLastError());
   CUDA_TRY(ctx, cudaMemcpyAsync(out, ctx->act[0].p, (size_t)n * d * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
   NNAL_SYNC_CHECKED(ctx);
   return NNAL_OK;
+}
+
+extern "C" int nnal_pool_feature_rows(nnal_ctx* ctx, const int64_t* pos, int64_t n, float* out) {
+  if (!ctx || n < 0) return NNAL_ERR_INVALID;
+  if (!ctx->pool_feat || ctx->keep < 1) NNAL_FAIL(ctx, NNAL_ERR_STATE, "pool pass did not keep features");
+  return gather_pool_rows(ctx, ctx->pool_feat, ctx->feat_dim, pos, n, out);
+}
+
+extern "C" int nnal_pool_prev_rows(nnal_ctx* ctx, const int64_t* pos, int64_t n, float* out) {
+  if (!ctx || n < 0) return NNAL_ERR_INVALID;
+  if (!ctx->pool_prev || ctx->keep < 2) NNAL_FAIL(ctx, NNAL_ERR_STATE, "pool pass did not keep the previous FC output");
+  if (ctx->feature_layer < 1 || ctx->layers[ctx->feature_layer - 1].type != NNAL_LAYER_FC)
+    NNAL_FAIL(ctx, NNAL_ERR_UNSUPPORTED, "the layer before the feature layer is not an FC layer");     // pool_prev is not written
+  return gather_pool_rows(ctx, ctx->pool_prev, ctx->prev_dim, pos, n, out);
 }
 
 extern "C" int nnal_pool_score(nnal_ctx* ctx, int kind, double eps) {

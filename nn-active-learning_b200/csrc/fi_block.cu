@@ -1,4 +1,4 @@
-// Greedy Fisher-information selection for multi-class models over the last FC layer (block form, sm_100a).
+// Greedy Fisher-information selection for multi-class models over the last FC layer or the last two (block form, sm_100a).
 //
 // Last-layer FI of a sample with posteriors pi (c classes) and feature vector u (d):  F_i = A(pi_i) (x) ut_i ut_i^T,
 // A(pi) = diag pi - pi pi^T (NN.LLFC_hess, NN.py:891-901), ut = [u;1], D = c(d+1).  A(pi) = L L^T with the closed-form
@@ -14,6 +14,20 @@
 //     append (block row of K_SS) -> build (alpha I + K_SS, identity-padded to a multiple of 64) -> nnal_gj64_invert ->
 //     Z + tr C -> eval (per-candidate loss, block arg-min, last-CTA global arg-min) -> column (s_{., w} for the winner).
 // The host only enqueues; results are read once at the end.
+//
+// Two layers (n_layers = 2: the last FC (W3, b3) and the one before it (W2, b2)).  a = input of the feature layer's FC
+// (d_p = prev_dim), at = [a;1], m = 1[u > 0], M = diag m.  The score of class y is
+//     g_y = [(e_y - pi) (x) ut ; (M W3^T (e_y - pi)) (x) at],   D = c(d+1) + d(d_p+1),
+// so F_i = sum_y pi_y g_y g_y^T = G_i G_i^T with the same L_i, and the block kernel keeps its shape:
+//     K_ij = L_i^T N_ij L_j,   N_ij = s_ij I_c + s'_ij Q_ij,
+//     s_ij = u_i.u_j + 1,  s'_ij = a_i.a_j + 1,  Q_ij = W3 diag(m_i o m_j) W3^T   (c x c, symmetric).
+// At c = 2 this is sqrt(w_i w_j) [2 s_ij + (delta2_i.delta2_j) s'_ij], the binary two-layer kernel of fi.cu.  The greedy step
+// is unchanged; only k_j changes, and with it
+//     Y_j = C k_j = (sum_a Z[:, a-block] N_{w_a j}) L_j
+// (~t^2 r c^2 multiply-adds per candidate and step).  A column of winner w holds, per candidate j, cw = c(c+1)/2 + 2
+// doubles [s_wj, s'_wj, Q_wj (upper triangle, row-major)].  Q_{., w} = Mask P_w is a GEMM with an exact 0/1 A operand
+// (Mask[j,k] = m_j[k]) and P_w[k,(y,z)] = m_w[k] W3[y,k] W3[z,k] (exact in float64: a product of two floats), accumulated
+// in float64 in a fixed order.  Set-up runs the same GEMM with P = P_1 (m_w = 1) for Q_jj.
 #include "nnal_common.cuh"
 #include "dots.cuh"
 #include "../../include/nnal_b200.h"
@@ -27,6 +41,7 @@ constexpr int64_t MAX_KR = 4096;       // k (c-1): order of the largest system i
 constexpr int RT = 8;                  // rows of Z per eval tile
 constexpr int EVAL_THREADS = 256;
 constexpr size_t EVAL_SMEM_MAX = 200 * 1024;
+constexpr size_t EVAL2_SMEM_MAX = 110 * 1024;
 
 struct State {
   int64_t n = 0;
@@ -54,6 +69,14 @@ struct State {
   long long* blk_idx = nullptr;
   int64_t cap_blk = 0, cap_blk_idx = 0;
   unsigned int* ticket = nullptr;
+  // two layers
+  int nl = 1, dp = 0, nq = 0, cw = 1;    // layers covered, prev dim, c(c+1)/2, doubles per candidate in a column
+  const float* A = nullptr;              // [.][dp] inputs of the feature layer's FC (rows as U)
+  const float* W3 = nullptr;             // [c][d] last FC weights
+  float *ownA = nullptr, *ownW = nullptr;
+  int64_t cap_a = 0, cap_w = 0;
+  double *Cd = nullptr, *Pw = nullptr;   // [n][cw] candidates' own columns (set-up), [d][nq] P_w of the current winner
+  int64_t cap_cd = 0, cap_pw = 0;
 };
 
 static State* get(nnal_ctx* ctx) {
@@ -130,6 +153,147 @@ __global__ void __launch_bounds__(256) column_kernel(const float* __restrict__ U
   }
 }
 
+// ---- two layers ----------------------------------------------------------------------------------------------------------
+// packed index of Q[y][z] = Q[z][y]: upper triangle, row-major
+__host__ __device__ inline int qidx(int y, int z, int c) {
+  if (y > z) { const int tmp = y; y = z; z = tmp; }
+  return y * c - (y * (y - 1)) / 2 + (z - y);
+}
+
+// (La^T N Lb)[y, z] with N = col[0] I + col[1] Q, Q packed at col + 2.  L[x, y] = 0 for x < y.
+__device__ inline double lnl(const double* __restrict__ La, const double* __restrict__ Lb, const double* __restrict__ col, int c,
+                             int r, int y, int z) {
+  double ll = 0.0, lq = 0.0;
+  for (int x = y; x < c; ++x) {
+    const double lay = La[x * r + y];
+    double qz = 0.0;
+    for (int x2 = z; x2 < c; ++x2) qz = fma(col[2 + qidx(x, x2, c)], Lb[x2 * r + z], qz);
+    ll = fma(lay, Lb[x * r + z], ll);
+    lq = fma(lay, qz, lq);
+  }
+  return col[0] * ll + col[1] * lq;
+}
+
+// s_{i,w} = u_i.u_w + 1 and s'_{i,w} = a_i.a_w + 1 into col[i][0..1] for every candidate; w = sel[t] (sel = null: w = i)
+__global__ void __launch_bounds__(256) dots2_kernel(const float* __restrict__ U, const float* __restrict__ A,
+                                                    const int64_t* __restrict__ rows, int64_t n, int d, int dp,
+                                                    const long long* __restrict__ sel, int t, double* __restrict__ col, int cw) {
+  const int lane = threadIdx.x & 31;
+  const int64_t rw = sel ? (rows ? rows[sel[t]] : sel[t]) : -1;
+  const int64_t nw = (int64_t)gridDim.x * (blockDim.x >> 5);
+  for (int64_t i = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); i < n; i += nw) {
+    const int64_t ri = rows ? rows[i] : i;
+    const int64_t rj = sel ? rw : ri;
+    const float *u = U + ri * d, *uw = U + rj * d, *a = A + ri * dp, *aw = A + rj * dp;
+    double su = 0.0, sa = 0.0;
+    for (int k = lane; k < d; k += 32) su = fma((double)u[k], (double)uw[k], su);
+    for (int k = lane; k < dp; k += 32) sa = fma((double)a[k], (double)aw[k], sa);
+    su = warp_sum(su);
+    sa = warp_sum(sa);
+    if (lane == 0) { col[i * cw] = su + 1.0; col[i * cw + 1] = sa + 1.0; }
+  }
+}
+
+// P[k][(y,z)] = m_w[k] W3[y][k] W3[z][k], w = sel[t] (sel = null: m_w = 1)
+__global__ void __launch_bounds__(256) pw_kernel(const float* __restrict__ W3, const float* __restrict__ U,
+                                                 const int64_t* __restrict__ rows, int d, int c, int nq,
+                                                 const long long* __restrict__ sel, int t, double* __restrict__ P) {
+  const float* uw = sel ? U + (rows ? rows[sel[t]] : sel[t]) * (int64_t)d : nullptr;
+  const int64_t total = (int64_t)d * nq;
+  for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
+    const int k = (int)(e / nq);
+    int q = (int)(e - (int64_t)k * nq), y = 0;
+    while (q >= c - y) { q -= c - y; ++y; }
+    const int z = y + q;
+    const bool on = !uw || uw[k] > 0.f;
+    P[e] = on ? (double)W3[(int64_t)y * d + k] * (double)W3[(int64_t)z * d + k] : 0.0;
+  }
+}
+
+// col[j][2 + q] = sum_k 1[u_j[k] > 0] P[k][q]: 64 candidates x 64 entries per CTA, 4 x 4 per thread, k in steps of 16,
+// float64 in ascending k (deterministic)
+constexpr int MG_J = 64, MG_Q = 64, MG_K = 16;
+__global__ void __launch_bounds__(256) maskgemm_kernel(const float* __restrict__ U, const int64_t* __restrict__ rows, int64_t n,
+                                                       int d, int nq, const double* __restrict__ P, double* __restrict__ col,
+                                                       int cw) {
+  __shared__ double Ms[MG_K][MG_J + 1];
+  __shared__ double Ps[MG_K][MG_Q];
+  const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
+  const int64_t j0 = (int64_t)blockIdx.x * MG_J;
+  const int q0 = blockIdx.y * MG_Q;
+  double acc[4][4];
+#pragma unroll
+  for (int i = 0; i < 4; ++i)
+#pragma unroll
+    for (int q = 0; q < 4; ++q) acc[i][q] = 0.0;
+  for (int k0 = 0; k0 < d; k0 += MG_K) {
+    for (int e = threadIdx.x; e < MG_J * MG_K; e += 256) {
+      const int jl = e / MG_K, kk = e - jl * MG_K;
+      const int64_t j = j0 + jl;
+      const int k = k0 + kk;
+      const float v = (j < n && k < d) ? U[(rows ? rows[j] : j) * (int64_t)d + k] : 0.f;
+      Ms[kk][jl] = v > 0.f ? 1.0 : 0.0;
+    }
+    for (int e = threadIdx.x; e < MG_K * MG_Q; e += 256) {
+      const int kk = e / MG_Q, ql = e - kk * MG_Q;
+      Ps[kk][ql] = (k0 + kk < d && q0 + ql < nq) ? P[(int64_t)(k0 + kk) * nq + q0 + ql] : 0.0;
+    }
+    __syncthreads();
+#pragma unroll
+    for (int kk = 0; kk < MG_K; ++kk) {
+      double m[4], p[4];
+#pragma unroll
+      for (int i = 0; i < 4; ++i) { m[i] = Ms[kk][ty + 16 * i]; p[i] = Ps[kk][tx + 16 * i]; }
+#pragma unroll
+      for (int i = 0; i < 4; ++i)
+#pragma unroll
+        for (int q = 0; q < 4; ++q) acc[i][q] = fma(m[i], p[q], acc[i][q]);
+    }
+    __syncthreads();
+  }
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const int64_t j = j0 + ty + 16 * i;
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+      const int qq = q0 + tx + 16 * q;
+      if (j < n && qq < nq) col[j * cw + 2 + qq] = acc[i][q];
+    }
+  }
+}
+
+// K_jj = L_j^T N_jj L_j from the candidates' own columns
+__global__ void __launch_bounds__(256) kd2_kernel(const double* __restrict__ Lall, const double* __restrict__ Cd, int64_t n, int c,
+                                                  int r, int cw, double* __restrict__ Kd) {
+  const int lane = threadIdx.x & 31;
+  const int64_t nw = (int64_t)gridDim.x * (blockDim.x >> 5);
+  for (int64_t i = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); i < n; i += nw) {
+    const double* L = Lall + i * (int64_t)c * r;
+    for (int e = lane; e < r * r; e += 32) {
+      const int y = e / r, z = e - y * r;
+      Kd[i * (int64_t)r * r + e] = lnl(L, L, Cd + i * cw, c, r, y, z);
+    }
+  }
+}
+
+// block row a = t-1 of K_SS and its transpose: K[(a,y),(b,z)] = (L_{w_a}^T N_{w_a w_b} L_{w_b})[y,z].  lnl(y,z) and lnl(z,y)
+// round differently, so in the diagonal block only y <= z computes and writes both entries (one writer per entry).
+__global__ void __launch_bounds__(256) append2_kernel(const double* __restrict__ Lsel, const double* __restrict__ Scols, int64_t lds,
+                                                      int cw, const long long* __restrict__ sel, int a, int c, int r,
+                                                      double* __restrict__ Kss, int64_t ldk) {
+  const int64_t total = (int64_t)(a + 1) * r * r;
+  const double* La = Lsel + (int64_t)a * c * r;
+  for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
+    const int b = (int)(e / (r * r));
+    const int yz = (int)(e - (int64_t)b * r * r);
+    const int y = yz / r, z = yz - (yz / r) * r;
+    if (b == a && y > z) continue;
+    const double v = lnl(La, Lsel + (int64_t)b * c * r, Scols + (int64_t)a * lds + sel[b] * cw, c, r, y, z);
+    Kss[(int64_t)(a * r + y) * ldk + b * r + z] = v;
+    Kss[(int64_t)(b * r + z) * ldk + a * r + y] = v;
+  }
+}
+
 // ---- system: block row a = t-1 of K_SS (and its transpose): K[(a,y),(b,z)] = (L_{w_a}^T L_{w_b})[y,z] s_{w_a w_b} -------------
 __global__ void __launch_bounds__(256) append_kernel(const double* __restrict__ Lsel, const double* __restrict__ Scols, int64_t lds,
                                                      const long long* __restrict__ sel, int a, int c, int r,
@@ -194,7 +358,7 @@ struct EvalArgs {
   const double* Lall; const double* Kd; const double* Z; int64_t ldz;
   const double* Scols; int64_t lds;
   double* Lsel; unsigned char* avail;
-  int64_t n; int c, r, t, JC, AT; double alpha;
+  int64_t n; int c, r, t, JC, AT, cw; double alpha;
   const double* trC;
   double* blk_loss; long long* blk_idx; unsigned int* ticket;
   long long* sel; double* red;
@@ -204,14 +368,14 @@ struct EvalLayout {
   int Ls, E, G, Zs, Ss, Ws, Ys, Ks, loss, total;     // offsets in doubles
 };
 
-__host__ __device__ inline EvalLayout eval_layout(int JC, int AT, int c, int r) {
+__host__ __device__ inline EvalLayout eval_layout(int JC, int AT, int c, int r, int cw) {
   EvalLayout l;
   int o = 0;
   l.Ls = o; o += JC * c * r;
   l.E = o; o += JC * r * r;
   l.G = o; o += JC * r * r;
   l.Zs = o; o += RT * AT * c;
-  l.Ss = o; o += AT * JC;
+  l.Ss = o; o += AT * JC * cw;
   l.Ws = o; o += JC * RT * c;
   l.Ys = o; o += JC * RT * r;
   l.Ks = o; o += JC * RT * r;
@@ -249,10 +413,12 @@ __device__ double block_loss(double* __restrict__ Sg, const double* __restrict__
   return tr;
 }
 
+// NL = 2: Ss holds the winners' whole columns [AT][JC][cw], W_j sums Z[:, a-block] N_{w_a j}, and k_j = L^T N L
+template <int NL>
 __global__ void __launch_bounds__(EVAL_THREADS) eval_kernel(EvalArgs ea) {
   extern __shared__ __align__(16) double sm[];
-  const int c = ea.c, r = ea.r, t = ea.t, JC = ea.JC, AT = ea.AT;
-  const EvalLayout lay = eval_layout(JC, AT, c, r);
+  const int c = ea.c, r = ea.r, t = ea.t, JC = ea.JC, AT = ea.AT, cw = NL == 2 ? ea.cw : 1;
+  const EvalLayout lay = eval_layout(JC, AT, c, r, cw);
   double* Ls = sm + lay.Ls;
   double* E = sm + lay.E;
   double* G = sm + lay.G;
@@ -285,17 +451,33 @@ __global__ void __launch_bounds__(EVAL_THREADS) eval_kernel(EvalArgs ea) {
         const int a = a0 + col / c;
         Zs[e] = (rho0 + q < m && a < t) ? ea.Z[(int64_t)(rho0 + q) * ea.ldz + (int64_t)a0 * c + col] : 0.0;
       }
-      for (int e = tid; e < AT * JC; e += blockDim.x) {
-        const int a = e / JC, jj = e - a * JC;
-        Ss[e] = (a0 + a < t && j0 + jj < ea.n) ? ea.Scols[(int64_t)(a0 + a) * ea.lds + j0 + jj] : 0.0;
+      if constexpr (NL == 1) {
+        for (int e = tid; e < AT * JC; e += blockDim.x) {
+          const int a = e / JC, jj = e - a * JC;
+          Ss[e] = (a0 + a < t && j0 + jj < ea.n) ? ea.Scols[(int64_t)(a0 + a) * ea.lds + j0 + jj] : 0.0;
+        }
+      } else {
+        for (int e = tid; e < AT * JC * cw; e += blockDim.x) {
+          const int a = e / (JC * cw), jf = e - a * JC * cw;
+          Ss[e] = (a0 + a < t && j0 + jf / cw < ea.n) ? ea.Scols[(int64_t)(a0 + a) * ea.lds + j0 * cw + jf] : 0.0;
+        }
       }
       __syncthreads();
       if (wt) {
         const int na = min(AT, t - a0);
         for (int a = 0; a < na; ++a) {
-          const double sa = Ss[a * JC + wj];
+          if constexpr (NL == 1) {
+            const double sa = Ss[a * JC + wj];
 #pragma unroll
-          for (int q = 0; q < RT; ++q) acc[q] = fma(sa, Zs[q * ZW + a * c + wx], acc[q]);
+            for (int q = 0; q < RT; ++q) acc[q] = fma(sa, Zs[q * ZW + a * c + wx], acc[q]);
+          } else {
+            const double* col = Ss + (a * JC + wj) * cw;           // N[x, wx] = s [x == wx] + s' Q[x, wx]
+            for (int x = 0; x < c; ++x) {
+              const double nx = fma(col[1], col[2 + qidx(x, wx, c)], x == wx ? col[0] : 0.0);
+#pragma unroll
+              for (int q = 0; q < RT; ++q) acc[q] = fma(nx, Zs[q * ZW + a * c + x], acc[q]);
+            }
+          }
         }
       }
     }
@@ -315,12 +497,17 @@ __global__ void __launch_bounds__(EVAL_THREADS) eval_kernel(EvalArgs ea) {
         if (row < m && j < ea.n) {
           const int ap = row / r, xp = row - (row / r) * r;
           const double* Wq = Ws + (jj * RT + q) * c;
-          const double* La = ea.Lsel + (int64_t)ap * c * r + xp;
-          for (int x = 0; x < c; ++x) {
-            yv = fma(Wq[x], Lj[x * r + y], yv);
-            kv = fma(La[x * r], Lj[x * r + y], kv);
+          if constexpr (NL == 1) {
+            const double* La = ea.Lsel + (int64_t)ap * c * r + xp;
+            for (int x = 0; x < c; ++x) {
+              yv = fma(Wq[x], Lj[x * r + y], yv);
+              kv = fma(La[x * r], Lj[x * r + y], kv);
+            }
+            kv *= ea.Scols[(int64_t)ap * ea.lds + j];
+          } else {
+            for (int x = 0; x < c; ++x) yv = fma(Wq[x], Lj[x * r + y], yv);
+            kv = lnl(ea.Lsel + (int64_t)ap * c * r, Lj, ea.Scols + (int64_t)ap * ea.lds + j * cw, c, r, xp, y);
           }
-          kv *= ea.Scols[(int64_t)ap * ea.lds + j];
         }
         Ys[(jj * RT + q) * r + y] = yv;
         Ks[(jj * RT + q) * r + y] = kv;
@@ -404,15 +591,31 @@ static int flat_grid(nnal_ctx* ctx, int64_t total) {
 }
 
 // candidates per eval CTA and winners per Z tile: as many candidates as 256 threads cover, fewer where shared memory runs out
-static void eval_plan(int c, int r, int* JC, int* AT, size_t* smem) {
+// (two layers: at most EVAL2_SMEM_MAX, so that two CTAs share an SM)
+static void eval_plan(int c, int r, int cw, int* JC, int* AT, size_t* smem) {
+  const size_t cap = cw == 1 ? EVAL_SMEM_MAX : EVAL2_SMEM_MAX;
   int jc = std::max(1, std::min(64, EVAL_THREADS / c)), at = 32;
   while (true) {
-    const size_t bytes = (size_t)eval_layout(jc, at, c, r).total * sizeof(double);
-    if (bytes <= EVAL_SMEM_MAX || (jc == 1 && at == 1)) { *JC = jc; *AT = at; *smem = bytes; return; }
-    if (at > 8) at /= 2;
+    const size_t bytes = (size_t)eval_layout(jc, at, c, r, cw).total * sizeof(double);
+    if (bytes <= cap || (jc == 1 && at == 1)) { *JC = jc; *AT = at; *smem = bytes; return; }
+    if (at > (cw == 1 ? 8 : 1)) at /= 2;
     else if (jc > 1) --jc;
     else at = std::max(1, at / 2);
   }
+}
+
+// Two-layer columns grow with k n c^2: a size the device cannot hold is refused here instead of failing inside cudaMalloc.
+// `held`: bytes of the buffer being grown, freed before the new allocation.
+static int check_fits(nnal_ctx* ctx, double want, double held, const char* what) {
+  size_t free_b = 0, total_b = 0;
+  CUDA_TRY(ctx, cudaMemGetInfo(&free_b, &total_b));
+  if (want > (double)free_b + held) {
+    char msg[256];
+    snprintf(msg, sizeof(msg), "two-layer block FI: %s need %.3g GB, %.3g GB of device memory free", what, want * 1e-9,
+             ((double)free_b + held) * 1e-9);
+    NNAL_FAIL(ctx, NNAL_ERR_UNSUPPORTED, msg);
+  }
+  return NNAL_OK;
 }
 
 static int setup(nnal_ctx* ctx, State* s) {
@@ -421,12 +624,34 @@ static int setup(nnal_ctx* ctx, State* s) {
   NNAL_TRY(grow(ctx, s->Lall, s->cap_L, n * c * r));
   NNAL_TRY(grow(ctx, s->Kd, s->cap_K, n * r * r));
   NNAL_TRY(grow(ctx, s->avail, s->cap_avail, n));
+  if (s->nl == 2) {
+    NNAL_TRY(check_fits(ctx, 8.0 * n * s->cw, 8.0 * s->cap_cd, "the candidates' own columns"));
+    NNAL_TRY(grow(ctx, s->Cd, s->cap_cd, n * s->cw));
+    NNAL_TRY(grow(ctx, s->Pw, s->cap_pw, (int64_t)s->d * s->nq));
+  }
   if (n == 0) return NNAL_OK;
-  setup_kernel<<<warp_grid(ctx, n), 256, 0, ctx->stream>>>(s->post, s->ldp, s->U, s->use_rows ? s->rows : nullptr, n, c, s->d,
-                                                           s->Lall, s->Kd, s->avail);
+  const int64_t* rows = s->use_rows ? s->rows : nullptr;
+  setup_kernel<<<warp_grid(ctx, n), 256, 0, ctx->stream>>>(s->post, s->ldp, s->U, rows, n, c, s->d, s->Lall, s->Kd, s->avail);
   ctx->launches++;
+  if (s->nl == 2) {
+    dots2_kernel<<<warp_grid(ctx, n), 256, 0, ctx->stream>>>(s->U, s->A, rows, n, s->d, s->dp, nullptr, 0, s->Cd, s->cw);
+    pw_kernel<<<flat_grid(ctx, (int64_t)s->d * s->nq), 256, 0, ctx->stream>>>(s->W3, s->U, rows, s->d, c, s->nq, nullptr, 0, s->Pw);
+    maskgemm_kernel<<<dim3((unsigned)((n + MG_J - 1) / MG_J), (unsigned)((s->nq + MG_Q - 1) / MG_Q)), 256, 0, ctx->stream>>>(
+        s->U, rows, n, s->d, s->nq, s->Pw, s->Cd, s->cw);
+    kd2_kernel<<<warp_grid(ctx, n), 256, 0, ctx->stream>>>(s->Lall, s->Cd, n, c, r, s->cw, s->Kd);
+    ctx->launches += 4;
+  }
   CUDA_TRY(ctx, cudaGetLastError());
   return NNAL_OK;
+}
+
+static void set_layers(State* s, int nl, int c, int dp, const float* A, const float* W3) {
+  s->nl = nl;
+  s->dp = nl == 2 ? dp : 0;
+  s->A = nl == 2 ? A : nullptr;
+  s->W3 = nl == 2 ? W3 : nullptr;
+  s->nq = c * (c + 1) / 2;
+  s->cw = nl == 2 ? s->nq + 2 : 1;
 }
 
 }  // namespace fib
@@ -435,18 +660,22 @@ int nnal_fi_block_release(nnal_ctx* ctx) {
   if (!ctx->fi_block_state) return NNAL_OK;
   fib::State* s = (fib::State*)ctx->fi_block_state;
   void* ptrs[] = {s->ownP, s->ownU, s->rows, s->Lall, s->Kd, s->avail, s->Scols, s->Kss, s->M, s->Z, s->Lsel, s->red, s->trC,
-                  s->sel, s->blk_loss, s->blk_idx, s->ticket};
+                  s->sel, s->blk_loss, s->blk_idx, s->ticket, s->ownA, s->ownW, s->Cd, s->Pw};
   for (void* p : ptrs) if (p) cudaFree(p);
   delete s;
   ctx->fi_block_state = nullptr;
   return NNAL_OK;
 }
 
-extern "C" int nnal_fi_block_set_candidates(nnal_ctx* ctx, const int64_t* cand, int64_t n_cand) {
+extern "C" int nnal_fi_block_set_candidates_nl(nnal_ctx* ctx, const int64_t* cand, int64_t n_cand, int n_layers) {
   if (!ctx || n_cand < 0) return NNAL_ERR_INVALID;
+  if (n_layers != 1 && n_layers != 2) NNAL_FAIL(ctx, NNAL_ERR_INVALID, "block FI covers the last 1 or 2 fully-connected layers");
   if (!ctx->pool_post || !ctx->pool_feat || ctx->keep < 1) NNAL_FAIL(ctx, NNAL_ERR_STATE, "pool pass did not keep the feature layer");
+  if (n_layers == 2 && (!ctx->pool_prev || ctx->keep < 2)) NNAL_FAIL(ctx, NNAL_ERR_STATE, "pool pass did not keep the previous FC output");
   if (ctx->n_class < 2 || ctx->n_class > fib::MAX_C) NNAL_FAIL(ctx, NNAL_ERR_UNSUPPORTED, "block FI supports 2 <= c <= 32");
   if (ctx->feature_layer != (int)ctx->layers.size() - 2) NNAL_FAIL(ctx, NNAL_ERR_UNSUPPORTED, "feature layer must feed the last FC layer");
+  if (n_layers == 2 && (ctx->feature_layer < 1 || ctx->layers[ctx->feature_layer - 1].type != NNAL_LAYER_FC))
+    NNAL_FAIL(ctx, NNAL_ERR_UNSUPPORTED, "two-layer block FI needs an FC layer before the feature layer");
   CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   const int64_t n = cand ? n_cand : ctx->pool_n;
   if (cand)
@@ -456,6 +685,7 @@ extern "C" int nnal_fi_block_set_candidates(nnal_ctx* ctx, const int64_t* cand, 
   s->have = false;
   s->n = n; s->c = ctx->n_class; s->r = ctx->n_class - 1; s->d = ctx->feat_dim;
   s->post = ctx->pool_post; s->ldp = ctx->pool_n; s->U = ctx->pool_feat;
+  fib::set_layers(s, n_layers, s->c, ctx->prev_dim, ctx->pool_prev, ctx->layers.back().W);
   s->use_rows = cand != nullptr;
   if (cand && n) {
     NNAL_TRY(fib::grow(ctx, s->rows, s->cap_rows, n));
@@ -467,8 +697,15 @@ extern "C" int nnal_fi_block_set_candidates(nnal_ctx* ctx, const int64_t* cand, 
   return NNAL_OK;
 }
 
-extern "C" int nnal_fi_block_set_factors(nnal_ctx* ctx, int64_t n, int c, int d, const float* post, const float* U) {
+extern "C" int nnal_fi_block_set_candidates(nnal_ctx* ctx, const int64_t* cand, int64_t n_cand) {
+  return nnal_fi_block_set_candidates_nl(ctx, cand, n_cand, 1);
+}
+
+extern "C" int nnal_fi_block_set_factors_nl(nnal_ctx* ctx, int64_t n, int c, int d, int d_prev, const float* post, const float* U,
+                                            const float* A_prev, const float* w_last) {
   if (!ctx || n < 0 || d <= 0 || (n > 0 && (!post || !U))) return NNAL_ERR_INVALID;
+  if ((A_prev != nullptr) != (w_last != nullptr) || (A_prev && d_prev <= 0))
+    NNAL_FAIL(ctx, NNAL_ERR_INVALID, "two-layer block FI needs both the previous activations and the last-layer weights");
   if (c < 2 || c > fib::MAX_C) NNAL_FAIL(ctx, NNAL_ERR_UNSUPPORTED, "block FI supports 2 <= c <= 32");
   CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   fib::State* s = fib::get(ctx);
@@ -480,11 +717,22 @@ extern "C" int nnal_fi_block_set_factors(nnal_ctx* ctx, int64_t n, int c, int d,
     CUDA_TRY(ctx, cudaMemcpyAsync(s->ownP, post, (size_t)n * c * 4, cudaMemcpyHostToDevice, ctx->stream));
     CUDA_TRY(ctx, cudaMemcpyAsync(s->ownU, U, (size_t)n * d * 4, cudaMemcpyHostToDevice, ctx->stream));
   }
+  if (A_prev) {
+    NNAL_TRY(fib::grow(ctx, s->ownA, s->cap_a, n * d_prev));
+    NNAL_TRY(fib::grow(ctx, s->ownW, s->cap_w, (int64_t)c * d));
+    if (n) CUDA_TRY(ctx, cudaMemcpyAsync(s->ownA, A_prev, (size_t)n * d_prev * 4, cudaMemcpyHostToDevice, ctx->stream));
+    CUDA_TRY(ctx, cudaMemcpyAsync(s->ownW, w_last, (size_t)c * d * 4, cudaMemcpyHostToDevice, ctx->stream));
+  }
   s->post = s->ownP; s->ldp = n; s->U = s->ownU; s->use_rows = false;
+  fib::set_layers(s, A_prev ? 2 : 1, c, d_prev, s->ownA, s->ownW);
   NNAL_TRY(fib::setup(ctx, s));
   CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
   s->have = true;
   return NNAL_OK;
+}
+
+extern "C" int nnal_fi_block_set_factors(nnal_ctx* ctx, int64_t n, int c, int d, const float* post, const float* U) {
+  return nnal_fi_block_set_factors_nl(ctx, n, c, d, 0, post, U, nullptr, nullptr);
 }
 
 extern "C" int nnal_fi_block_greedy(nnal_ctx* ctx, int64_t k, double delta, int64_t* sel_out, double* obj_out, double* red_out) {
@@ -492,19 +740,20 @@ extern "C" int nnal_fi_block_greedy(nnal_ctx* ctx, int64_t k, double delta, int6
   if (!ctx->fi_block_state || !((fib::State*)ctx->fi_block_state)->have) NNAL_FAIL(ctx, NNAL_ERR_STATE, "block FI candidates not set");
   fib::State* s = (fib::State*)ctx->fi_block_state;
   const int64_t n = s->n;
-  const int c = s->c, r = s->r;
+  const int c = s->c, r = s->r, cw = s->cw;
   if (k > n) k = n;
   if (k * r > fib::MAX_KR) NNAL_FAIL(ctx, NNAL_ERR_UNSUPPORTED, "block FI greedy supports k (c-1) <= 4096");
   if (k == 0) return NNAL_OK;
   CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   const int64_t mmax = k * r;
   const int npmax = (int)((mmax + 63) / 64 * 64);
-  const int64_t ldk = mmax, ldz = k * c, lds = n;
+  const int64_t ldk = mmax, ldz = k * c, lds = n * cw;    // column t of candidate j, entry e: Scols[t lds + j cw + e]
   int JC, AT;
   size_t smem;
-  fib::eval_plan(c, r, &JC, &AT, &smem);
+  fib::eval_plan(c, r, cw, &JC, &AT, &smem);
   const int nblk = (int)((n + JC - 1) / JC);
-  NNAL_TRY(fib::grow(ctx, s->Scols, s->cap_scols, k * n));
+  if (s->nl == 2) NNAL_TRY(fib::check_fits(ctx, 8.0 * k * lds, 8.0 * s->cap_scols, "the winners' columns"));
+  NNAL_TRY(fib::grow(ctx, s->Scols, s->cap_scols, k * lds));
   NNAL_TRY(fib::grow(ctx, s->Kss, s->cap_kss, mmax * mmax));
   NNAL_TRY(fib::grow(ctx, s->M, s->cap_m, (int64_t)npmax * npmax));
   NNAL_TRY(fib::grow(ctx, s->Z, s->cap_z, mmax * ldz));
@@ -520,7 +769,8 @@ extern "C" int nnal_fi_block_greedy(nnal_ctx* ctx, int64_t k, double delta, int6
   }
   static bool attr = false;
   if (!attr) {
-    CUDA_TRY(ctx, cudaFuncSetAttribute(fib::eval_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fib::EVAL_SMEM_MAX));
+    CUDA_TRY(ctx, cudaFuncSetAttribute(fib::eval_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fib::EVAL_SMEM_MAX));
+    CUDA_TRY(ctx, cudaFuncSetAttribute(fib::eval_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fib::EVAL_SMEM_MAX));
     attr = true;
   }
   CUDA_TRY(ctx, cudaMemsetAsync(s->avail, 1, (size_t)n, ctx->stream));
@@ -528,7 +778,7 @@ extern "C" int nnal_fi_block_greedy(nnal_ctx* ctx, int64_t k, double delta, int6
   const int64_t* rows = s->use_rows ? s->rows : nullptr;
   fib::EvalArgs ea;
   ea.Lall = s->Lall; ea.Kd = s->Kd; ea.Z = s->Z; ea.ldz = ldz; ea.Scols = s->Scols; ea.lds = lds;
-  ea.Lsel = s->Lsel; ea.avail = s->avail; ea.n = n; ea.c = c; ea.r = r; ea.JC = JC; ea.AT = AT;
+  ea.Lsel = s->Lsel; ea.avail = s->avail; ea.n = n; ea.c = c; ea.r = r; ea.JC = JC; ea.AT = AT; ea.cw = cw;
   ea.trC = s->trC; ea.blk_loss = s->blk_loss; ea.blk_idx = s->blk_idx; ea.ticket = s->ticket; ea.sel = s->sel; ea.red = s->red;
   for (int t = 0; t < (int)k; ++t) {
     const double alpha = (double)(t + 1) * delta;
@@ -536,8 +786,12 @@ extern "C" int nnal_fi_block_greedy(nnal_ctx* ctx, int64_t k, double delta, int6
       prof_begin(ctx, NNAL_PROF_FIB_SYSTEM);
       const int m = t * r;
       const int np = (m + 63) / 64 * 64;
-      fib::append_kernel<<<fib::flat_grid(ctx, (int64_t)t * r * r), 256, 0, ctx->stream>>>(s->Lsel, s->Scols, lds, s->sel, t - 1, c,
-                                                                                             r, s->Kss, ldk);
+      if (s->nl == 2)
+        fib::append2_kernel<<<fib::flat_grid(ctx, (int64_t)t * r * r), 256, 0, ctx->stream>>>(s->Lsel, s->Scols, lds, cw, s->sel,
+                                                                                                t - 1, c, r, s->Kss, ldk);
+      else
+        fib::append_kernel<<<fib::flat_grid(ctx, (int64_t)t * r * r), 256, 0, ctx->stream>>>(s->Lsel, s->Scols, lds, s->sel, t - 1,
+                                                                                               c, r, s->Kss, ldk);
       fib::build_kernel<<<fib::flat_grid(ctx, (int64_t)np * np), 256, 0, ctx->stream>>>(s->Kss, ldk, m, np, alpha, s->M);
       ctx->launches += 2;
       NNAL_TRY(nnal_gj64_invert(ctx, s->M, np));
@@ -549,13 +803,24 @@ extern "C" int nnal_fi_block_greedy(nnal_ctx* ctx, int64_t k, double delta, int6
     prof_begin(ctx, NNAL_PROF_FIB_EVAL);
     ea.t = t;
     ea.alpha = alpha;
-    fib::eval_kernel<<<nblk, fib::EVAL_THREADS, smem, ctx->stream>>>(ea);
+    if (s->nl == 2) fib::eval_kernel<2><<<nblk, fib::EVAL_THREADS, smem, ctx->stream>>>(ea);
+    else fib::eval_kernel<1><<<nblk, fib::EVAL_THREADS, smem, ctx->stream>>>(ea);
     ctx->launches++;
     prof_end(ctx);
     if (t + 1 < (int)k) {
       prof_begin(ctx, NNAL_PROF_FIB_COLUMN);
-      fib::column_kernel<<<fib::warp_grid(ctx, n), 256, 0, ctx->stream>>>(s->U, rows, n, s->d, s->sel, t, s->Scols + (int64_t)t * lds);
-      ctx->launches++;
+      double* col = s->Scols + (int64_t)t * lds;
+      if (s->nl == 2) {
+        fib::dots2_kernel<<<fib::warp_grid(ctx, n), 256, 0, ctx->stream>>>(s->U, s->A, rows, n, s->d, s->dp, s->sel, t, col, cw);
+        fib::pw_kernel<<<fib::flat_grid(ctx, (int64_t)s->d * s->nq), 256, 0, ctx->stream>>>(s->W3, s->U, rows, s->d, c, s->nq,
+                                                                                              s->sel, t, s->Pw);
+        fib::maskgemm_kernel<<<dim3((unsigned)((n + fib::MG_J - 1) / fib::MG_J), (unsigned)((s->nq + fib::MG_Q - 1) / fib::MG_Q)),
+                               256, 0, ctx->stream>>>(s->U, rows, n, s->d, s->nq, s->Pw, col, cw);
+        ctx->launches += 3;
+      } else {
+        fib::column_kernel<<<fib::warp_grid(ctx, n), 256, 0, ctx->stream>>>(s->U, rows, n, s->d, s->sel, t, col);
+        ctx->launches++;
+      }
       prof_end(ctx);
     }
     CUDA_TRY(ctx, cudaGetLastError());
@@ -565,7 +830,7 @@ extern "C" int nnal_fi_block_greedy(nnal_ctx* ctx, int64_t k, double delta, int6
   CUDA_TRY(ctx, cudaMemcpyAsync(sel_out, s->sel, (size_t)k * 8, cudaMemcpyDeviceToHost, ctx->stream));
   CUDA_TRY(ctx, cudaMemcpyAsync(red.data(), s->red, (size_t)k * 8, cudaMemcpyDeviceToHost, ctx->stream));
   CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-  const double D = (double)c * (s->d + 1.0);
+  const double D = (double)c * (s->d + 1.0) + (s->nl == 2 ? (double)s->d * (s->dp + 1.0) : 0.0);
   for (int64_t t = 0; t < k; ++t) {
     if (red_out) red_out[t] = red[t];
     if (obj_out) obj_out[t] = (D - (double)(t + 1) * r) / delta + red[t];

@@ -509,27 +509,42 @@ class Engine(object):
         self._chk(self.lib.nnal_fi_greedy(self.h, k, float(delta), _ptr(sel), _ptr(obj), _ptr(red)))
         return sel, obj, red
 
-    def fi_block_set_candidates(self, cand=None):
-        """Multi-class block-form FI (last FC layer): candidates = pool positions ``cand`` (None: every pool sample) of
-        the current pool pass, which must have kept the feature layer."""
+    def fi_block_set_candidates(self, cand=None, n_layers=1):
+        """Multi-class block-form FI over the last ``n_layers`` (1 or 2) FC layers: candidates = pool positions ``cand``
+        (None: every pool sample) of the current pool pass, which must have kept the feature layer (and, for two layers,
+        the previous FC output: ``keep >= 2``)."""
         if cand is None:
-            self._chk(self.lib.nnal_fi_block_set_candidates(self.h, None, 0))
+            self._chk(self.lib.nnal_fi_block_set_candidates_nl(self.h, None, 0, int(n_layers)))
             self._fi_block_n = self._pool_n
         else:
             cand = np.ascontiguousarray(cand, dtype=np.int64).ravel()
             self.h2d_bytes += cand.nbytes
-            self._chk(self.lib.nnal_fi_block_set_candidates(self.h, _ptr(cand) if cand.size else None, cand.size))
+            self._chk(self.lib.nnal_fi_block_set_candidates_nl(self.h, _ptr(cand) if cand.size else None, cand.size,
+                                                               int(n_layers)))
             self._fi_block_n = cand.size
 
-    def fi_block_set_factors(self, post, U):
-        """Multi-class block-form FI candidates from host factors: ``post`` [c,n] posteriors, ``U`` [n,d] features."""
+    def fi_block_set_factors(self, post, U, A_prev=None, w_last=None):
+        """Multi-class block-form FI candidates from host factors: ``post`` [c,n] posteriors, ``U`` [n,d] features; for
+        the last two FC layers also ``A_prev`` [n,d_prev] (input of the feature layer's FC) and ``w_last`` [c,d] (last FC
+        weights), both or neither."""
         post = np.ascontiguousarray(post, dtype=np.float32)
         U = np.ascontiguousarray(U, dtype=np.float32)
         if post.ndim != 2 or U.ndim != 2 or post.shape[1] != U.shape[0]:
             raise ValueError('post must be [c,n] and U [n,d] for the same n')
         c, n = post.shape
+        d = U.shape[1]
+        if (A_prev is None) != (w_last is None):
+            raise ValueError('two-layer FI needs both A_prev and w_last')
+        if A_prev is not None:
+            A_prev = np.ascontiguousarray(A_prev, dtype=np.float32)
+            w_last = np.ascontiguousarray(w_last, dtype=np.float32)
+            if A_prev.ndim != 2 or A_prev.shape[0] != n or A_prev.shape[1] < 1 or w_last.shape != (c, d):
+                raise ValueError('A_prev must be [n,d_prev] and w_last [c,d]')
+            self.h2d_bytes += A_prev.nbytes + w_last.nbytes
         self.h2d_bytes += post.nbytes + U.nbytes
-        self._chk(self.lib.nnal_fi_block_set_factors(self.h, n, c, U.shape[1], _ptr(post), _ptr(U)))
+        self._chk(self.lib.nnal_fi_block_set_factors_nl(self.h, n, c, d, 0 if A_prev is None else A_prev.shape[1], _ptr(post),
+                                                        _ptr(U), None if A_prev is None else _ptr(A_prev),
+                                                        None if A_prev is None else _ptr(w_last)))
         self._fi_block_n = n
 
     def fi_block_greedy(self, k, delta):
@@ -737,6 +752,17 @@ class Engine(object):
         self.d2h_bytes += out.nbytes
         self._chk(self.lib.nnal_pool_feature_rows(self.h, _ptr(pos) if pos.size else None, pos.size,
                                                   _ptr(out) if pos.size else None))
+        return out
+
+    def pool_prev_rows(self, pos):
+        """Rows of the previous FC layer's output (input of the feature layer's FC) at pool positions ``pos`` as
+        ``[len(pos), prev_dim]`` float32; the pool pass must have kept it (``keep >= 2``)."""
+        pos = np.ascontiguousarray(pos, dtype=np.int64).ravel()
+        out = np.empty((pos.size, self.prev_dim), dtype=np.float32)
+        self.h2d_bytes += pos.nbytes
+        self.d2h_bytes += out.nbytes
+        self._chk(self.lib.nnal_pool_prev_rows(self.h, _ptr(pos) if pos.size else None, pos.size,
+                                               _ptr(out) if pos.size else None))
         return out
 
     def rep_set(self, cols, excl_pos, k):

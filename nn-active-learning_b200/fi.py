@@ -593,29 +593,39 @@ def query_whole(model, expr, pool_inds, session):
 
 
 def query_whole_block(model, expr, pool_inds, session, return_objective=False):
-    """``NNAL.CNN_query(..., 'fi')`` with ``expr.pars['fi_mode'] = 'block-greedy'``: greedy minimisation of the last-layer
-    FI objective ``tr((sum_{i in S} F_i/|S| + delta I)^-1)`` for any number of classes c >= 2 (c <= 32, k (c-1) <= 4096),
-    ``F_i = (diag pi_i - pi_i pi_i^T) (x) [u_i;1][u_i;1]^T`` (NN.LLFC_hess, NN.py:891-901), in the block form of
-    csrc/fi_block.cu.  Entropy pre-filter to B exactly as ``query_whole``, then the greedy over ``min(k, B)`` steps.
-    Keys read: ``k``, ``B``, ``fi_diag_load`` (default 1e-5); ``fi_layers`` is ignored (last FC layer only, as in
-    ``query_whole``).  Returns positions into ``pool_inds`` in selection order (and, with ``return_objective``, the
-    objective and its kernel-dependent part per step).
+    """``NNAL.CNN_query(..., 'fi')`` with ``expr.pars['fi_mode'] = 'block-greedy'``: greedy minimisation of the FI
+    objective ``tr((sum_{i in S} F_i/|S| + delta I)^-1)`` for any number of classes c >= 2 (c <= 32, k (c-1) <= 4096) in
+    the block form of csrc/fi_block.cu.  ``expr.pars['fi_layers']`` (default 1) picks the parameters: 1 = the last FC
+    layer, ``F_i = (diag pi_i - pi_i pi_i^T) (x) [u_i;1][u_i;1]^T`` (NN.LLFC_hess, NN.py:891-901); 2 = the last two FC
+    layers, as the binary path's default, adding the score ``(M_i W3^T (e_y - pi_i)) (x) [a_i;1]`` of the previous FC
+    layer (M_i = diag 1[u_i > 0], a_i its input).  Entropy pre-filter to B exactly as ``query_whole``, then the greedy
+    over ``min(k, B)`` steps.  Keys read: ``k``, ``B``, ``fi_diag_load`` (default 1e-5), ``fi_layers`` (1 or 2; anything
+    else raises ValueError).  Returns positions into ``pool_inds`` in selection order (and, with ``return_objective``,
+    the objective and its kernel-dependent part per step).
 
-    Several ranks: every rank reads its own candidates' posteriors and feature rows, the B candidates are all-gathered and
-    put in pre-filter order on every rank, and every rank runs the same deterministic greedy on them."""
+    Several ranks: every rank reads its own candidates' posteriors and feature rows (and, for two layers, the previous FC
+    output), the B candidates are all-gathered and put in pre-filter order on every rank, and every rank runs the same
+    deterministic greedy on them."""
     from .NNAL import _posteriors_on_device
     k, B = int(expr.pars['k']), int(expr.pars['B'])
     delta = float(expr.pars.get('fi_diag_load', 1e-5))
+    nl = expr.pars.get('fi_layers', 1)
+    if nl not in (1, 2):
+        raise ValueError("fi_layers must be 1 or 2 for fi_mode='block-greedy', got %r" % (nl,))
+    nl = int(nl)
     pool_inds = np.asarray(pool_inds)
     n = len(pool_inds)
-    eng, lo, hi = _posteriors_on_device(model, expr, pool_inds, session, keep=1)
+    eng, lo, hi = _posteriors_on_device(model, expr, pool_inds, session, keep=nl)
     if B < n:
         eng.pool_score(L.SCORE_NEG_ENTROPY, 1e-8)
         sel_inds, _ = dist.topk_global(eng, B, lo, n)
     else:
         sel_inds = np.arange(n, dtype=np.int64)
     if not dist.is_dist():
-        eng.fi_block_set_candidates(sel_inds - lo)
+        if nl == 1:
+            eng.fi_block_set_candidates(sel_inds - lo)
+        else:
+            eng.fi_block_set_candidates(sel_inds - lo, nl)
     else:
         own = (sel_inds >= lo) & (sel_inds < hi)
         rows = sel_inds[own] - lo
@@ -628,7 +638,14 @@ def query_whole_block(model, expr, pool_inds, session, return_objective=False):
         Fg = dist.allgather_concat(np.ascontiguousarray(F, dtype=np.float32).ravel()).reshape(-1, d)
         order = np.argsort(gpos, kind='stable')
         perm = order[np.searchsorted(gpos[order], sel_inds)]          # gathered row of every candidate, pre-filter order
-        eng.fi_block_set_factors(P[perm].T, Fg[perm])
+        if nl == 1:
+            eng.fi_block_set_factors(P[perm].T, Fg[perm])
+        else:
+            A = eng.pool_prev_rows(rows)
+            Ag = dist.allgather_concat(np.ascontiguousarray(A, dtype=np.float32).ravel()).reshape(-1, A.shape[1])
+            layers = list(model.layer_dict.items()) if isinstance(model.layer_dict, dict) else list(model.layer_dict)
+            W3 = np.asarray(model.get_weights(session)[layers[-1][0]][0], dtype=np.float32)     # [c, d]
+            eng.fi_block_set_factors(P[perm].T, Fg[perm], Ag[perm], W3)
     chosen, obj, red = eng.fi_block_greedy(min(k, len(sel_inds)), delta)
     q = sel_inds[chosen]
     if return_objective == 'reduced':
