@@ -57,6 +57,10 @@ typedef struct { int32_t type, out, kh, kw; } nnal_layer_spec;
 #define NNAL_SCORE_MC_BINARY 10 /* |mean_t P_t(class1) - 0.5| over the MC-dropout passes (PW_NNAL.py:67-87, 232-244) */
 #define NNAL_SCORE_NEG_BALD 11  /* -(H(mean_t P_t) - mean_t H(P_t)), zeros bumped by 1e-6 (PW_NNAL.py:247-282): ascending
                                    top-k of it = np.argsort(-scores)[:k] */
+/* The same two scorers for any 2 <= c <= 32 classes, H = -sum_j p_j log p_j over the running means of every class (zeros
+ * bumped by 1e-6).  At c = 2 they are computed from the binary running means with P(class 0) = 1 - P(class 1). */
+#define NNAL_SCORE_MC_NEG_ENTROPY 12 /* -H(mean_t P_t): predictive entropy, k largest (MC-entropy / ensemble) */
+#define NNAL_SCORE_MC_NEG_BALD 13    /* -(H(mean_t P_t) - mean_t H(P_t)): k largest mutual information (BALD / QBC-JS) */
 
 /* ---- context ------------------------------------------------------------------------------- */
 int nnal_version(void);
@@ -147,19 +151,25 @@ int nnal_pool_eval_device_inds(nnal_ctx* ctx, int subject, const int64_t* d_inds
 /* MC-dropout (replaces feeding x_feed_dict = {model.keep_prob: model.dropout_rate} to PW_NN.batch_eval T times,
  * PW_NNAL.py:67-87, 232-282).  Configure BEFORE nnal_pool_begin; the following nnal_pool_eval* calls evaluate the conv
  * trunk once per chunk and the FC tail T times with tf.nn.dropout semantics (x / keep_prob where kept, NN.py:167-171)
- * on the outputs of `layers` (model.dropout_layers: FC layers only), keeping float64 running means of P(class 1) and of
- * the per-pass binary entropies for every pool sample.  Masks are Philox4x32-10 words keyed by `seed`, counter
- * {unit/4, pos0 + pool position, first_pass + t, layer}: independent of chunking and of how the pool is sharded.
- * T = 0 switches MC mode off.  Binary models only. */
+ * on the outputs of `layers` (model.dropout_layers: FC layers only), keeping float64 running means of the posteriors and
+ * of the per-pass entropies for every pool sample (c = 2: of P(class 1) and the binary entropy; 3 <= c <= 32: of every
+ * class).  Masks are Philox4x32-10 words keyed by `seed`, counter {unit/4, pos0 + pool position, first_pass + t, layer}:
+ * independent of chunking and of how the pool is sharded.  T = 0 switches MC mode off.  NNAL_ERR_UNSUPPORTED for more
+ * than 32 classes or when a hidden FC layer does not run on the tensor-core path. */
 int nnal_pool_mc_config(nnal_ctx* ctx, int T, double keep_prob, unsigned long long seed, unsigned int first_pass,
                         long long pos0, const int* layers, int n_layers);
 /* Committee scorers 'ensemble' / 'QBC-JS' (PW_NNAL.py:453-545): fold member t's deterministic pool pass (the current
  * posteriors) into the same running means, av = (x + t av) / (t + 1).  t = 0 opens the accumulation,
- * nnal_pool_ensemble_end closes it; every member scores the same pool.  Scores: NNAL_SCORE_MC_BINARY / _NEG_BALD. */
+ * nnal_pool_ensemble_end closes it; every member scores the same pool.  2 <= c <= 32.  Scores: NNAL_SCORE_MC_BINARY /
+ * _NEG_BALD (c = 2), NNAL_SCORE_MC_NEG_ENTROPY / _MC_NEG_BALD (any c). */
 int nnal_pool_ensemble_accumulate(nnal_ctx* ctx, int t);
 int nnal_pool_ensemble_end(nnal_ctx* ctx);
-/* running means after the pool pass: av_post [n_total], av_ent [n_total] (either may be NULL) */
+/* binary running means after the pool pass: av_post [n_total] of P(class 1), av_ent [n_total] (either may be NULL);
+ * NNAL_ERR_INVALID for c != 2 */
 int nnal_pool_mc_read(nnal_ctx* ctx, double* av_post, double* av_ent);
+/* running means of every class: av_post [c][n_total], av_ent [n_total] (either may be NULL).  At c = 2 row 0 is
+ * 1 - row 1, the complement the binary scores use. */
+int nnal_pool_mc_read_classes(nnal_ctx* ctx, double* av_post, double* av_ent);
 /* posteriors [c][n_total] float32 (layout of model.posteriors, NN.py:184-188) */
 int nnal_pool_posteriors(nnal_ctx* ctx, float* out);
 /* model.feature_layer as [feat_dim][n] columns start..start+n (PW_NN.py:530-531 layout) */

@@ -15,7 +15,9 @@ def _pool_images(expr, pool_inds):
     return np.asarray(expr.pool_images[np.asarray(pool_inds)], dtype=np.float32)
 
 
-def _posteriors_on_device(model, expr, pool_inds, session, keep=0):
+def _posteriors_on_device(model, expr, pool_inds, session, keep=0, mc=None):
+    """Pool pass over this rank's block [lo, hi) of the pool.  ``mc = (T, keep_prob)`` runs T MC-dropout passes of the
+    FC tail; the masks are keyed by global pool position (pos0 = lo), so they do not depend on the sharding."""
     eng = get_engine()
     eng.set_model(model, session)
     pool_inds = np.asarray(pool_inds)
@@ -23,8 +25,14 @@ def _posteriors_on_device(model, expr, pool_inds, session, keep=0):
     rank, world = dist.rank_world()
     b = dist.shard_bounds(n, world)
     lo, hi = int(b[rank]), int(b[rank + 1])
-    eng.pool_begin(hi - lo, keep)
-    eng.pool_eval_images(_pool_images(expr, pool_inds[lo:hi]), 0)
+    if mc is not None:
+        eng.pool_mc_config(mc[0], mc[1], model.dropout_layers, pos0=lo)
+    try:
+        eng.pool_begin(hi - lo, keep)
+        eng.pool_eval_images(_pool_images(expr, pool_inds[lo:hi]), 0)
+    finally:
+        if mc is not None:
+            eng.pool_mc_config(0, 1., [])
     return eng, lo, hi
 
 
@@ -35,7 +43,15 @@ def CNN_query(model, expr, pool_inds, method_name, session, col=True, extra_feed
     (NNAL.py:298-310).  ``fi``: see ``nnal_b200.fi.query_whole``; ``expr.pars['fi_mode'] = 'sdp'`` runs the reference's
     own multiclass A-matrix + SDP + sampling pipeline (``nnal_b200.fi.query_whole_sdp``); ``'block-greedy'`` runs the greedy
     FI selection for any number of classes (``nnal_b200.fi.query_whole_block``) over the last FC layer, or over the last two
-    with ``expr.pars['fi_layers'] = 2``."""
+    with ``expr.pars['fi_layers'] = 2``.
+
+    Bayesian and committee scorers, for 2 <= c <= 32 classes (the binary definitions of PW_NNAL.py:67-87, 247-282 and
+    :453-545 extended to c classes; ties go to the lowest position):
+    ``MC-entropy`` / ``BALD``: ``expr.pars['MC_iters']`` MC-dropout passes at ``model.dropout_rate`` on
+    ``model.dropout_layers`` (FC layers; the conv trunk runs once), float64 running means of every class posterior and of
+    the per-pass entropies; k largest predictive entropies H(mean p), resp. k largest H(mean p) - mean H(p).
+    ``ensemble`` / ``QBC-JS``: the same two scores over a committee, the weights of ``expr.pretrained_paths`` loaded into
+    ``expr.model_holder`` one after the other (``perform_assign_ops``), each evaluated deterministically."""
     k = expr.pars['k']
     if method_name == 'random':
         return np.random.permutation(len(pool_inds))[:k]
@@ -53,6 +69,25 @@ def CNN_query(model, expr, pool_inds, method_name, session, col=True, extra_feed
         if expr.pars.get('fi_mode', 'greedy') == 'block-greedy':
             return fi.query_whole_block(model, expr, pool_inds, session)
         return fi.query_whole(model, expr, pool_inds, session)
+    if method_name in ('MC-entropy', 'BALD'):
+        eng, lo, hi = _posteriors_on_device(model, expr, pool_inds, session,
+                                            mc=(int(expr.pars['MC_iters']), float(model.dropout_rate)))
+        eng.pool_score(L.SCORE_MC_NEG_ENTROPY if method_name == 'MC-entropy' else L.SCORE_MC_NEG_BALD)
+        q, _ = dist.topk_global(eng, k, lo, len(pool_inds))
+        return q
+    if method_name in ('ensemble', 'QBC-JS'):
+        eng = None
+        try:
+            for i, path in enumerate(expr.pretrained_paths):
+                expr.model_holder.perform_assign_ops(path, session)
+                eng, lo, hi = _posteriors_on_device(expr.model_holder, expr, pool_inds, session)
+                eng.pool_ensemble_accumulate(i)
+        finally:
+            if eng is not None:
+                eng.pool_ensemble_end()
+        eng.pool_score(L.SCORE_MC_NEG_ENTROPY if method_name == 'ensemble' else L.SCORE_MC_NEG_BALD)
+        q, _ = dist.topk_global(eng, k, lo, len(pool_inds))
+        return q
     if method_name == 'rep-entropy':
         from . import rep
         return rep.query_rep_entropy_whole(model, expr, pool_inds, session)

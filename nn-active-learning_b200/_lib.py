@@ -52,6 +52,7 @@ SIGNATURES = {
     'nnal_pool_score': (C.c_int, [c_vp, C.c_int, C.c_double]),
     'nnal_pool_mc_config': (C.c_int, [c_vp, C.c_int, C.c_double, C.c_ulonglong, C.c_uint, C.c_longlong, c_vp, C.c_int]),
     'nnal_pool_mc_read': (C.c_int, [c_vp, c_vp, c_vp]),
+    'nnal_pool_mc_read_classes': (C.c_int, [c_vp, c_vp, c_vp]),
     'nnal_pool_ensemble_accumulate': (C.c_int, [c_vp, C.c_int]),
     'nnal_pool_ensemble_end': (C.c_int, [c_vp]),
     'nnal_pool_scores_read': (C.c_int, [c_vp, c_vp]),
@@ -125,6 +126,7 @@ F32, F64 = 0, 1
 NORM_NONE, NORM_BATCH_EVAL, NORM_MULTIMG = 0, 1, 2
 SCORE_BINARY, SCORE_NEG_ENTROPY, SCORE_ENTROPY, SCORE_NEG_FI_TRACE = 0, 1, 2, 3
 SCORE_MC_BINARY, SCORE_NEG_BALD = 10, 11
+SCORE_MC_NEG_ENTROPY, SCORE_MC_NEG_BALD = 12, 13
 
 _lib = None
 

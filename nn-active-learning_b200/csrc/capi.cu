@@ -608,6 +608,26 @@ extern "C" int nnal_entropy_device_f32(nnal_ctx* ctx, const float* d_post, int c
 // ---------------------------------------------------------------------------------------------
 // pool pass
 // ---------------------------------------------------------------------------------------------
+// MC-dropout and committee statistics: c = 2 keeps the binary running means (P(class 1), PW_NNAL.py:80); 3 <= c <= 32
+// keeps the running mean of every class.
+static int check_mc_classes(nnal_ctx* ctx) {
+  if (ctx->n_class < 2 || ctx->n_class > 32)
+    NNAL_FAIL(ctx, NNAL_ERR_UNSUPPORTED, "MC-dropout and committee scores need 2 to 32 classes");
+  return NNAL_OK;
+}
+// Running-mean storage for n pool samples; free_pool resets the capacity when the class count changes.
+static int reserve_mc(nnal_ctx* ctx, int64_t n) {
+  if ((size_t)n <= ctx->pool_cap_mc) return NNAL_OK;
+  const size_t rows = ctx->n_class == 2 ? 1 : (size_t)ctx->n_class;
+  if (ctx->pool_mc_post) { CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream)); cudaFree(ctx->pool_mc_post); cudaFree(ctx->pool_mc_ent); }
+  ctx->pool_mc_post = ctx->pool_mc_ent = nullptr;
+  ctx->pool_cap_mc = 0;
+  CUDA_TRY(ctx, cudaMalloc(&ctx->pool_mc_post, (size_t)n * rows * sizeof(double)));
+  CUDA_TRY(ctx, cudaMalloc(&ctx->pool_mc_ent, (size_t)n * sizeof(double)));
+  ctx->pool_cap_mc = (size_t)n;
+  return NNAL_OK;
+}
+
 extern "C" int nnal_pool_begin(nnal_ctx* ctx, int64_t n_total, int keep) {
   if (!ctx || n_total < 0 || keep < 0 || keep > 2) return NNAL_ERR_INVALID;
   if (ctx->layers.empty()) NNAL_FAIL(ctx, NNAL_ERR_STATE, "model not set");
@@ -636,14 +656,8 @@ extern "C" int nnal_pool_begin(nnal_ctx* ctx, int64_t n_total, int keep) {
   if (keep >= 2) NNAL_TRY(grow((void**)&ctx->pool_prev, ctx->pool_cap_nprev, (size_t)ctx->prev_dim * sizeof(float)));
   if (ctx->mc_T > 0) {
     if (keep != 0) NNAL_FAIL(ctx, NNAL_ERR_INVALID, "MC-dropout passes do not keep features");
-    if (ctx->n_class != 2) NNAL_FAIL(ctx, NNAL_ERR_UNSUPPORTED, "MC-dropout scores are defined for the binary patch model");
-    if ((size_t)n_total > ctx->pool_cap_mc) {
-      if (ctx->pool_mc_post) { CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream)); cudaFree(ctx->pool_mc_post); cudaFree(ctx->pool_mc_ent); }
-      ctx->pool_mc_post = ctx->pool_mc_ent = nullptr;
-      CUDA_TRY(ctx, cudaMalloc(&ctx->pool_mc_post, (size_t)n_total * sizeof(double)));
-      CUDA_TRY(ctx, cudaMalloc(&ctx->pool_mc_ent, (size_t)n_total * sizeof(double)));
-      ctx->pool_cap_mc = (size_t)n_total;
-    }
+    NNAL_TRY(check_mc_classes(ctx));
+    NNAL_TRY(reserve_mc(ctx, n_total));
   }
   if (!ctx->ens_open) ctx->mc_have = ctx->mc_T > 0;
   ctx->pool_n = n_total;
@@ -660,6 +674,10 @@ extern "C" int nnal_pool_mc_config(nnal_ctx* ctx, int T, double keep_prob, unsig
   if (T == 0) return NNAL_OK;
   if (!(keep_prob > 0.0 && keep_prob <= 1.0) || n_layers < 0 || (n_layers > 0 && !layers)) NNAL_FAIL(ctx, NNAL_ERR_INVALID, "keep_prob must be in (0, 1]");
   if (ctx->fc_first < 0) NNAL_FAIL(ctx, NNAL_ERR_STATE, "model not set");
+  NNAL_TRY(check_mc_classes(ctx));
+  for (int j = ctx->fc_first; j < (int)ctx->layers.size() - 1; ++j)
+    if (!nnal_layer_on_tc(ctx, j))
+      NNAL_FAIL(ctx, NNAL_ERR_UNSUPPORTED, "MC-dropout: the hidden FC layers must run on the tensor-core path");
   ctx->mc_sites.clear();
   for (int i = 0; i < n_layers; ++i) {
     if (layers[i] < ctx->fc_first || layers[i] >= (int)ctx->layers.size())
@@ -685,18 +703,17 @@ extern "C" int nnal_pool_mc_config(nnal_ctx* ctx, int T, double keep_prob, unsig
 extern "C" int nnal_pool_ensemble_accumulate(nnal_ctx* ctx, int t) {
   if (!ctx || t < 0) return NNAL_ERR_INVALID;
   if (!ctx->pool_post || ctx->pool_n <= 0) NNAL_FAIL(ctx, NNAL_ERR_STATE, "no pool pass");
-  if (ctx->n_class != 2) NNAL_FAIL(ctx, NNAL_ERR_UNSUPPORTED, "committee scores are defined for the binary patch model");
+  NNAL_TRY(check_mc_classes(ctx));
   if (t > 0 && !ctx->ens_open) NNAL_FAIL(ctx, NNAL_ERR_STATE, "committee accumulation starts with member 0");
   CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   if ((size_t)ctx->pool_n > ctx->pool_cap_mc) {
     if (t > 0) NNAL_FAIL(ctx, NNAL_ERR_STATE, "committee members must score the same pool");
-    if (ctx->pool_mc_post) { CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream)); cudaFree(ctx->pool_mc_post); cudaFree(ctx->pool_mc_ent); }
-    ctx->pool_mc_post = ctx->pool_mc_ent = nullptr;
-    CUDA_TRY(ctx, cudaMalloc(&ctx->pool_mc_post, (size_t)ctx->pool_n * sizeof(double)));
-    CUDA_TRY(ctx, cudaMalloc(&ctx->pool_mc_ent, (size_t)ctx->pool_n * sizeof(double)));
-    ctx->pool_cap_mc = (size_t)ctx->pool_n;
+    NNAL_TRY(reserve_mc(ctx, ctx->pool_n));
   }
-  NNAL_TRY(nnal_k_mc_accumulate(ctx, ctx->pool_post, ctx->pool_n, 0, ctx->pool_n, t, ctx->pool_mc_post, ctx->pool_mc_ent));
+  prof_begin(ctx, NNAL_PROF_MC_ACCUM);
+  NNAL_TRY(nnal_k_mc_accumulate(ctx, ctx->pool_post, ctx->n_class, ctx->pool_n, 0, ctx->pool_n, t, ctx->pool_mc_post,
+                                ctx->pool_mc_ent));
+  prof_end(ctx);
   ctx->ens_open = 1;
   ctx->mc_have = 1;
   return NNAL_OK;
@@ -710,10 +727,27 @@ extern "C" int nnal_pool_ensemble_end(nnal_ctx* ctx) {
 extern "C" int nnal_pool_mc_read(nnal_ctx* ctx, double* av_post, double* av_ent) {
   if (!ctx) return NNAL_ERR_INVALID;
   if (!ctx->pool_mc_post || !ctx->mc_have) NNAL_FAIL(ctx, NNAL_ERR_STATE, "no MC-dropout pass has run");
+  if (ctx->n_class != 2) NNAL_FAIL(ctx, NNAL_ERR_INVALID, "binary running means need a 2-class model (nnal_pool_mc_read_classes)");
   CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   if (av_post) CUDA_TRY(ctx, cudaMemcpyAsync(av_post, ctx->pool_mc_post, (size_t)ctx->pool_n * 8, cudaMemcpyDeviceToHost, ctx->stream));
   if (av_ent) CUDA_TRY(ctx, cudaMemcpyAsync(av_ent, ctx->pool_mc_ent, (size_t)ctx->pool_n * 8, cudaMemcpyDeviceToHost, ctx->stream));
   NNAL_SYNC_CHECKED(ctx);
+  return NNAL_OK;
+}
+
+extern "C" int nnal_pool_mc_read_classes(nnal_ctx* ctx, double* av_post, double* av_ent) {
+  if (!ctx) return NNAL_ERR_INVALID;
+  if (!ctx->pool_mc_post || !ctx->mc_have) NNAL_FAIL(ctx, NNAL_ERR_STATE, "no MC-dropout pass has run");
+  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  const size_t n = (size_t)ctx->pool_n;
+  const bool binary = ctx->n_class == 2;
+  // c = 2 keeps P(class 1) only: it goes to row 1, and row 0 is 1 - row 1 as the binary scores take it
+  if (av_post) CUDA_TRY(ctx, cudaMemcpyAsync(binary ? av_post + n : av_post, ctx->pool_mc_post, (binary ? n : n * ctx->n_class) * 8,
+                                             cudaMemcpyDeviceToHost, ctx->stream));
+  if (av_ent) CUDA_TRY(ctx, cudaMemcpyAsync(av_ent, ctx->pool_mc_ent, n * 8, cudaMemcpyDeviceToHost, ctx->stream));
+  NNAL_SYNC_CHECKED(ctx);
+  if (av_post && binary)
+    for (size_t i = 0; i < n; ++i) av_post[i] = 1.0 - av_post[n + i];
   return NNAL_OK;
 }
 
@@ -895,11 +929,14 @@ extern "C" int nnal_pool_prev_rows(nnal_ctx* ctx, const int64_t* pos, int64_t n,
 extern "C" int nnal_pool_score(nnal_ctx* ctx, int kind, double eps) {
   if (!ctx) return NNAL_ERR_INVALID;
   if (!ctx->pool_post) NNAL_FAIL(ctx, NNAL_ERR_STATE, "no pool pass");
-  if (kind == NNAL_SCORE_MC_BINARY || kind == NNAL_SCORE_NEG_BALD) {
+  if (kind == NNAL_SCORE_MC_BINARY || kind == NNAL_SCORE_NEG_BALD || kind == NNAL_SCORE_MC_NEG_ENTROPY ||
+      kind == NNAL_SCORE_MC_NEG_BALD) {
+    if (kind < NNAL_SCORE_MC_NEG_ENTROPY && ctx->n_class != 2)
+      NNAL_FAIL(ctx, NNAL_ERR_INVALID, "binary MC scores need a 2-class model (NNAL_SCORE_MC_NEG_ENTROPY / _MC_NEG_BALD)");
     if (!ctx->pool_mc_post || !ctx->mc_have) NNAL_FAIL(ctx, NNAL_ERR_STATE, "MC scores need an MC-dropout pool pass");
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     prof_begin(ctx, NNAL_PROF_SCORE);
-    int rc = nnal_k_scores_mc(ctx, ctx->pool_mc_post, ctx->pool_mc_ent, ctx->pool_n, kind, ctx->pool_score);
+    int rc = nnal_k_scores_mc(ctx, ctx->pool_mc_post, ctx->pool_mc_ent, ctx->n_class, ctx->pool_n, kind, ctx->pool_score);
     prof_end(ctx);
     return rc;
   }

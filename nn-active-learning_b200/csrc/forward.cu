@@ -100,8 +100,10 @@ int nnal_forward_chunk(nnal_ctx* ctx, int64_t nb, int64_t offset, int input_form
     if (ctx->mc_T > 0 && i == ctx->fc_first) {
       // MC-dropout: the conv trunk is deterministic (PW1 drops out the FC outputs only, NN.py:1338) and was computed
       // once; the FC tail runs T times with fresh masks.  The tail ping-pongs between the activation buffer that does
-      // not hold the trunk output and a third buffer.
-      if (!cur.split) NNAL_FAIL(ctx, NNAL_ERR_UNSUPPORTED, "MC-dropout needs the tensor-core path (trunk output in split planes)");
+      // not hold the trunk output and a third buffer.  The trunk's last layer writes the split planes the tail's first
+      // FC layer takes, on either path; an FC-only net's fp32 input is split once here, not once per pass.
+      if (i < nl - 1) NNAL_TRY(to_split(cur));
+      else NNAL_TRY(to_f32(cur));
       size_t maxfc = 0;
       for (int j = i; j < nl; ++j) maxfc = std::max(maxfc, (size_t)ctx->layers[j].out_dim);
       NNAL_TRY(devbuf_reserve(ctx, ctx->act_mc, (size_t)nb * maxfc * sizeof(float)));
@@ -135,7 +137,10 @@ int nnal_forward_chunk(nnal_ctx* ctx, int64_t nb, int64_t offset, int input_form
           }
           prof_end(ctx);
         }
-        NNAL_TRY(nnal_k_mc_accumulate(ctx, ctx->pool_post, ctx->pool_n, offset, nb, t, ctx->pool_mc_post, ctx->pool_mc_ent));
+        prof_begin(ctx, NNAL_PROF_MC_ACCUM);
+        NNAL_TRY(nnal_k_mc_accumulate(ctx, ctx->pool_post, ctx->n_class, ctx->pool_n, offset, nb, t, ctx->pool_mc_post,
+                                      ctx->pool_mc_ent));
+        prof_end(ctx);
       }
       return NNAL_OK;
     }

@@ -205,8 +205,9 @@ struct nnal_ctx {
   int ens_open = 0;                      // committee accumulation in progress: pool passes of the members keep the running means
   DropSpec mc_drop;                      // keep, threshold, seed, first pass id, global position of pool offset 0
   std::vector<int> mc_sites;             // layer indices whose OUTPUT is dropped out (NN.py:167-171)
-  double* pool_mc_post = nullptr;        // [pool_n] running mean of P(class 1) over the passes (float64, PW_NNAL.py:80)
-  double* pool_mc_ent = nullptr;         // [pool_n] running mean of the per-pass binary entropies (PW_NNAL.py:262-268)
+  double* pool_mc_post = nullptr;        // running means over the passes (float64, PW_NNAL.py:80): c = 2: [pool_n] of P(class 1);
+                                         // c > 2: [c][pool_n] of every class
+  double* pool_mc_ent = nullptr;         // [pool_n] running mean of the per-pass entropies (PW_NNAL.py:262-268)
   size_t pool_cap_mc = 0;
   DevBuf act_mc;                         // third activation buffer: the conv trunk's output must survive the T tail passes
   unsigned int* ovf_word = nullptr;      // device flag set by nnal_ovf_note (shared by the contexts of one device)
@@ -253,6 +254,7 @@ static inline void prof_end(nnal_ctx* ctx) {
 #define NNAL_PROF_GATHER 100
 #define NNAL_PROF_SCORE 101
 #define NNAL_PROF_TOPK 102
+#define NNAL_PROF_MC_ACCUM 103          // MC-dropout / committee running means (score.cu nnal_k_mc_accumulate)
 #define NNAL_PROF_FI_SETUP 110
 #define NNAL_PROF_FI_GRAM 111
 #define NNAL_PROF_FI_GREEDY 112
@@ -294,9 +296,9 @@ int nnal_k_permute_fc_weight(nnal_ctx*, const float* Wtf, float* Wnative, int ou
 // score.cu
 int nnal_k_head(nnal_ctx*, const Layer& fc_last, const float* feat, int64_t n, int64_t pool_n, int64_t offset,
                 float* post /*[c][pool_n]*/, float* logits_out /*[n][c] or null*/, const DropSpec* drop = nullptr);
-int nnal_k_mc_accumulate(nnal_ctx*, const float* post, int64_t pool_n, int64_t offset, int64_t n, int t,
+int nnal_k_mc_accumulate(nnal_ctx*, const float* post, int c, int64_t pool_n, int64_t offset, int64_t n, int t,
                          double* av_post, double* av_ent);
-int nnal_k_scores_mc(nnal_ctx*, const double* av_post, const double* av_ent, int64_t n, int kind, double* score);
+int nnal_k_scores_mc(nnal_ctx*, const double* av_post, const double* av_ent, int c, int64_t n, int kind, double* score);
 int nnal_k_scores_f32(nnal_ctx*, const float* post, int c, int64_t n, int kind, double eps, double* score);
 int nnal_k_scores_f64(nnal_ctx*, const double* post, int c, int64_t n, int kind, double eps, double* score);
 int nnal_k_entropy_f32(nnal_ctx*, const float* post, int c, int64_t n, float eps, float* H);

@@ -159,12 +159,32 @@ __global__ void __launch_bounds__(256) mc_accum_kernel(const float* __restrict__
     av_ent[i] = t == 0 ? e : (e + t * av_ent[i]) / (t + 1);
   }
 }
-int nnal_k_mc_accumulate(nnal_ctx* ctx, const float* post, int64_t pool_n, int64_t offset, int64_t n, int t,
+// c > 2: the same recurrences over every class, av_post [c][pool_n] (the layout of the head's posteriors) and
+//   ents = -sum_j p_j log p_j with zeros bumped by 1e-6.  Memory-bound: 4c B read, 16c + 16 B read and written per sample.
+__global__ void __launch_bounds__(256) mc_class_accum_kernel(const float* __restrict__ post, int c, int64_t stride, int64_t n,
+                                                              int t, double* __restrict__ av_post, double* __restrict__ av_ent) {
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    double e = 0.0;
+    for (int j = 0; j < c; ++j) {
+      double p = (double)post[(int64_t)j * stride + i];
+      double* a = av_post + (int64_t)j * stride + i;
+      *a = t == 0 ? p : (p + t * *a) / (t + 1);
+      if (p == 0.0) p += 1e-6;
+      e -= p * log(p);
+    }
+    av_ent[i] = t == 0 ? e : (e + t * av_ent[i]) / (t + 1);
+  }
+}
+// c == 2 keeps the binary statistics (av_post = mean P(class 1), [pool_n]); c > 2 keeps every class ([c][pool_n])
+int nnal_k_mc_accumulate(nnal_ctx* ctx, const float* post, int c, int64_t pool_n, int64_t offset, int64_t n, int t,
                          double* av_post, double* av_ent) {
   if (n == 0) return NNAL_OK;
   int64_t blocks = (n + 255) / 256;
   int grid = (int)(blocks < (int64_t)ctx->sm_count * 16 ? blocks : (int64_t)ctx->sm_count * 16);
-  mc_accum_kernel<<<grid, 256, 0, ctx->stream>>>(post + pool_n + offset, n, t, av_post + offset, av_ent + offset);
+  if (c == 2)
+    mc_accum_kernel<<<grid, 256, 0, ctx->stream>>>(post + pool_n + offset, n, t, av_post + offset, av_ent + offset);
+  else
+    mc_class_accum_kernel<<<grid, 256, 0, ctx->stream>>>(post + offset, c, pool_n, n, t, av_post + offset, av_ent + offset);
   ctx->launches++;
   CUDA_TRY(ctx, cudaGetLastError());
   return NNAL_OK;
@@ -172,6 +192,8 @@ int nnal_k_mc_accumulate(nnal_ctx* ctx, const float* post, int64_t pool_n, int64
 //   kind 10 (MC-entropy): |av_posts - 0.5|                                           (PW_NNAL.py:84-85, 241)
 //   kind 11 (BALD):       -(H(av_posts) - av_ents), H with the same 1e-6 zero bumps   (PW_NNAL.py:270-278; ascending
 //                         top-k of the negated score = argsort(-scores)[:k])
+//   kind 12:              -H(av_posts), the predictive entropy of kind 10's c-class form (monotone in |av_posts - 0.5|)
+//   kind 13:              kind 11
 __global__ void __launch_bounds__(256) mc_score_kernel(const double* __restrict__ av_post, const double* __restrict__ av_ent,
                                                         int64_t n, int kind, double* __restrict__ score) {
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
@@ -182,16 +204,32 @@ __global__ void __launch_bounds__(256) mc_score_kernel(const double* __restrict_
       double q = 1.0 - p;
       if (p == 0.0) p += 1e-6;
       if (q == 0.0) q += 1e-6;
-      v = -((-p * log(p) - q * log(q)) - av_ent[i]);
+      const double h = -p * log(p) - q * log(q);
+      v = kind == 12 ? -h : -(h - av_ent[i]);
     }
     score[i] = v + 0.0;
   }
 }
-int nnal_k_scores_mc(nnal_ctx* ctx, const double* av_post, const double* av_ent, int64_t n, int kind, double* score) {
+// c > 2, av_post [c][n]:  kind 12: -H(av_posts);  kind 13: -(H(av_posts) - av_ents);  zeros bumped by 1e-6
+__global__ void __launch_bounds__(256) mc_class_score_kernel(const double* __restrict__ av_post, const double* __restrict__ av_ent,
+                                                              int c, int64_t n, int kind, double* __restrict__ score) {
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    double h = 0.0;
+    for (int j = 0; j < c; ++j) {
+      double p = av_post[(int64_t)j * n + i];
+      if (p == 0.0) p += 1e-6;
+      h -= p * log(p);
+    }
+    const double v = kind == 12 ? -h : -(h - av_ent[i]);
+    score[i] = v + 0.0;
+  }
+}
+int nnal_k_scores_mc(nnal_ctx* ctx, const double* av_post, const double* av_ent, int c, int64_t n, int kind, double* score) {
   if (n == 0) return NNAL_OK;
   int64_t blocks = (n + 255) / 256;
   int grid = (int)(blocks < (int64_t)ctx->sm_count * 16 ? blocks : (int64_t)ctx->sm_count * 16);
-  mc_score_kernel<<<grid, 256, 0, ctx->stream>>>(av_post, av_ent, n, kind, score);
+  if (c == 2) mc_score_kernel<<<grid, 256, 0, ctx->stream>>>(av_post, av_ent, n, kind, score);
+  else mc_class_score_kernel<<<grid, 256, 0, ctx->stream>>>(av_post, av_ent, c, n, kind, score);
   ctx->launches++;
   CUDA_TRY(ctx, cudaGetLastError());
   return NNAL_OK;

@@ -382,6 +382,14 @@ class Engine(object):
         self._chk(self.lib.nnal_pool_mc_read(self.h, _ptr(av_post), _ptr(av_ent)))
         return av_post, av_ent
 
+    def pool_mc_class_means(self):
+        """Running means of every class after an MC-dropout or committee pass: (av_post [c,n], av_ent [n]), float64."""
+        av_post = np.empty((self.n_class, self._pool_n), dtype=np.float64)
+        av_ent = np.empty(self._pool_n, dtype=np.float64)
+        self.d2h_bytes += av_post.nbytes + av_ent.nbytes
+        self._chk(self.lib.nnal_pool_mc_read_classes(self.h, _ptr(av_post), _ptr(av_ent)))
+        return av_post, av_ent
+
     def pool_score(self, kind, eps=0.0):
         self._chk(self.lib.nnal_pool_score(self.h, int(kind), float(eps)))
 
