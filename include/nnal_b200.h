@@ -57,7 +57,7 @@ typedef struct { int32_t type, out, kh, kw; } nnal_layer_spec;
 #define NNAL_SCORE_MC_BINARY 10 /* |mean_t P_t(class1) - 0.5| over the MC-dropout passes (PW_NNAL.py:67-87, 232-244) */
 #define NNAL_SCORE_NEG_BALD 11  /* -(H(mean_t P_t) - mean_t H(P_t)), zeros bumped by 1e-6 (PW_NNAL.py:247-282): ascending
                                    top-k of it = np.argsort(-scores)[:k] */
-/* The same two scorers for any 2 <= c <= 32 classes, H = -sum_j p_j log p_j over the running means of every class (zeros
+/* The same two scorers for 2 <= c <= 32 and c >= 64 classes, H = -sum_j p_j log p_j over the running means of every class (zeros
  * bumped by 1e-6).  At c = 2 they are computed from the binary running means with P(class 0) = 1 - P(class 1). */
 #define NNAL_SCORE_MC_NEG_ENTROPY 12 /* -H(mean_t P_t): predictive entropy, k largest (MC-entropy / ensemble) */
 #define NNAL_SCORE_MC_NEG_BALD 13    /* -(H(mean_t P_t) - mean_t H(P_t)): k largest mutual information (BALD / QBC-JS) */
@@ -104,7 +104,9 @@ int nnal_model_set(nnal_ctx* ctx, const nnal_layer_spec* specs, int n_layers, in
 int nnal_model_set_weights(nnal_ctx* ctx, int layer, const float* W, const float* b);
 int nnal_model_info(nnal_ctx* ctx, int* n_class, int* feat_dim, int* prev_dim);
 /* multiply-accumulates per sample of layer `layer` and the kernel family it runs on: 0 FP32 CUDA cores, 1 tcgen05
- * (conv_tc_kernel / fc_tc_pair_kernel), 2 tcgen05 weight-stationary conv (conv_wt_kernel) */
+ * (conv_tc_kernel / fc_tc_pair_kernel), 2 tcgen05 weight-stationary conv (conv_wt_kernel).  The last FC layer: 0 for
+ * c <= 32 (fused head kernel); for c >= 64 (wide head) 1 when its logits GEMM runs on fc_tc_pair_kernel (input width
+ * >= 64 and a multiple of 8, tensor cores on), else 0.  33 <= c <= 63 classes: the pool pass returns NNAL_ERR_UNSUPPORTED. */
 int nnal_model_layer_info(nnal_ctx* ctx, int layer, int* type, long long* macs_per_sample, int* uses_tc);
 
 /* ---- volumes: the padded multi-modality images the query functions receive ----------------- */
@@ -152,15 +154,16 @@ int nnal_pool_eval_device_inds(nnal_ctx* ctx, int subject, const int64_t* d_inds
  * PW_NNAL.py:67-87, 232-282).  Configure BEFORE nnal_pool_begin; the following nnal_pool_eval* calls evaluate the conv
  * trunk once per chunk and the FC tail T times with tf.nn.dropout semantics (x / keep_prob where kept, NN.py:167-171)
  * on the outputs of `layers` (model.dropout_layers: FC layers only), keeping float64 running means of the posteriors and
- * of the per-pass entropies for every pool sample (c = 2: of P(class 1) and the binary entropy; 3 <= c <= 32: of every
- * class).  Masks are Philox4x32-10 words keyed by `seed`, counter {unit/4, pos0 + pool position, first_pass + t, layer}:
- * independent of chunking and of how the pool is sharded.  T = 0 switches MC mode off.  NNAL_ERR_UNSUPPORTED for more
- * than 32 classes or when a hidden FC layer does not run on the tensor-core path. */
+ * of the per-pass entropies for every pool sample (c = 2: of P(class 1) and the binary entropy; 3 <= c <= 32 and c >= 64: of
+ * every class).  Masks are Philox4x32-10 words keyed by `seed`, counter {unit/4, pos0 + pool position, first_pass + t, layer}:
+ * independent of chunking and of how the pool is sharded.  T = 0 switches MC mode off.  NNAL_ERR_UNSUPPORTED for 33 to
+ * 63 classes, when a hidden FC layer does not run on the tensor-core path, or when the logits of a head with 64 or more
+ * classes are a dropout site and that head does not run on the tensor cores. */
 int nnal_pool_mc_config(nnal_ctx* ctx, int T, double keep_prob, unsigned long long seed, unsigned int first_pass,
                         long long pos0, const int* layers, int n_layers);
 /* Committee scorers 'ensemble' / 'QBC-JS' (PW_NNAL.py:453-545): fold member t's deterministic pool pass (the current
  * posteriors) into the same running means, av = (x + t av) / (t + 1).  t = 0 opens the accumulation,
- * nnal_pool_ensemble_end closes it; every member scores the same pool.  2 <= c <= 32.  Scores: NNAL_SCORE_MC_BINARY /
+ * nnal_pool_ensemble_end closes it; every member scores the same pool.  2 <= c <= 32 or c >= 64.  Scores: NNAL_SCORE_MC_BINARY /
  * _NEG_BALD (c = 2), NNAL_SCORE_MC_NEG_ENTROPY / _MC_NEG_BALD (any c). */
 int nnal_pool_ensemble_accumulate(nnal_ctx* ctx, int t);
 int nnal_pool_ensemble_end(nnal_ctx* ctx);

@@ -45,7 +45,11 @@ def CNN_query(model, expr, pool_inds, method_name, session, col=True, extra_feed
     FI selection for any number of classes (``nnal_b200.fi.query_whole_block``) over the last FC layer, or over the last two
     with ``expr.pars['fi_layers'] = 2``.
 
-    Bayesian and committee scorers, for 2 <= c <= 32 classes (the binary definitions of PW_NNAL.py:67-87, 247-282 and
+    Class counts: every method runs for 2 <= c <= 32 (fused head kernel) and for c >= 64 (wide head: FC GEMM for the
+    logits, then a streaming softmax; chosen from the model's class count); 33 <= c <= 63 raises NnalError
+    (NNAL_ERR_UNSUPPORTED).  ``fi_mode = 'block-greedy'`` stays limited to c <= 32.
+
+    Bayesian and committee scorers, for those class counts (the binary definitions of PW_NNAL.py:67-87, 247-282 and
     :453-545 extended to c classes; ties go to the lowest position):
     ``MC-entropy`` / ``BALD``: ``expr.pars['MC_iters']`` MC-dropout passes at ``model.dropout_rate`` on
     ``model.dropout_layers`` (FC layers; the conv trunk runs once), float64 running means of every class posterior and of

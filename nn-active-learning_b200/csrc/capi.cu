@@ -204,6 +204,7 @@ extern "C" int nnal_ctx_destroy(nnal_ctx* ctx) {
   nnal_p2p_release(ctx);
   free_buf(ctx->stage); free_buf(ctx->inds); free_buf(ctx->act[0]); free_buf(ctx->act[1]); free_buf(ctx->xin);
   free_buf(ctx->featbuf); free_buf(ctx->prevbuf); free_buf(ctx->logits); free_buf(ctx->splitA[0]); free_buf(ctx->splitA[1]);
+  free_buf(ctx->head_logits);
   free_buf(ctx->topk_ws); free_buf(ctx->fi_ws);
   cudaStreamDestroy(ctx->stream);
   if (ctx->ovf_host) cudaFreeHost(ctx->ovf_host);
@@ -609,10 +610,11 @@ extern "C" int nnal_entropy_device_f32(nnal_ctx* ctx, const float* d_post, int c
 // pool pass
 // ---------------------------------------------------------------------------------------------
 // MC-dropout and committee statistics: c = 2 keeps the binary running means (P(class 1), PW_NNAL.py:80); 3 <= c <= 32
-// keeps the running mean of every class.
+// and c >= 64 keep the running mean of every class.  33 <= c <= 63 has no head (nnal_k_head).
 static int check_mc_classes(nnal_ctx* ctx) {
-  if (ctx->n_class < 2 || ctx->n_class > 32)
-    NNAL_FAIL(ctx, NNAL_ERR_UNSUPPORTED, "MC-dropout and committee scores need 2 to 32 classes");
+  const int c = ctx->n_class;
+  if (c < 2 || (c > 32 && c < NNAL_WIDE_HEAD_MIN))
+    NNAL_FAIL(ctx, NNAL_ERR_UNSUPPORTED, "MC-dropout and committee scores need 2 to 32 or at least 64 classes");
   return NNAL_OK;
 }
 // Running-mean storage for n pool samples; free_pool resets the capacity when the class count changes.
@@ -683,6 +685,9 @@ extern "C" int nnal_pool_mc_config(nnal_ctx* ctx, int T, double keep_prob, unsig
     if (layers[i] < ctx->fc_first || layers[i] >= (int)ctx->layers.size())
       NNAL_FAIL(ctx, NNAL_ERR_UNSUPPORTED, "dropout sites must be FC layers (the conv trunk is evaluated once)");
     ctx->mc_sites.push_back(layers[i]);
+    // a wide head drops out its logits in the tensor-core GEMM's epilogue
+    if (layers[i] == (int)ctx->layers.size() - 1 && ctx->n_class >= NNAL_WIDE_HEAD_MIN && !nnal_layer_on_tc(ctx, layers[i]))
+      NNAL_FAIL(ctx, NNAL_ERR_UNSUPPORTED, "MC-dropout on the logits of a head with 64 or more classes needs the tensor-core path");
   }
   DropSpec d;
   d.keep = (float)keep_prob;

@@ -18,8 +18,10 @@ struct Act {
 bool layer_on_tc(const nnal_ctx* ctx, int i) {
   if (!ctx->use_tc) return false;
   const int nl = (int)ctx->layers.size();
-  if (i < 0 || i >= nl - 1) return false;               // the last FC runs in the fused head kernel
+  if (i < 0 || i >= nl) return false;
   const Layer& L = ctx->layers[i];
+  // the last FC: c <= 32 runs in the fused head kernel, c >= 64 as the wide head's logits GEMM where it is supported
+  if (i == nl - 1) return L.out_dim >= NNAL_WIDE_HEAD_MIN && nnal_tc_head_supported(ctx, L);
   if (L.type == NNAL_LAYER_CONV) return nnal_tc_conv_supported(ctx, L);
   if (L.type == NNAL_LAYER_FC) return nnal_tc_fc_supported(ctx, L);
   return false;
@@ -31,6 +33,16 @@ bool consumer_wants_split(const nnal_ctx* ctx, int i) {
   int j = i + 1;
   while (j < nl && ctx->layers[j].type == NNAL_LAYER_POOL) ++j;
   return layer_on_tc(ctx, j);
+}
+
+// wide head on the tensor cores from split features [nb][elems]: logits GEMM into the head's scratch, then the softmax
+// into the pool posteriors at `offset`
+int wide_head_planes(nnal_ctx* ctx, const Layer& L, const Act& a, int64_t nb, int64_t offset, const DropSpec* drop) {
+  const int ldz = nnal_head_ldz(L.out_dim);
+  NNAL_TRY(devbuf_reserve(ctx, ctx->head_logits, (size_t)nb * ldz * sizeof(float)));
+  float* z = (float*)ctx->head_logits.p;
+  NNAL_TRY(nnal_tc_head_planes(ctx, L, a.hi, a.lo, (int)a.elems, z, nb, drop));
+  return nnal_k_softmax_wide(ctx, z, ldz, nb, L.out_dim, ctx->pool_n, offset, ctx->pool_post);
 }
 
 }  // namespace
@@ -102,7 +114,7 @@ int nnal_forward_chunk(nnal_ctx* ctx, int64_t nb, int64_t offset, int input_form
       // once; the FC tail runs T times with fresh masks.  The tail ping-pongs between the activation buffer that does
       // not hold the trunk output and a third buffer.  The trunk's last layer writes the split planes the tail's first
       // FC layer takes, on either path; an FC-only net's fp32 input is split once here, not once per pass.
-      if (i < nl - 1) NNAL_TRY(to_split(cur));
+      if (layer_on_tc(ctx, i)) NNAL_TRY(to_split(cur));
       else NNAL_TRY(to_f32(cur));
       size_t maxfc = 0;
       for (int j = i; j < nl; ++j) maxfc = std::max(maxfc, (size_t)ctx->layers[j].out_dim);
@@ -119,7 +131,12 @@ int nnal_forward_chunk(nnal_ctx* ctx, int64_t nb, int64_t offset, int input_form
           bool site = false;
           for (int sj : ctx->mc_sites) site |= (sj == j);
           prof_begin(ctx, j);
-          if (j == nl - 1) {
+          if (j == nl - 1 && layer_on_tc(ctx, j)) {
+            // wide head on the tensor cores: the logits' dropout runs in the GEMM epilogue (rows are chunk-relative)
+            if (!h.split) NNAL_FAIL(ctx, NNAL_ERR_UNSUPPORTED, "MC-dropout: the wide head expects split features");
+            d.row0 += offset;
+            NNAL_TRY(wide_head_planes(ctx, F, h, nb, offset, site ? &d : nullptr));
+          } else if (j == nl - 1) {
             if (h.split) NNAL_FAIL(ctx, NNAL_ERR_UNSUPPORTED, "MC-dropout: the head expects fp32 features");
             NNAL_TRY(nnal_k_head(ctx, F, h.f32, nb, ctx->pool_n, offset, ctx->pool_post, nullptr, site ? &d : nullptr));
           } else {
@@ -146,8 +163,13 @@ int nnal_forward_chunk(nnal_ctx* ctx, int64_t nb, int64_t offset, int input_form
     }
     prof_begin(ctx, i);
     if (i == nl - 1) {
-      NNAL_TRY(to_f32(cur));
-      NNAL_TRY(nnal_k_head(ctx, L, cur.f32, nb, ctx->pool_n, offset, ctx->pool_post, nullptr));
+      if (layer_on_tc(ctx, i)) {
+        NNAL_TRY(to_split(cur));
+        NNAL_TRY(wide_head_planes(ctx, L, cur, nb, offset, nullptr));
+      } else {
+        NNAL_TRY(to_f32(cur));
+        NNAL_TRY(nnal_k_head(ctx, L, cur.f32, nb, ctx->pool_n, offset, ctx->pool_post, nullptr));
+      }
       prof_end(ctx);
       break;
     }

@@ -567,20 +567,51 @@ int nnal_tc_fc_planes(nnal_ctx* ctx, const Layer& L, const nnal_h* Ah, const nna
                              out, L.out_dim, out_hi, out_lo, L.out_dim, drop);
 }
 
-// fp32 A operand [n][K]: split into planes first (used by the isolated test hook and mixed pipelines)
-int nnal_tc_fc(nnal_ctx* ctx, const Layer& L, const float* in, float* out, int64_t n) {
-  if (n == 0) return NNAL_OK;
+// Wide classifier head (c >= 64 classes): the logits GEMM.  Its own predicate, so the hidden layers keep theirs: the class
+// count need not be a multiple of 8 (W's planes have c rows; TMA zero-fills the last 256-row block), the input width must
+// be (16-byte rows of the A planes).  The planes are built by nnal_tc_prepare_layer for every FC with in, out >= 64.
+bool nnal_tc_head_supported(const nnal_ctx*, const Layer& L) {
+  return L.type == NNAL_LAYER_FC && L.Wh != nullptr && L.out_dim >= NNAL_WIDE_HEAD_MIN && L.in_dim >= 64 && (L.in_dim % 8) == 0;
+}
+
+// logits [n][ldz] = A . W^T + b, ldz = nnal_head_ldz(c): the epilogue's full 16-column groups store float4 at row * ldz + col0,
+// so the row stride must keep 16-byte alignment for any c; columns >= c are not written.  No ReLU; `drop` (MC-dropout on
+// the logits) uses the epilogue's tf.nn.dropout with drop->row0 the global position of chunk row 0.
+int nnal_tc_head_planes(nnal_ctx* ctx, const Layer& L, const nnal_h* Ah, const nnal_h* Al, int lda, float* logits, int64_t n,
+                        const DropSpec* drop) {
+  return nnal_tc_gemm_planes(ctx, Ah, Al, lda, n, L.Wh, L.Wl, L.k_pad, L.out_dim, L.in_dim, L.b, L.w_scale_inv, 0, 0, logits,
+                             nnal_head_ldz(L.out_dim), nullptr, nullptr, 0, drop);
+}
+
+// fp32 A operand [n][K] -> hi/lo planes [n][Kp] in ctx->splitA
+static int split_operand(nnal_ctx* ctx, const Layer& L, const float* in, int64_t n, nnal_h** Ah, nnal_h** Al) {
   const int K = L.in_dim, Kp = L.k_pad;
   const size_t plane = (size_t)n * Kp * 2;
   NNAL_TRY(devbuf_reserve(ctx, ctx->splitA[0], plane));
   NNAL_TRY(devbuf_reserve(ctx, ctx->splitA[1], plane));
-  nnal_h* Ah = (nnal_h*)ctx->splitA[0].p;
-  nnal_h* Al = (nnal_h*)ctx->splitA[1].p;
+  *Ah = (nnal_h*)ctx->splitA[0].p;
+  *Al = (nnal_h*)ctx->splitA[1].p;
   int64_t total = n * (int64_t)(Kp / 2);
   int grid = (int)((total + 255) / 256 < (int64_t)ctx->sm_count * 16 ? (total + 255) / 256 : (int64_t)ctx->sm_count * 16);
-  tc::split_kernel<<<grid, 256, 0, ctx->stream>>>(in, Ah, Al, n, K, Kp, 1.f);
+  tc::split_kernel<<<grid, 256, 0, ctx->stream>>>(in, *Ah, *Al, n, K, Kp, 1.f);
   ctx->launches++;
-  return nnal_tc_fc_planes(ctx, L, Ah, Al, Kp, out, nullptr, nullptr, n);
+  return NNAL_OK;
+}
+
+// fp32 A operand [n][K]: split into planes first (used by the isolated test hook and mixed pipelines)
+int nnal_tc_fc(nnal_ctx* ctx, const Layer& L, const float* in, float* out, int64_t n) {
+  if (n == 0) return NNAL_OK;
+  nnal_h *Ah, *Al;
+  NNAL_TRY(split_operand(ctx, L, in, n, &Ah, &Al));
+  return nnal_tc_fc_planes(ctx, L, Ah, Al, L.k_pad, out, nullptr, nullptr, n);
+}
+
+// the wide head's logits from fp32 features (shrunk-gradient forward, fp32 activations)
+int nnal_tc_head(nnal_ctx* ctx, const Layer& L, const float* in, float* logits, int64_t n, const DropSpec* drop) {
+  if (n == 0) return NNAL_OK;
+  nnal_h *Ah, *Al;
+  NNAL_TRY(split_operand(ctx, L, in, n, &Ah, &Al));
+  return nnal_tc_head_planes(ctx, L, Ah, Al, L.k_pad, logits, n, drop);
 }
 
 // flat fp32 <-> fp16 hi/lo conversions (format changes between CUDA-core and tensor-core layers)

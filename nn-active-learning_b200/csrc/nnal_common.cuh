@@ -175,6 +175,7 @@ struct nnal_ctx {
   // workspaces
   DevBuf inds, act[2], xin, featbuf, prevbuf, logits;
   DevBuf splitA[2];                      // fp16 hi/lo activation planes
+  DevBuf head_logits;                    // wide head (c >= 64): logits [chunk][ldz] between the FC GEMM and the softmax
   // pool state
   int64_t pool_n = 0;
   int keep = 0;                          // 0: posteriors only, 1: + features (fc_{L-1} out), 2: + previous fc out
@@ -294,8 +295,14 @@ int nnal_k_pool(nnal_ctx*, const Layer&, const float* in, float* out, int64_t n)
 int nnal_k_fc_simt(nnal_ctx*, const Layer&, const float* in, float* out, int64_t n);
 int nnal_k_permute_fc_weight(nnal_ctx*, const float* Wtf, float* Wnative, int out, int C, int H, int W);
 // score.cu
+// Classifier head: c <= 32 runs the fused head kernel; c >= NNAL_WIDE_HEAD_MIN the FC GEMM into a logits scratch with row
+// stride nnal_head_ldz(c) (tensor cores) or c (CUDA cores), then wide_softmax_kernel.  33..63 classes are unsupported.
+#define NNAL_WIDE_HEAD_MIN 64
+static inline int nnal_head_ldz(int c) { return (c + 7) / 8 * 8; }
 int nnal_k_head(nnal_ctx*, const Layer& fc_last, const float* feat, int64_t n, int64_t pool_n, int64_t offset,
                 float* post /*[c][pool_n]*/, float* logits_out /*[n][c] or null*/, const DropSpec* drop = nullptr);
+int nnal_k_softmax_wide(nnal_ctx*, const float* logits /*[n][ldz]*/, int64_t ldz, int64_t n, int c, int64_t pool_n,
+                        int64_t offset, float* post /*[c][pool_n]*/);
 int nnal_k_mc_accumulate(nnal_ctx*, const float* post, int c, int64_t pool_n, int64_t offset, int64_t n, int t,
                          double* av_post, double* av_ent);
 int nnal_k_scores_mc(nnal_ctx*, const double* av_post, const double* av_ent, int c, int64_t n, int kind, double* score);
@@ -310,6 +317,10 @@ int nnal_tc_release(nnal_ctx*);
 int nnal_tc_fc(nnal_ctx*, const Layer&, const float* in, float* out, int64_t n);
 int nnal_tc_fc_planes(nnal_ctx*, const Layer&, const nnal_h* Ah, const nnal_h* Al, int lda, float* out,
                       nnal_h* out_hi, nnal_h* out_lo, int64_t n, const DropSpec* drop = nullptr);
+bool nnal_tc_head_supported(const nnal_ctx*, const Layer&);
+int nnal_tc_head_planes(nnal_ctx*, const Layer&, const nnal_h* Ah, const nnal_h* Al, int lda, float* logits /*[n][ldz]*/,
+                        int64_t n, const DropSpec* drop = nullptr);
+int nnal_tc_head(nnal_ctx*, const Layer&, const float* in, float* logits /*[n][ldz]*/, int64_t n, const DropSpec* drop = nullptr);
 int nnal_tc_gemm_planes(nnal_ctx*, const nnal_h* Ah, const nnal_h* Al, int64_t lda, int64_t M, const nnal_h* Bh,
                         const nnal_h* Bl, int64_t ldb, int N, int64_t K, const float* bias, float scale, int relu,
                         int accum, float* out, int ldo, nnal_h* out_hi, nnal_h* out_lo, int ld_split,

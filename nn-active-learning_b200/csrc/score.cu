@@ -1,4 +1,5 @@
-// Scoring kernels: fused last-FC + softmax head, entropy / binary-uncertainty scores, exact top-k.
+// Scoring kernels: fused last-FC + softmax head (2..32 classes), the wide head's softmax (64 classes or more), entropy /
+// binary-uncertainty scores, exact top-k.
 //
 // Reference behaviour replaced:
 //   * posteriors = softmax over classes of the last FC output (NN.py:184-188, 322-327)
@@ -76,9 +77,115 @@ __global__ void __launch_bounds__(256) head_kernel(const float* __restrict__ fea
   }
 }
 
+// ------------------------------------------------------------------------------------------
+// wide head (c >= 64): the logits come from the FC GEMM (tensor cores or CUDA cores) into a [n][ldz] scratch; this kernel
+// turns them into post[j][pool_n] at offset + s, exp(z - max) / sum.  Memory-bound: per sample 4c B read twice (the second
+// read from L2) and 4c B written.  One CTA per tile of 32 pool positions, aligned to multiples of 32 of the global position
+// offset + s, so every warp store of a class row covers the same 32-position group (partial at both ends of the range).
+// Pass 1: one warp per sample, max and sum over the row.  Pass 2: 32 x 128 (sample x class) blocks through shared
+// memory, read along the logits rows and written along the class rows.  Nothing is sized by c.  Pass 1 reads the row twice
+// (max, then the sum of exponentials; the second read hits L1/L2) with four independent loads per lane in flight: an online
+// max/sum loop carries a dependency through every element and ran at 13 % of the HBM bound at c = 1,000.
+// ------------------------------------------------------------------------------------------
+constexpr int WSM_THREADS = 512, WSM_CB = 4;
+__global__ void __launch_bounds__(WSM_THREADS) wide_softmax_kernel(const float* __restrict__ z, int64_t ldz, int64_t n, int c,
+                                                                    int64_t pool_n, int64_t offset, float* __restrict__ post) {
+  constexpr int NW = WSM_THREADS / 32;
+  __shared__ float t[WSM_CB][32][33];
+  __shared__ float s_max[32], s_sum[32];
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  const int64_t g_first = offset & ~(int64_t)31;                 // first tile's global position
+  const int64_t ntiles = ((offset + n + 31) >> 5) - (offset >> 5);
+  for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
+    const int64_t s0 = g_first + tile * 32 - offset;             // chunk-relative sample of tile row 0 (may be < 0)
+    for (int r = wid; r < 32; r += NW) {
+      const int64_t s = s0 + r;
+      float m = -INFINITY, sum = 0.f;
+      if (s >= 0 && s < n) {
+        const float* row = z + s * ldz;
+        float m4[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
+        for (int j = lane; j < c; j += 128) {
+#pragma unroll
+          for (int u = 0; u < 4; ++u)
+            if (j + 32 * u < c) m4[u] = fmaxf(m4[u], row[j + 32 * u]);
+        }
+        m = fmaxf(fmaxf(m4[0], m4[1]), fmaxf(m4[2], m4[3]));
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
+        float e4[4] = {0.f, 0.f, 0.f, 0.f};
+        for (int j = lane; j < c; j += 128) {
+#pragma unroll
+          for (int u = 0; u < 4; ++u)
+            if (j + 32 * u < c) e4[u] += expf(row[j + 32 * u] - m);
+        }
+        sum = (e4[0] + e4[1]) + (e4[2] + e4[3]);
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, o);
+      }
+      if (lane == 0) { s_max[r] = m; s_sum[r] = sum; }
+    }
+    __syncthreads();
+    for (int j0 = 0; j0 < c; j0 += 32 * WSM_CB) {              // WSM_CB blocks of 32 classes per barrier pair
+      for (int r = wid; r < 32; r += NW) {                       // sample r, class j0 + 32 u + lane
+        const int64_t s = s0 + r;
+        if (s >= 0 && s < n) {
+#pragma unroll
+          for (int u = 0; u < WSM_CB; ++u) {
+            const int j = j0 + 32 * u + lane;
+            if (j < c) t[u][r][lane] = expf(z[s * ldz + j] - s_max[r]) / s_sum[r];
+          }
+        }
+      }
+      __syncthreads();
+      for (int r = wid; r < 32; r += NW) {                       // class j0 + 32 u + r, sample lane
+        const int64_t s = s0 + lane;
+        if (s >= 0 && s < n) {
+#pragma unroll
+          for (int u = 0; u < WSM_CB; ++u) {
+            const int j = j0 + 32 * u + r;
+            if (j < c) post[(int64_t)j * pool_n + offset + s] = t[u][lane][r];
+          }
+        }
+      }
+      __syncthreads();
+    }
+  }
+}
+
+int nnal_k_softmax_wide(nnal_ctx* ctx, const float* logits, int64_t ldz, int64_t n, int c, int64_t pool_n, int64_t offset,
+                        float* post) {
+  if (n == 0) return NNAL_OK;
+  const int64_t ntiles = ((offset + n + 31) >> 5) - (offset >> 5);
+  const int grid = (int)(ntiles < (int64_t)ctx->sm_count * 4 ? ntiles : (int64_t)ctx->sm_count * 4);
+  wide_softmax_kernel<<<grid, WSM_THREADS, 0, ctx->stream>>>(logits, ldz, n, c, pool_n, offset, post);
+  ctx->launches++;
+  CUDA_TRY(ctx, cudaGetLastError());
+  return NNAL_OK;
+}
+
+// c >= 64 from fp32 features: the logits GEMM on the tensor cores (the head's own predicate, nnal_tc_head_supported) or
+// the CUDA-core FC kernel, then the softmax.  Dropout on the logits is applied by the tensor-core GEMM's epilogue only:
+// MC-dropout needs the hidden FC layers on the tensor cores, so its wide head never takes the CUDA-core path.
+static int wide_head_f32(nnal_ctx* ctx, const Layer& L, const float* feat, int64_t n, int64_t pool_n, int64_t offset,
+                         float* post, const DropSpec* drop) {
+  const int c = L.out_dim;
+  if (ctx->use_tc && nnal_tc_head_supported(ctx, L)) {
+    const int ldz = nnal_head_ldz(c);
+    NNAL_TRY(devbuf_reserve(ctx, ctx->head_logits, (size_t)n * ldz * sizeof(float)));
+    NNAL_TRY(nnal_tc_head(ctx, L, feat, (float*)ctx->head_logits.p, n, drop));
+    return nnal_k_softmax_wide(ctx, (const float*)ctx->head_logits.p, ldz, n, c, pool_n, offset, post);
+  }
+  if (drop && drop->thresh)
+    NNAL_FAIL(ctx, NNAL_ERR_UNSUPPORTED, "MC-dropout on the logits of a head with more than 32 classes needs the tensor-core path");
+  NNAL_TRY(devbuf_reserve(ctx, ctx->head_logits, (size_t)n * c * sizeof(float)));
+  NNAL_TRY(nnal_k_fc_simt(ctx, L, feat, (float*)ctx->head_logits.p, n));
+  return nnal_k_softmax_wide(ctx, (const float*)ctx->head_logits.p, c, n, c, pool_n, offset, post);
+}
+
 int nnal_k_head(nnal_ctx* ctx, const Layer& L, const float* feat, int64_t n, int64_t pool_n, int64_t offset,
                 float* post, float* logits_out, const DropSpec* dropp) {
   if (n == 0) return NNAL_OK;
+  if (L.out_dim >= NNAL_WIDE_HEAD_MIN && !logits_out) return wide_head_f32(ctx, L, feat, n, pool_n, offset, post, dropp);
   const DropSpec drop = dropp ? *dropp : DropSpec();
   int c = L.out_dim, d = L.in_dim;
   int64_t blocks = (n * 32 + 255) / 256;
@@ -90,7 +197,7 @@ int nnal_k_head(nnal_ctx* ctx, const Layer& L, const float* feat, int64_t n, int
   else if (c <= 32)
     head_kernel<32><<<grid, 256, 0, ctx->stream>>>(feat, L.W, L.b, n, d, c, pool_n, offset, post, logits_out, drop);
   else
-    NNAL_FAIL(ctx, NNAL_ERR_UNSUPPORTED, "more than 32 classes not supported by the fused head");
+    NNAL_FAIL(ctx, NNAL_ERR_UNSUPPORTED, "33 to 63 classes are not supported (fused head: 2 to 32, wide head: 64 or more)");
   ctx->launches++;
   CUDA_TRY(ctx, cudaGetLastError());
   return NNAL_OK;

@@ -594,7 +594,8 @@ def query_whole(model, expr, pool_inds, session):
 
 def query_whole_block(model, expr, pool_inds, session, return_objective=False):
     """``NNAL.CNN_query(..., 'fi')`` with ``expr.pars['fi_mode'] = 'block-greedy'``: greedy minimisation of the FI
-    objective ``tr((sum_{i in S} F_i/|S| + delta I)^-1)`` for any number of classes c >= 2 (c <= 32, k (c-1) <= 4096) in
+    objective ``tr((sum_{i in S} F_i/|S| + delta I)^-1)`` for 2 <= c <= 32 classes (k (c-1) <= 4096; with more classes the
+    library raises NNAL_ERR_UNSUPPORTED after the pool pass, before it allocates the block system) in
     the block form of csrc/fi_block.cu.  ``expr.pars['fi_layers']`` (default 1) picks the parameters: 1 = the last FC
     layer, ``F_i = (diag pi_i - pi_i pi_i^T) (x) [u_i;1][u_i;1]^T`` (NN.LLFC_hess, NN.py:891-901); 2 = the last two FC
     layers, as the binary path's default, adding the score ``(M_i W3^T (e_y - pi_i)) (x) [a_i;1]`` of the previous FC
