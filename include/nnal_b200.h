@@ -382,7 +382,8 @@ int nnal_pool_prev_rows(nnal_ctx* ctx, const int64_t* pos, int64_t n, float* out
 /* Kernel-selection switches for TESTS (there are no environment variables): "chunk" / "bw_chunk" (samples per chunk of the
  * forward / shrunk-gradient pass), "no_fused_gather", "conv_wt" (0..3), "conv_x16" (set before the weights are uploaded),
  * "wt_flags", "sdp_no_coop", "bw_no_ws", "bw_no_tc8", "bw_no_tc", "bw_simt_fwd" select fallback kernels so that every code
- * path can be held to the same parity bar.  The product path never calls this. */
+ * path can be held to the same parity bar; "conv_grid" (0 = off) caps the number of persistent CTAs of the tensor-core
+ * convolutions, so that a few dozen samples run many sample groups on each CTA.  The product path never calls this. */
 int nnal_debug_option(nnal_ctx* ctx, const char* name, long value);
 /* Declares a pool of n samples with the given float64 scores (no model, no pool pass): drives nnal_pool_topk /
  * nnal_pool_topk_device with arbitrary scores in tests. */
@@ -399,6 +400,18 @@ int nnal_debug_fc(nnal_ctx* ctx, const float* A, const float* W, const float* b,
  * 5 = PW1 conv1 with the 5 filter columns folded into the channel axis (x-im2col'd input, conv_tc.cu CfgConv1X). */
 int nnal_debug_conv(nnal_ctx* ctx, const float* x, const float* W, const float* b, int64_t n, int H, int Wd, int Cin,
                     int Cout, int ks, int use_tc, float* out);
+
+/* Data gradient of one conv layer (SAME, stride 1) on host buffers: dz [n][H][Wd][Cout] and the forward filter
+ * W [ks][ks][Cin][Cout] give d_in [n][H][Wd][Cin] = correlation of dz with the flipped, transposed filter, float32.
+ * use_tc = 1: the tensor-core kernel of the shrunk-gradient pass (dz as power-of-two scaled fp16 hi/lo planes;
+ * NNAL_ERR_UNSUPPORTED for a shape without a tile plan); 0: the fp32 CUDA-core kernel (debug options bw_no_ws / bw_no_tc8). */
+int nnal_debug_conv_bwd(nnal_ctx* ctx, const float* dz, const float* W, int64_t n, int H, int Wd, int Cin, int Cout, int ks,
+                        int use_tc, float* out);
+
+/* The model's first layer (PW1 conv1) with the patch gather fused in, over n voxel ids of an uploaded 3-modality float32
+ * volume (25 x 25 x 1 patches, normalised as the pool pass does): conv1's output [n][25][25][24] in float32. */
+int nnal_debug_conv1_gather(nnal_ctx* ctx, int subject, const int64_t* inds, int64_t n, const double* stats, int norm_mode,
+                            float* out);
 
 #ifdef __cplusplus
 }

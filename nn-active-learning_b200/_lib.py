@@ -66,6 +66,9 @@ SIGNATURES = {
     'nnal_debug_fc': (C.c_int, [c_vp, c_vp, c_vp, c_vp, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_int, c_vp]),
     'nnal_debug_conv': (C.c_int, [c_vp, c_vp, c_vp, c_vp, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                   C.c_int, c_vp]),
+    'nnal_debug_conv_bwd': (C.c_int, [c_vp, c_vp, c_vp, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
+                                      c_vp]),
+    'nnal_debug_conv1_gather': (C.c_int, [c_vp, C.c_int, c_vp, C.c_int64, c_vp, C.c_int, c_vp]),
     'nnal_rep_set': (C.c_int, [c_vp, c_vp, C.c_int64, c_vp, C.c_int64, C.c_int64]),
     'nnal_rep_step_scores': (C.c_int, [c_vp, c_vp]),
     'nnal_rep_step_pick': (C.c_int, [c_vp, C.c_int64, c_vp]),

@@ -29,6 +29,7 @@ extern "C" int nnal_debug_option(nnal_ctx* ctx, const char* name, long value) {
   else if (n == "bw_simt_fwd") d.bw_simt_fwd = (int)value;
   else if (n == "fi_flags") d.fi_flags = (int)value;
   else if (n == "plain_upload") d.plain_upload = (int)value;
+  else if (n == "conv_grid") d.conv_grid = (int)value;
   else if (n == "conv_wt") ctx->use_wt = (int)value;       // 0 conv_tc.cu only, 1 conv_wt.cu where faster, 2 (default) + pool fusion, 3 wherever supported
   else if (n == "conv_x16") ctx->use_x16 = (int)value;     // conv1 on the x-im2col'd input (set BEFORE the weights are uploaded)
   else NNAL_FAIL(ctx, NNAL_ERR_INVALID, "unknown debug option");
@@ -337,7 +338,7 @@ extern "C" int nnal_model_info(nnal_ctx* ctx, int* n_class, int* feat_dim, int* 
 
 // power-of-two scale that lifts max|W| to [2^13, 2^14): fp16 hi terms stay far from overflow and the
 // lo terms (2^-11 of hi) stay out of the subnormal range for all but negligible weights
-static void nnal_set_weight_scale(Layer& L, const float* W, size_t n) {
+void nnal_set_weight_scale(Layer& L, const float* W, size_t n) {
   float mx = 0.f;
   for (size_t i = 0; i < n; ++i) { float a = fabsf(W[i]); if (a > mx && a < 3.0e38f) mx = a; }
   int e = 0;
@@ -1214,6 +1215,50 @@ extern "C" int nnal_debug_conv(nnal_ctx* ctx, const float* x, const float* W, co
     if (cudaMemcpyAsync(out, dO, oe_out * 4, cudaMemcpyDeviceToHost, ctx->stream) != cudaSuccess ||
         cudaStreamSynchronize(ctx->stream) != cudaSuccess) {
       ctx->err = std::string("debug_conv: ") + cudaGetErrorString(cudaGetLastError()); rc = NNAL_ERR_CUDA;
+    }
+  }
+  if (rc == NNAL_OK && nnal_ovf_enqueue(ctx) == NNAL_OK && cudaStreamSynchronize(ctx->stream) == cudaSuccess) rc = nnal_ovf_test(ctx);
+  cleanup();
+  return rc;
+}
+
+// test hook: conv1 of the model with the patch gather fused in (conv_tc.cu CfgConv1XG) over `n` voxels of an uploaded volume:
+// conv1's float32 output [n][25][25][24] (merged fp16 hi/lo planes) on the host
+extern "C" int nnal_debug_conv1_gather(nnal_ctx* ctx, int subject, const int64_t* inds, int64_t n, const double* stats,
+                                       int norm_mode, float* out) {
+  if (!ctx || !inds || !out || n <= 0) return NNAL_ERR_INVALID;
+  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  if (ctx->layers.empty() || !ctx->layers[0].has_weights) NNAL_FAIL(ctx, NNAL_ERR_STATE, "model weights not set");
+  const Volume* v;
+  NNAL_TRY(check_gather_args(ctx, subject, n, 25, 25, 1, &v));
+  const Layer& L = ctx->layers[0];
+  if (!nnal_tc_conv1_fused_supported(ctx, L, *v, 25, 25, 1))
+    NNAL_FAIL(ctx, NNAL_ERR_UNSUPPORTED, "first layer / volume not covered by the conv1 that gathers its own input");
+  double* d_stats;
+  NNAL_TRY(upload_stats(ctx, stats, v->m, norm_mode, &d_stats));
+  const size_t oe = (size_t)n * 25 * 25 * L.out_c;
+  int64_t* dI = nullptr;
+  nnal_h* oh = nullptr;
+  float* dO = nullptr;
+  auto cleanup = [&]() {
+    cudaStreamSynchronize(ctx->stream);
+    if (dI) cudaFree(dI); if (oh) cudaFree(oh); if (dO) cudaFree(dO);
+  };
+  if (cudaMalloc(&dI, (size_t)n * 8) != cudaSuccess || cudaMalloc(&oh, oe * 4) != cudaSuccess || cudaMalloc(&dO, oe * 4) != cudaSuccess) {
+    cleanup(); NNAL_FAIL(ctx, NNAL_ERR_CUDA, "debug_conv1_gather allocation failed");
+  }
+  int rc = NNAL_OK;
+  if (cudaMemcpyAsync(dI, inds, (size_t)n * 8, cudaMemcpyHostToDevice, ctx->stream) != cudaSuccess) {
+    ctx->err = std::string("debug_conv1_gather: ") + cudaGetErrorString(cudaGetLastError()); rc = NNAL_ERR_CUDA;
+  }
+  FusedGather fg;
+  fg.vol = v; fg.d_inds = dI; fg.h_stats = stats; fg.norm_mode = norm_mode; fg.d1 = 25; fg.d2 = 25; fg.d3 = 1;
+  if (rc == NNAL_OK) rc = nnal_tc_conv1_fused(ctx, L, fg, oh, oh + oe, n);
+  if (rc == NNAL_OK) rc = nnal_k_merge_flat(ctx, oh, oh + oe, dO, (int64_t)oe);
+  if (rc == NNAL_OK) {
+    if (cudaMemcpyAsync(out, dO, oe * 4, cudaMemcpyDeviceToHost, ctx->stream) != cudaSuccess ||
+        cudaStreamSynchronize(ctx->stream) != cudaSuccess) {
+      ctx->err = std::string("debug_conv1_gather: ") + cudaGetErrorString(cudaGetLastError()); rc = NNAL_ERR_CUDA;
     }
   }
   if (rc == NNAL_OK && nnal_ovf_enqueue(ctx) == NNAL_OK && cudaStreamSynchronize(ctx->stream) == cudaSuccess) rc = nnal_ovf_test(ctx);

@@ -873,8 +873,7 @@ static int launch(nnal_ctx* ctx, const Layer& L, const nnal_h* in_hi, const nnal
   }
   ConvParams p;
   p.wpack = (const uint8_t*)(wpack ? wpack : L.Wh); p.bias = L.b; p.out_hi = out_hi; p.out_lo = out_lo; p.out_f32 = out_f32; p.n = (int)n; p.w_scale_inv = C::RAW ? scale_inv : L.w_scale_inv;
-  const int ngroups = (int)((n + C::G - 1) / C::G);
-  const int grid = ngroups < ctx->sm_count ? ngroups : ctx->sm_count;
+  const int grid = nnal_conv_grid(ctx, (n + C::G - 1) / C::G);
   conv_tc_kernel<C><<<grid, C::THREADS, C::SMEM, ctx->stream>>>(tmHi, tmLo, p, ga);
   ctx->launches++;
   CUDA_TRY(ctx, cudaGetLastError());

@@ -532,8 +532,7 @@ static int launch(nnal_ctx* ctx, const Layer& L, const nnal_h* in_hi, const nnal
   Params p;
   p.wpack = (const uint8_t*)L.Wt; p.bias = L.b; p.out_hi = out_hi; p.out_lo = out_lo; p.n = (int)n; p.w_scale_inv = L.w_scale_inv;
   p.flags = ctx->dbg.wt_flags;
-  const int ngroups = (int)((n + C::G - 1) / C::G);
-  const int grid = ngroups < ctx->sm_count ? ngroups : ctx->sm_count;
+  const int grid = nnal_conv_grid(ctx, (n + C::G - 1) / C::G);
   conv_wt_kernel<C><<<grid, C::THREADS, C::SMEM, ctx->stream>>>(tmHiL, tmLoL, tmHiU, tmLoU, p);
   ctx->launches++;
   CUDA_TRY(ctx, cudaGetLastError());

@@ -152,6 +152,7 @@ struct DebugOpts {
   int plain_upload = 0;        // volumes: one cudaMemcpyAsync per modality even from pageable memory (instead of the threaded pinned staging)
   int fi_flags = 0;            // fi.cu: 1 skip the column pass, 2 skip the evaluation, 4 skip stand-alone inversions (timing experiments, results are garbage);
                                // 8 one-pivot-at-a-time inverse inside the column kernel instead of the pipelined step, 16 no speculative columns (tests)
+  int conv_grid = 0;           // caps the persistent grid of conv_tc_kernel / conv_wt_kernel (0: min(groups, SMs)): few CTAs run many sample groups each
 };
 
 struct nnal_ctx {
@@ -266,6 +267,13 @@ static inline void prof_end(nnal_ctx* ctx) {
 #define NNAL_PROF_BW_FORWARD 120
 #define NNAL_PROF_BW_BACKWARD 121
 
+// persistent grid of the tensor-core convolutions: one CTA per sample group up to the SM count (or the conv_grid cap)
+static inline int nnal_conv_grid(const nnal_ctx* ctx, int64_t ngroups) {
+  int64_t g = ngroups < ctx->sm_count ? ngroups : ctx->sm_count;
+  if (ctx->dbg.conv_grid > 0 && g > ctx->dbg.conv_grid) g = ctx->dbg.conv_grid;
+  return (int)g;
+}
+
 static inline int cdiv(long long a, long long b) { return (int)((a + b - 1) / b); }
 
 // fp16 range guard: enqueue the flag read on the stream (before a synchronisation the caller does anyway), then test it
@@ -345,6 +353,8 @@ bool nnal_tc_conv_bwd_supported(const nnal_ctx*, const Layer&);
 int nnal_tc_conv_bwd_prepare(nnal_ctx*, const Layer&, void** packed);
 int nnal_tc_conv_bwd(nnal_ctx*, const Layer&, const void* packed, const nnal_h* dz_hi, const nnal_h* dz_lo, float* d_in, int64_t n,
                      float scale_inv);
+// power-of-two scale that lifts max|W| of a layer's weights (host array) to [2^13, 2^14) (capi.cu)
+void nnal_set_weight_scale(Layer& L, const float* W, size_t n);
 bool nnal_tc_conv_pool_supported(const nnal_ctx*, const Layer&);
 int nnal_tc_conv_pool(nnal_ctx*, const Layer&, const nnal_h* in_hi, const nnal_h* in_lo, nnal_h* out_hi, nnal_h* out_lo,
                       int64_t n);

@@ -796,6 +796,50 @@ int check_model(nnal_ctx* ctx) {
 
 }  // namespace
 
+// test hook: the data gradient of one conv layer, d_in = correlation of dz with the flipped filter, on host buffers.  use_tc = 1
+// takes the path of shrunk_chunk (power-of-two scaled dz planes, tensor-core kernel on the packed flipped, transposed filter),
+// use_tc = 0 the fp32 CUDA-core kernel (honouring bw_no_ws / bw_no_tc8).
+extern "C" int nnal_debug_conv_bwd(nnal_ctx* ctx, const float* dz, const float* W, int64_t n, int H, int Wd, int Cin, int Cout,
+                                   int ks, int use_tc, float* out) {
+  if (!ctx || !dz || !W || !out || n <= 0 || H <= 0 || Wd <= 0 || Cin <= 0 || Cout <= 0 || ks <= 0) return NNAL_ERR_INVALID;
+  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  Layer L;
+  L.type = NNAL_LAYER_CONV; L.kh = L.kw = ks; L.in_h = L.out_h = H; L.in_w = L.out_w = Wd; L.in_c = Cin; L.out_c = Cout; L.relu = 1;
+  const size_t ze = (size_t)n * H * Wd * Cout, ie = (size_t)n * H * Wd * Cin, wn = (size_t)ks * ks * Cin * Cout;
+  float *dZ = nullptr, *dI = nullptr;
+  void* packed = nullptr;
+  auto cleanup = [&]() {
+    cudaStreamSynchronize(ctx->stream);
+    if (dZ) cudaFree(dZ); if (dI) cudaFree(dI); if (L.W) cudaFree(L.W); if (packed) cudaFree(packed);
+  };
+  if (cudaMalloc(&dZ, ze * 4) != cudaSuccess || cudaMalloc(&dI, ie * 4) != cudaSuccess || cudaMalloc(&L.W, wn * 4) != cudaSuccess) {
+    cleanup(); NNAL_FAIL(ctx, NNAL_ERR_CUDA, "debug_conv_bwd allocation failed");
+  }
+  int rc = NNAL_OK;
+  if (cudaMemcpyAsync(dZ, dz, ze * 4, cudaMemcpyHostToDevice, ctx->stream) != cudaSuccess ||
+      cudaMemcpyAsync(L.W, W, wn * 4, cudaMemcpyHostToDevice, ctx->stream) != cudaSuccess) {
+    ctx->err = std::string("debug_conv_bwd: ") + cudaGetErrorString(cudaGetLastError()); rc = NNAL_ERR_CUDA;
+  }
+  L.has_weights = true;
+  nnal_set_weight_scale(L, W, wn);
+  if (rc == NNAL_OK && use_tc) {
+    if (!nnal_tc_conv_bwd_supported(ctx, L)) { ctx->err = "conv gradient shape not covered by the tensor-core kernel"; rc = NNAL_ERR_UNSUPPORTED; }
+    if (rc == NNAL_OK) rc = nnal_tc_conv_bwd_prepare(ctx, L, &packed);
+    if (rc == NNAL_OK) rc = conv_bwd_data_tc(ctx, bw_state(ctx), L, packed, dZ, dI, n);
+  } else if (rc == NNAL_OK) {
+    rc = conv_bwd_data(ctx, L, dZ, dI, n);
+  }
+  if (rc == NNAL_OK) {
+    if (cudaMemcpyAsync(out, dI, ie * 4, cudaMemcpyDeviceToHost, ctx->stream) != cudaSuccess ||
+        cudaStreamSynchronize(ctx->stream) != cudaSuccess) {
+      ctx->err = std::string("debug_conv_bwd: ") + cudaGetErrorString(cudaGetLastError()); rc = NNAL_ERR_CUDA;
+    }
+  }
+  if (rc == NNAL_OK && nnal_ovf_enqueue(ctx) == NNAL_OK && cudaStreamSynchronize(ctx->stream) == cudaSuccess) rc = nnal_ovf_test(ctx);
+  cleanup();
+  return rc;
+}
+
 int nnal_bw_release(nnal_ctx* ctx) {
   if (!ctx->bw_state) return NNAL_OK;
   BwState* st = (BwState*)ctx->bw_state;

@@ -127,6 +127,27 @@ class Engine(object):
                                            _ptr(out)))
         return out
 
+    def debug_conv_bwd(self, dz, W, use_tc):
+        """Data gradient [n, H, Wd, Cin] of one conv layer from dz [n, H, Wd, Cout] and its filter [ks, ks, Cin, Cout]:
+        use_tc 1 the tensor-core kernel of the shrunk-gradient pass, 0 the fp32 CUDA-core kernel."""
+        dz = np.ascontiguousarray(dz, dtype=np.float32)
+        W = np.ascontiguousarray(W, dtype=np.float32)
+        n, H, Wd, Cout = dz.shape
+        ks, _, Cin, _ = W.shape
+        out = np.empty((n, H, Wd, Cin), dtype=np.float32)
+        self._chk(self.lib.nnal_debug_conv_bwd(self.h, _ptr(dz), _ptr(W), n, H, Wd, Cin, Cout, ks, int(use_tc), _ptr(out)))
+        return out
+
+    def debug_conv1_gather(self, subject, inds, stats, norm_mode=L.NORM_BATCH_EVAL):
+        """Output [n, 25, 25, 24] of the model's conv1 gathering its own 25 x 25 x 1 patches at ``inds`` from the volume
+        uploaded as ``subject``."""
+        inds = np.ascontiguousarray(inds, dtype=np.int64).ravel()
+        st = None if stats is None else np.ascontiguousarray(stats, dtype=np.float64)
+        out = np.empty((inds.size, 25, 25, 24), dtype=np.float32)
+        self._chk(self.lib.nnal_debug_conv1_gather(self.h, int(subject), _ptr(inds), inds.size,
+                                                   None if st is None else _ptr(st), int(norm_mode), _ptr(out)))
+        return out
+
     def set_tensor_cores(self, enable):
         self._chk(self.lib.nnal_set_tensor_cores(self.h, 1 if enable else 0))
 
