@@ -261,7 +261,8 @@ int nnal_fi_step_pack(nnal_ctx* ctx, int64_t step, void* d_msg);
 int nnal_fi_step_apply_gathered(nnal_ctx* ctx, int64_t step, const void* d_msgs, int world, int rank);
 int nnal_fi_result(nnal_ctx* ctx, int64_t k, int64_t* gids_out, double* red_out);
 
-/* Greedy FI selection for multi-class models (2 <= c <= 32), last FC layer (or the last two, below), in block form (csrc/fi_block.cu):
+/* Greedy FI selection for multi-class models (2 <= c <= 32; any c with a class cap, below), last FC layer (or the last two,
+ * below), in block form (csrc/fi_block.cu):
  * F_i = A(pi_i) (x) [u_i;1][u_i;1]^T with A(pi) = diag pi - pi pi^T = L_i L_i^T (closed-form c x (c-1) factor of the
  * float64-renormalised posteriors), block kernel K_ij = (L_i^T L_j)(u_i.u_j + 1), D = c(d+1), r = c-1.  Same objective
  * f(S) = tr((sum_{i in S} F_i/|S| + delta I)^-1) = (D - |S| r)/delta + red(S), red(S) = tr((delta I + K_SS/|S|)^-1), and
@@ -282,6 +283,21 @@ int nnal_fi_block_set_candidates_nl(nnal_ctx* ctx, const int64_t* cand, int64_t 
 int nnal_fi_block_set_factors_nl(nnal_ctx* ctx, int64_t n, int c, int d, int d_prev, const float* post, const float* U,
                                  const float* A_prev, const float* w_last);
 int nnal_fi_block_greedy(nnal_ctx* ctx, int64_t k, double delta, int64_t* sel_out, double* obj_out, double* red_out);
+/* Block form for any class count (last FC layer only), keeping each candidate's q = min(r, c) most probable classes,
+ * 2 <= r <= 32 (else NNAL_ERR_INVALID).  Kept: the q largest float32 posteriors (ties: lower class index), stored in ascending
+ * class order and renormalised in float64 over the kept classes (summed in ascending class order); F_i is the block-form FI of
+ * that truncated posterior, L_i its q x (q-1) factor, and K_ij = s_ij sum over the classes i and j share of L_i^T L_j.  The
+ * greedy reports f = (D - |S| (q-1))/delta + red with D = c(d+1) and needs k (q-1) <= 4096.  With r >= c (c <= 32) every
+ * class is kept in order and the results equal nnal_fi_block_set_candidates' bit for bit.
+ * nnal_fi_block_set_candidates_cls: from the current pool pass, as nnal_fi_block_set_candidates.
+ * nnal_fi_block_set_factors_cls: from host factors in kept form, cls[n][r] class ids (0 <= id < c, strictly ascending per
+ * candidate, else NNAL_ERR_INVALID), p[n][r] their posteriors, U[n][d]; 2 <= r <= min(32, c).
+ * nnal_pool_top_classes: the kept classes of pool rows `rows` (NULL: rows 0..n-1) of the current pool pass, q = min(r, c)
+ * per row: cls_out[n][q] ids ascending and p_out[n][q] their float32 posteriors, as the in-place set-up selects them. */
+int nnal_fi_block_set_candidates_cls(nnal_ctx* ctx, const int64_t* cand, int64_t n_cand, int r);
+int nnal_fi_block_set_factors_cls(nnal_ctx* ctx, int64_t n, int c, int r, int d, const int32_t* cls, const float* p,
+                                  const float* U);
+int nnal_pool_top_classes(nnal_ctx* ctx, const int64_t* rows, int64_t n, int r, int32_t* cls_out, float* p_out);
 
 /* All-gather of the per-step messages over NVLink peer memory instead of NCCL (csrc/p2p.cu): 100 dependent steps of one small
  * message each are latency bound, and one kernel that stores into the peers' buffers and spins on their flags costs a third of

@@ -47,7 +47,8 @@ def CNN_query(model, expr, pool_inds, method_name, session, col=True, extra_feed
 
     Class counts: every method runs for 2 <= c <= 32 (fused head kernel) and for c >= 64 (wide head: FC GEMM for the
     logits, then a streaming softmax; chosen from the model's class count); 33 <= c <= 63 raises NnalError
-    (NNAL_ERR_UNSUPPORTED).  ``fi_mode = 'block-greedy'`` stays limited to c <= 32.
+    (NNAL_ERR_UNSUPPORTED).  ``fi_mode = 'block-greedy'`` runs for c <= 32, and for any c with ``expr.pars['fi_classes'] = r``
+    (2 <= r <= 32, last FC layer only): each candidate keeps its min(r, c) most probable classes, renormalised.
 
     Bayesian and committee scorers, for those class counts (the binary definitions of PW_NNAL.py:67-87, 247-282 and
     :453-545 extended to c classes; ties go to the lowest position):

@@ -104,6 +104,9 @@ SIGNATURES = {
     'nnal_fi_block_greedy': (C.c_int, [c_vp, C.c_int64, C.c_double, c_vp, c_vp, c_vp]),
     'nnal_fi_block_set_candidates_nl': (C.c_int, [c_vp, c_vp, C.c_int64, C.c_int]),
     'nnal_fi_block_set_factors_nl': (C.c_int, [c_vp, C.c_int64, C.c_int, C.c_int, C.c_int, c_vp, c_vp, c_vp, c_vp]),
+    'nnal_fi_block_set_candidates_cls': (C.c_int, [c_vp, c_vp, C.c_int64, C.c_int]),
+    'nnal_fi_block_set_factors_cls': (C.c_int, [c_vp, C.c_int64, C.c_int, C.c_int, C.c_int, c_vp, c_vp, c_vp]),
+    'nnal_pool_top_classes': (C.c_int, [c_vp, c_vp, C.c_int64, C.c_int, c_vp, c_vp]),
     'nnal_p2p_alloc':(C.c_int, [c_vp, C.c_int, C.c_int, C.c_int64, c_vp]),
     'nnal_p2p_open': (C.c_int, [c_vp, c_vp]),
     'nnal_p2p_allgather': (C.c_int, [c_vp, c_vp, C.c_int64, C.c_uint64, c_vp]),

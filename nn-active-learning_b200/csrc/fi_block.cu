@@ -28,16 +28,26 @@
 // doubles [s_wj, s'_wj, Q_wj (upper triangle, row-major)].  Q_{., w} = Mask P_w is a GEMM with an exact 0/1 A operand
 // (Mask[j,k] = m_j[k]) and P_w[k,(y,z)] = m_w[k] W3[y,k] W3[z,k] (exact in float64: a product of two floats), accumulated
 // in float64 in a fixed order.  Set-up runs the same GEMM with P = P_1 (m_w = 1) for Q_jj.
+//
+// Kept classes (one layer).  Every candidate carries an ascending list of q class ids and the float32 posteriors of those
+// classes: without a class cap the identity 0..c-1 (q = c <= 32), with a cap r the r-hat = min(r, c) most probable classes
+// (ties: lower class index, topc_kernel), renormalised over the kept ones.  L_i is then q x (q-1) in kept order, and every
+// sum over classes above runs over the classes two candidates share, in ascending class order:
+//     K_ij = s_ij sum_{cls_i[x] = cls_j[x']} L_i[x,:]^T L_j[x',:],   Z = C Lblk^T keeps q columns per winner,
+//     W_j[rho, x'] = sum_a s_{w_a j} Z[rho, (a, x)] over the x with cls_{w_a}[x] = cls_j[x'],   Y_j = W_j L_j.
+// With the identity list these are the dense sums in the same order, so an uncapped run is the dense block form bit for bit.
+// The two-layer kernels run on the identity list only (q = c).
 #include "nnal_common.cuh"
 #include "dots.cuh"
 #include "../../include/nnal_b200.h"
 #include <algorithm>
+#include <climits>
 #include <cmath>
 
 namespace fib {
 
-constexpr int MAX_C = 32;              // the fused head's class limit
-constexpr int64_t MAX_KR = 4096;       // k (c-1): order of the largest system inverted per step
+constexpr int MAX_C = 32;              // the fused head's class limit; the most classes kept per candidate
+constexpr int64_t MAX_KR = 4096;       // k (q-1): order of the largest system inverted per step
 constexpr int RT = 8;                  // rows of Z per eval tile
 constexpr int EVAL_THREADS = 256;
 constexpr size_t EVAL_SMEM_MAX = 200 * 1024;
@@ -45,8 +55,8 @@ constexpr size_t EVAL2_SMEM_MAX = 110 * 1024;
 
 struct State {
   int64_t n = 0;
-  int c = 0, r = 0, d = 0;
-  const float* post = nullptr;           // [c][ldp] posteriors
+  int c = 0, q = 0, r = 0, d = 0;       // classes, classes kept per candidate, r = q-1
+  const float* post = nullptr;           // [c][ldp] posteriors (null: kept classes given by the host)
   int64_t ldp = 0;
   const float* U = nullptr;              // [.][d] feature rows
   int64_t* rows = nullptr;               // candidate i -> row of post / U (null: identity)
@@ -54,7 +64,10 @@ struct State {
   bool have = false;                     // candidates set
   float *ownP = nullptr, *ownU = nullptr;
   int64_t cap_p = 0, cap_u = 0, cap_rows = 0;
-  double *Lall = nullptr, *Kd = nullptr; // [n][c][r], [n][r][r]
+  int* cls = nullptr;                    // [n][q] kept class ids, ascending
+  float* pk = nullptr;                   // [n][q] their posteriors
+  int64_t cap_cls = 0, cap_pk = 0;
+  double *Lall = nullptr, *Kd = nullptr; // [n][q][r], [n][r][r]
   int64_t cap_L = 0, cap_K = 0;
   unsigned char* avail = nullptr;
   int64_t cap_avail = 0;
@@ -65,6 +78,8 @@ struct State {
   int64_t cap_kss = 0, cap_m = 0, cap_z = 0, cap_lsel = 0, cap_red = 0;
   long long* sel = nullptr;
   int64_t cap_sel = 0;
+  int* Csel = nullptr;                   // [k][q] the winners' class ids
+  int64_t cap_csel = 0;
   double* blk_loss = nullptr;
   long long* blk_idx = nullptr;
   int64_t cap_blk = 0, cap_blk_idx = 0;
@@ -77,6 +92,11 @@ struct State {
   int64_t cap_a = 0, cap_w = 0;
   double *Cd = nullptr, *Pw = nullptr;   // [n][cw] candidates' own columns (set-up), [d][nq] P_w of the current winner
   int64_t cap_cd = 0, cap_pw = 0;
+  // nnal_pool_top_classes
+  int64_t* tc_rows = nullptr;
+  int* tc_cls = nullptr;
+  float* tc_p = nullptr;
+  int64_t cap_tc_rows = 0, cap_tc_cls = 0, cap_tc_p = 0;
 };
 
 static State* get(nnal_ctx* ctx) {
@@ -94,36 +114,92 @@ static int grow(nnal_ctx* ctx, T*& p, int64_t& cap, int64_t want) {
   return NNAL_OK;
 }
 
-// ---- setup: per candidate L_i (c x r) from the renormalised float64 posteriors and K_ii = L_i^T L_i (|u_i|^2 + 1) ----------
-__global__ void __launch_bounds__(256) setup_kernel(const float* __restrict__ post, int64_t ldp, const float* __restrict__ U,
-                                                    const int64_t* __restrict__ rows, int64_t n, int c, int d,
-                                                    double* __restrict__ Lall, double* __restrict__ Kd,
-                                                    unsigned char* __restrict__ avail) {
+// ---- kept classes: the q largest of c posteriors per candidate (ties: lower class index), written in ascending class order ----
+// One warp per candidate.  Lane l < q holds one kept entry; the classes stream past in chunks of 32 (one per lane), and a
+// chunk entry that beats the worst kept entry replaces it.  Requires q <= c (every placeholder gets replaced).
+__device__ inline void worst_kept(float kv, int ki, int q, float& wv, int& wi, int& wl) {
   const int lane = threadIdx.x & 31;
-  const int r = c - 1;
+  wv = lane < q ? kv : INFINITY;                              // lanes >= q never hold the worst
+  wi = lane < q ? ki : -1;
+  wl = lane;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    const float ov = __shfl_xor_sync(0xffffffffu, wv, o);
+    const int oi = __shfl_xor_sync(0xffffffffu, wi, o), ol = __shfl_xor_sync(0xffffffffu, wl, o);
+    // worst: smallest value, then largest class, then lowest lane (placeholders tie: every lane must agree on one)
+    if (ov < wv || (ov == wv && (oi > wi || (oi == wi && ol < wl)))) { wv = ov; wi = oi; wl = ol; }
+  }
+}
+
+__global__ void __launch_bounds__(256) topc_kernel(const float* __restrict__ post, int64_t ldp, const int64_t* __restrict__ rows,
+                                                   int64_t n, int c, int q, int* __restrict__ cls, float* __restrict__ pk) {
+  const int lane = threadIdx.x & 31;
   const int64_t nw = (int64_t)gridDim.x * (blockDim.x >> 5);
   for (int64_t i = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); i < n; i += nw) {
+    const int64_t row = rows ? rows[i] : i;
+    float kv = -INFINITY, wv;
+    int ki = INT_MAX, wi, wl;
+    worst_kept(kv, ki, q, wv, wi, wl);
+    for (int x0 = 0; x0 < c; x0 += 32) {
+      const int x = x0 + lane;
+      bool live = x < c;
+      const float v = live ? post[(int64_t)x * ldp + row] : 0.f;
+      while (true) {
+        const unsigned m = __ballot_sync(0xffffffffu, live && (v > wv || (v == wv && x < wi)));
+        if (!m) break;
+        const int src = __ffs(m) - 1;
+        const float nv = __shfl_sync(0xffffffffu, v, src);
+        const int nx = __shfl_sync(0xffffffffu, x, src);
+        if (lane == wl) { kv = nv; ki = nx; }
+        if (lane == src) live = false;
+        worst_kept(kv, ki, q, wv, wi, wl);
+      }
+    }
+    int rank = 0;
+    for (int l = 0; l < q; ++l) rank += __shfl_sync(0xffffffffu, ki, l) < ki;
+    if (lane < q) {
+      cls[i * q + rank] = ki;
+      pk[i * q + rank] = kv;
+    }
+  }
+}
+
+// ---- setup: per candidate L_i (q x r) from the kept posteriors renormalised in float64, K_ii = L_i^T L_i (|u_i|^2 + 1) -------
+__global__ void __launch_bounds__(256) setup_kernel(const float* __restrict__ pk, const float* __restrict__ U,
+                                                    const int64_t* __restrict__ rows, int64_t n, int q, int d,
+                                                    double* __restrict__ Lall, double* __restrict__ Kd,
+                                                    unsigned char* __restrict__ avail) {
+  __shared__ double ps[8][MAX_C], tail[8][MAX_C + 1];
+  const int lane = threadIdx.x & 31, wp = threadIdx.x >> 5;
+  const int r = q - 1;
+  double* p = ps[wp];
+  double* tl = tail[wp];
+  const int64_t nw = (int64_t)gridDim.x * (blockDim.x >> 5);
+  for (int64_t i = (int64_t)blockIdx.x * (blockDim.x >> 5) + wp; i < n; i += nw) {
     const int64_t row = rows ? rows[i] : i;
     const float* u = U + row * (int64_t)d;
     double uu = 0.0;
     for (int k = lane; k < d; k += 32) { const double v = (double)u[k]; uu = fma(v, v, uu); }
     uu = warp_sum(uu);
-    double* L = Lall + i * (int64_t)c * r;
-    if (lane == 0) {
-      double p[MAX_C], tail[MAX_C + 1];
+    if (lane < q) p[lane] = (double)pk[i * q + lane];
+    __syncwarp();
+    if (lane == 0) {                                          // ascending class order: the sums of the dense form
       double sum = 0.0;
-      for (int j = 0; j < c; ++j) { p[j] = (double)post[(int64_t)j * ldp + row]; sum += p[j]; }
-      for (int j = 0; j < c; ++j) p[j] = sum > 0.0 ? p[j] / sum : 0.0;
-      tail[c] = 0.0;
-      for (int j = c - 1; j >= 0; --j) tail[j] = tail[j + 1] + p[j];
-      for (int j = 0; j < r; ++j) {
-        const double a = tail[j], b = tail[j + 1];
-        const bool zero = !(p[j] > 0.0) || !(b > 0.0);
-        const double dj = zero ? 0.0 : sqrt(p[j] * b / a);
-        const double off = zero ? 0.0 : sqrt(p[j] / (a * b));
-        for (int i2 = 0; i2 < c; ++i2) L[i2 * r + j] = i2 < j ? 0.0 : (i2 == j ? dj : -p[i2] * off);
-      }
+      for (int j = 0; j < q; ++j) sum += p[j];
+      for (int j = 0; j < q; ++j) p[j] = sum > 0.0 ? p[j] / sum : 0.0;
+      tl[q] = 0.0;
+      for (int j = q - 1; j >= 0; --j) tl[j] = tl[j + 1] + p[j];
       avail[i] = 1;
+    }
+    __syncwarp();
+    double* L = Lall + i * (int64_t)q * r;
+    if (lane < r) {
+      const int j = lane;
+      const double a = tl[j], b = tl[j + 1];
+      const bool zero = !(p[j] > 0.0) || !(b > 0.0);
+      const double dj = zero ? 0.0 : sqrt(p[j] * b / a);
+      const double off = zero ? 0.0 : sqrt(p[j] / (a * b));
+      for (int i2 = 0; i2 < q; ++i2) L[i2 * r + j] = i2 < j ? 0.0 : (i2 == j ? dj : -p[i2] * off);
     }
     __syncwarp();
     const double sq = uu + 1.0;
@@ -131,9 +207,10 @@ __global__ void __launch_bounds__(256) setup_kernel(const float* __restrict__ po
     for (int e = lane; e < r * r; e += 32) {
       const int y = e / r, z = e - y * r;
       double acc = 0.0;
-      for (int x = 0; x < c; ++x) acc = fma(L[x * r + y], L[x * r + z], acc);
+      for (int x = 0; x < q; ++x) acc = fma(L[x * r + y], L[x * r + z], acc);
       K[e] = acc * sq;
     }
+    __syncwarp();                                             // p and tl are reused by the warp's next candidate
   }
 }
 
@@ -295,18 +372,27 @@ __global__ void __launch_bounds__(256) append2_kernel(const double* __restrict__
 }
 
 // ---- system: block row a = t-1 of K_SS (and its transpose): K[(a,y),(b,z)] = (L_{w_a}^T L_{w_b})[y,z] s_{w_a w_b} -------------
-__global__ void __launch_bounds__(256) append_kernel(const double* __restrict__ Lsel, const double* __restrict__ Scols, int64_t lds,
-                                                     const long long* __restrict__ sel, int a, int c, int r,
+// (sum over the classes both winners kept, ascending)
+__global__ void __launch_bounds__(256) append_kernel(const double* __restrict__ Lsel, const int* __restrict__ Csel,
+                                                     const double* __restrict__ Scols, int64_t lds,
+                                                     const long long* __restrict__ sel, int a, int q, int r,
                                                      double* __restrict__ Kss, int64_t ldk) {
   const int64_t total = (int64_t)(a + 1) * r * r;
-  const double* La = Lsel + (int64_t)a * c * r;
+  const double* La = Lsel + (int64_t)a * q * r;
+  const int* Ca = Csel + (int64_t)a * q;
   for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
     const int b = (int)(e / (r * r));
     const int yz = (int)(e - (int64_t)b * r * r);
     const int y = yz / r, z = yz - (yz / r) * r;
-    const double* Lb = Lsel + (int64_t)b * c * r;
+    const double* Lb = Lsel + (int64_t)b * q * r;
+    const int* Cb = Csel + (int64_t)b * q;
     double acc = 0.0;
-    for (int x = 0; x < c; ++x) acc = fma(La[x * r + y], Lb[x * r + z], acc);
+    for (int xa = 0, xb = 0; xa < q && xb < q;) {
+      const int ga = Ca[xa], gb = Cb[xb];
+      if (ga == gb) acc = fma(La[xa * r + y], Lb[xb * r + z], acc);
+      xa += ga <= gb;
+      xb += gb <= ga;
+    }
     const double v = acc * Scols[(int64_t)a * lds + sel[b]];
     Kss[(int64_t)(a * r + y) * ldk + b * r + z] = v;
     Kss[(int64_t)(b * r + z) * ldk + a * r + y] = v;
@@ -322,17 +408,17 @@ __global__ void __launch_bounds__(256) build_kernel(const double* __restrict__ K
   }
 }
 
-// Z[rho, (a,x)] = sum_y C[rho, (a,y)] L_{w_a}[x,y]
-__global__ void __launch_bounds__(256) z_kernel(const double* __restrict__ Cm, int np, const double* __restrict__ Lsel, int t, int c,
+// Z[rho, (a,x)] = sum_y C[rho, (a,y)] L_{w_a}[x,y]   (x: winner a's kept classes)
+__global__ void __launch_bounds__(256) z_kernel(const double* __restrict__ Cm, int np, const double* __restrict__ Lsel, int t, int q,
                                                 int r, double* __restrict__ Z, int64_t ldz) {
   const int m = t * r;
-  const int64_t total = (int64_t)m * t * c;
+  const int64_t total = (int64_t)m * t * q;
   for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
-    const int rho = (int)(e / ((int64_t)t * c));
-    const int col = (int)(e - (int64_t)rho * t * c);
-    const int a = col / c, x = col - (col / c) * c;
+    const int rho = (int)(e / ((int64_t)t * q));
+    const int col = (int)(e - (int64_t)rho * t * q);
+    const int a = col / q, x = col - (col / q) * q;
     const double* Crow = Cm + (int64_t)rho * np + a * r;
-    const double* La = Lsel + (int64_t)a * c * r + x * r;
+    const double* La = Lsel + (int64_t)a * q * r + x * r;
     double acc = 0.0;
     for (int y = 0; y < r; ++y) acc = fma(Crow[y], La[y], acc);
     Z[(int64_t)rho * ldz + col] = acc;
@@ -357,29 +443,32 @@ __global__ void __launch_bounds__(256) trace_kernel(const double* __restrict__ C
 struct EvalArgs {
   const double* Lall; const double* Kd; const double* Z; int64_t ldz;
   const double* Scols; int64_t lds;
+  const int* cls; int* Csel;
   double* Lsel; unsigned char* avail;
-  int64_t n; int c, r, t, JC, AT, cw; double alpha;
+  int64_t n; int q, r, t, JC, AT, cw; double alpha;
   const double* trC;
   double* blk_loss; long long* blk_idx; unsigned int* ticket;
   long long* sel; double* red;
 };
 
 struct EvalLayout {
-  int Ls, E, G, Zs, Ss, Ws, Ys, Ks, loss, total;     // offsets in doubles
+  int Ls, E, G, Zs, Ss, Ws, Ys, Ks, loss, Cj, Ct, total;     // offsets in doubles (Cj, Ct: int arrays)
 };
 
-__host__ __device__ inline EvalLayout eval_layout(int JC, int AT, int c, int r, int cw) {
+__host__ __device__ inline EvalLayout eval_layout(int JC, int AT, int q, int r, int cw) {
   EvalLayout l;
   int o = 0;
-  l.Ls = o; o += JC * c * r;
+  l.Ls = o; o += JC * q * r;
   l.E = o; o += JC * r * r;
   l.G = o; o += JC * r * r;
-  l.Zs = o; o += RT * AT * c;
+  l.Zs = o; o += RT * AT * q;
   l.Ss = o; o += AT * JC * cw;
-  l.Ws = o; o += JC * RT * c;
+  l.Ws = o; o += JC * RT * q;
   l.Ys = o; o += JC * RT * r;
   l.Ks = o; o += JC * RT * r;
   l.loss = o; o += JC;
+  l.Cj = o; o += (JC * q + 1) / 2;
+  l.Ct = o; o += (AT * q + 1) / 2;
   l.total = o;
   return l;
 }
@@ -413,12 +502,25 @@ __device__ double block_loss(double* __restrict__ Sg, const double* __restrict__
   return tr;
 }
 
-// NL = 2: Ss holds the winners' whole columns [AT][JC][cw], W_j sums Z[:, a-block] N_{w_a j}, and k_j = L^T N L
-template <int NL>
+// position of class g in the ascending list C[0..q-1], -1 if absent: first try `hint` (exact for the identity list), else bisect
+__device__ inline int find_class(const int* C, int q, int g, int hint) {
+  if (C[hint] == g) return hint;
+  int lo = 0, hi = q;
+  while (lo < hi) {
+    const int mid = (lo + hi) >> 1;
+    if (C[mid] < g) lo = mid + 1;
+    else hi = mid;
+  }
+  return lo < q && C[lo] == g ? lo : -1;
+}
+
+// NL = 2: Ss holds the winners' whole columns [AT][JC][cw], W_j sums Z[:, a-block] N_{w_a j}, and k_j = L^T N L (q = c).
+// ALL: every candidate keeps every class (q = c), so each id list is 0..c-1 and every class lookup is its hint.
+template <int NL, bool ALL>
 __global__ void __launch_bounds__(EVAL_THREADS) eval_kernel(EvalArgs ea) {
   extern __shared__ __align__(16) double sm[];
-  const int c = ea.c, r = ea.r, t = ea.t, JC = ea.JC, AT = ea.AT, cw = NL == 2 ? ea.cw : 1;
-  const EvalLayout lay = eval_layout(JC, AT, c, r, cw);
+  const int q = ea.q, r = ea.r, t = ea.t, JC = ea.JC, AT = ea.AT, cw = NL == 2 ? ea.cw : 1;
+  const EvalLayout lay = eval_layout(JC, AT, q, r, cw);
   double* Ls = sm + lay.Ls;
   double* E = sm + lay.E;
   double* G = sm + lay.G;
@@ -428,34 +530,38 @@ __global__ void __launch_bounds__(EVAL_THREADS) eval_kernel(EvalArgs ea) {
   double* Ys = sm + lay.Ys;
   double* Ks = sm + lay.Ks;
   double* lossv = sm + lay.loss;
+  int* Cj = (int*)(sm + lay.Cj);                  // [JC][q] the candidates' class ids
+  int* Ct = (int*)(sm + lay.Ct);                  // [AT][q] class ids of the winners in the Z tile
   const int tid = threadIdx.x;
   const int64_t j0 = (int64_t)blockIdx.x * JC;
-  for (int e = tid; e < JC * c * r; e += blockDim.x) {
-    const int64_t j = j0 + e / (c * r);
-    Ls[e] = j < ea.n ? ea.Lall[j0 * c * r + e] : 0.0;
+  for (int e = tid; e < JC * q * r; e += blockDim.x) {
+    const int64_t j = j0 + e / (q * r);
+    Ls[e] = j < ea.n ? ea.Lall[j0 * q * r + e] : 0.0;
   }
+  for (int e = tid; e < JC * q; e += blockDim.x) Cj[e] = j0 + e / q < ea.n ? ea.cls[j0 * q + e] : -1;
   for (int e = tid; e < 2 * JC * r * r; e += blockDim.x) E[e] = 0.0;      // E and G are adjacent
   const int m = t * r;
-  const int ZW = AT * c;
+  const int ZW = AT * q;
   for (int rho0 = 0; rho0 < m; rho0 += RT) {
-    // W_j[rho, x] = sum_a s_{w_a j} Z[rho, (a,x)]
-    const bool wt = tid < JC * c;
-    const int wj = wt ? tid / c : 0, wx = wt ? tid - (tid / c) * c : 0;
+    // W_j[rho, x'] = sum_a s_{w_a j} Z[rho, (a,x)],  cls_{w_a}[x] = cls_j[x']
+    const bool wt = tid < JC * q;
+    const int wj = wt ? tid / q : 0, wx = wt ? tid - (tid / q) * q : 0;
     double acc[RT];
 #pragma unroll
-    for (int q = 0; q < RT; ++q) acc[q] = 0.0;
+    for (int qq = 0; qq < RT; ++qq) acc[qq] = 0.0;
     for (int a0 = 0; a0 < t; a0 += AT) {
       __syncthreads();
       for (int e = tid; e < RT * ZW; e += blockDim.x) {
-        const int q = e / ZW, col = e - q * ZW;
-        const int a = a0 + col / c;
-        Zs[e] = (rho0 + q < m && a < t) ? ea.Z[(int64_t)(rho0 + q) * ea.ldz + (int64_t)a0 * c + col] : 0.0;
+        const int qq = e / ZW, col = e - qq * ZW;
+        const int a = a0 + col / q;
+        Zs[e] = (rho0 + qq < m && a < t) ? ea.Z[(int64_t)(rho0 + qq) * ea.ldz + (int64_t)a0 * q + col] : 0.0;
       }
       if constexpr (NL == 1) {
         for (int e = tid; e < AT * JC; e += blockDim.x) {
           const int a = e / JC, jj = e - a * JC;
           Ss[e] = (a0 + a < t && j0 + jj < ea.n) ? ea.Scols[(int64_t)(a0 + a) * ea.lds + j0 + jj] : 0.0;
         }
+        for (int e = tid; e < AT * q; e += blockDim.x) Ct[e] = a0 + e / q < t ? ea.Csel[(int64_t)a0 * q + e] : -1;
       } else {
         for (int e = tid; e < AT * JC * cw; e += blockDim.x) {
           const int a = e / (JC * cw), jf = e - a * JC * cw;
@@ -467,15 +573,18 @@ __global__ void __launch_bounds__(EVAL_THREADS) eval_kernel(EvalArgs ea) {
         const int na = min(AT, t - a0);
         for (int a = 0; a < na; ++a) {
           if constexpr (NL == 1) {
-            const double sa = Ss[a * JC + wj];
+            const int x = ALL ? wx : find_class(Ct + a * q, q, Cj[wj * q + wx], wx);
+            if (x >= 0) {
+              const double sa = Ss[a * JC + wj];
 #pragma unroll
-            for (int q = 0; q < RT; ++q) acc[q] = fma(sa, Zs[q * ZW + a * c + wx], acc[q]);
+              for (int qq = 0; qq < RT; ++qq) acc[qq] = fma(sa, Zs[qq * ZW + a * q + x], acc[qq]);
+            }
           } else {
             const double* col = Ss + (a * JC + wj) * cw;           // N[x, wx] = s [x == wx] + s' Q[x, wx]
-            for (int x = 0; x < c; ++x) {
-              const double nx = fma(col[1], col[2 + qidx(x, wx, c)], x == wx ? col[0] : 0.0);
+            for (int x = 0; x < q; ++x) {
+              const double nx = fma(col[1], col[2 + qidx(x, wx, q)], x == wx ? col[0] : 0.0);
 #pragma unroll
-              for (int q = 0; q < RT; ++q) acc[q] = fma(nx, Zs[q * ZW + a * c + x], acc[q]);
+              for (int qq = 0; qq < RT; ++qq) acc[qq] = fma(nx, Zs[qq * ZW + a * q + x], acc[qq]);
             }
           }
         }
@@ -483,34 +592,38 @@ __global__ void __launch_bounds__(EVAL_THREADS) eval_kernel(EvalArgs ea) {
     }
     if (wt) {
 #pragma unroll
-      for (int q = 0; q < RT; ++q) Ws[(wj * RT + q) * c + wx] = acc[q];
+      for (int qq = 0; qq < RT; ++qq) Ws[(wj * RT + qq) * q + wx] = acc[qq];
     }
     __syncthreads();
-    // Y_j[rho, y] = W_j[rho, :] L_j[:, y];   k_j[rho, y] = s_{w_a' j} (L_{w_a'}^T L_j)[x', y],  rho = (a', x')
+    // Y_j[rho, y] = W_j[rho, :] L_j[:, y];   k_j[rho, y] = s_{w_a' j} (L_{w_a'}^T L_j)[x', y] over shared classes,  rho = (a', x')
     if (tid < JC * r) {
       const int jj = tid / r, y = tid - (tid / r) * r;
       const int64_t j = j0 + jj;
-      const double* Lj = Ls + jj * c * r;
-      for (int q = 0; q < RT; ++q) {
-        const int row = rho0 + q;
+      const double* Lj = Ls + jj * q * r;
+      for (int qq = 0; qq < RT; ++qq) {
+        const int row = rho0 + qq;
         double yv = 0.0, kv = 0.0;
         if (row < m && j < ea.n) {
           const int ap = row / r, xp = row - (row / r) * r;
-          const double* Wq = Ws + (jj * RT + q) * c;
+          const double* Wq = Ws + (jj * RT + qq) * q;
           if constexpr (NL == 1) {
-            const double* La = ea.Lsel + (int64_t)ap * c * r + xp;
-            for (int x = 0; x < c; ++x) {
-              yv = fma(Wq[x], Lj[x * r + y], yv);
-              kv = fma(La[x * r], Lj[x * r + y], kv);
+            const double* La = ea.Lsel + (int64_t)ap * q * r + xp;
+            const int* Ca = ea.Csel + (int64_t)ap * q;
+            const int* Cjj = Cj + jj * q;
+            for (int x = 0; x < q; ++x) {                      // j's classes ascending: the shared ones in class order
+              const double lj = Lj[x * r + y];
+              yv = fma(Wq[x], lj, yv);
+              const int xa = ALL ? x : find_class(Ca, q, Cjj[x], x);
+              if (xa >= 0) kv = fma(La[xa * r], lj, kv);
             }
             kv *= ea.Scols[(int64_t)ap * ea.lds + j];
           } else {
-            for (int x = 0; x < c; ++x) yv = fma(Wq[x], Lj[x * r + y], yv);
-            kv = lnl(ea.Lsel + (int64_t)ap * c * r, Lj, ea.Scols + (int64_t)ap * ea.lds + j * cw, c, r, xp, y);
+            for (int x = 0; x < q; ++x) yv = fma(Wq[x], Lj[x * r + y], yv);
+            kv = lnl(ea.Lsel + (int64_t)ap * q * r, Lj, ea.Scols + (int64_t)ap * ea.lds + j * cw, q, r, xp, y);
           }
         }
-        Ys[(jj * RT + q) * r + y] = yv;
-        Ks[(jj * RT + q) * r + y] = kv;
+        Ys[(jj * RT + qq) * r + y] = yv;
+        Ks[(jj * RT + qq) * r + y] = kv;
       }
     }
     __syncthreads();
@@ -524,9 +637,9 @@ __global__ void __launch_bounds__(EVAL_THREADS) eval_kernel(EvalArgs ea) {
       for (int z = 0; z < r; ++z) {
         double e = Ej[z], g = Gj[z];
 #pragma unroll
-        for (int q = 0; q < RT; ++q) {
-          e = fma(Yj[q * r + y], Yj[q * r + z], e);
-          g = fma(Kj[q * r + y], Yj[q * r + z], g);
+        for (int qq = 0; qq < RT; ++qq) {
+          e = fma(Yj[qq * r + y], Yj[qq * r + z], e);
+          g = fma(Kj[qq * r + y], Yj[qq * r + z], g);
         }
         Ej[z] = e;
         Gj[z] = g;
@@ -578,7 +691,8 @@ __global__ void __launch_bounds__(EVAL_THREADS) eval_kernel(EvalArgs ea) {
     win = bi;
   }
   __syncthreads();
-  for (int e = tid; e < c * r; e += blockDim.x) ea.Lsel[(int64_t)t * c * r + e] = ea.Lall[win * c * r + e];
+  for (int e = tid; e < q * r; e += blockDim.x) ea.Lsel[(int64_t)t * q * r + e] = ea.Lall[win * q * r + e];
+  for (int e = tid; e < q; e += blockDim.x) ea.Csel[(int64_t)t * q + e] = ea.cls[win * q + e];
 }
 
 static int warp_grid(nnal_ctx* ctx, int64_t n) {
@@ -592,11 +706,11 @@ static int flat_grid(nnal_ctx* ctx, int64_t total) {
 
 // candidates per eval CTA and winners per Z tile: as many candidates as 256 threads cover, fewer where shared memory runs out
 // (two layers: at most EVAL2_SMEM_MAX, so that two CTAs share an SM)
-static void eval_plan(int c, int r, int cw, int* JC, int* AT, size_t* smem) {
+static void eval_plan(int q, int r, int cw, int* JC, int* AT, size_t* smem) {
   const size_t cap = cw == 1 ? EVAL_SMEM_MAX : EVAL2_SMEM_MAX;
-  int jc = std::max(1, std::min(64, EVAL_THREADS / c)), at = 32;
+  int jc = std::max(1, std::min(64, EVAL_THREADS / q)), at = 32;
   while (true) {
-    const size_t bytes = (size_t)eval_layout(jc, at, c, r, cw).total * sizeof(double);
+    const size_t bytes = (size_t)eval_layout(jc, at, q, r, cw).total * sizeof(double);
     if (bytes <= cap || (jc == 1 && at == 1)) { *JC = jc; *AT = at; *smem = bytes; return; }
     if (at > (cw == 1 ? 8 : 1)) at /= 2;
     else if (jc > 1) --jc;
@@ -618,10 +732,20 @@ static int check_fits(nnal_ctx* ctx, double want, double held, const char* what)
   return NNAL_OK;
 }
 
+// kept classes of n candidates (rows: positions in post, null = identity) into cls / pk [n][q]
+static void launch_topc(nnal_ctx* ctx, const float* post, int64_t ldp, const int64_t* rows, int64_t n, int c, int q, int* cls,
+                        float* pk) {
+  topc_kernel<<<warp_grid(ctx, n), 256, 0, ctx->stream>>>(post, ldp, rows, n, c, q, cls, pk);
+  ctx->launches++;
+}
+
+// s->post set: kept classes are selected from it first; null: s->cls / s->pk already hold them
 static int setup(nnal_ctx* ctx, State* s) {
   const int64_t n = s->n;
-  const int c = s->c, r = s->r;
-  NNAL_TRY(grow(ctx, s->Lall, s->cap_L, n * c * r));
+  const int c = s->c, q = s->q, r = s->r;
+  NNAL_TRY(grow(ctx, s->cls, s->cap_cls, n * q));
+  NNAL_TRY(grow(ctx, s->pk, s->cap_pk, n * q));
+  NNAL_TRY(grow(ctx, s->Lall, s->cap_L, n * q * r));
   NNAL_TRY(grow(ctx, s->Kd, s->cap_K, n * r * r));
   NNAL_TRY(grow(ctx, s->avail, s->cap_avail, n));
   if (s->nl == 2) {
@@ -631,7 +755,8 @@ static int setup(nnal_ctx* ctx, State* s) {
   }
   if (n == 0) return NNAL_OK;
   const int64_t* rows = s->use_rows ? s->rows : nullptr;
-  setup_kernel<<<warp_grid(ctx, n), 256, 0, ctx->stream>>>(s->post, s->ldp, s->U, rows, n, c, s->d, s->Lall, s->Kd, s->avail);
+  if (s->post) launch_topc(ctx, s->post, s->ldp, rows, n, c, q, s->cls, s->pk);
+  setup_kernel<<<warp_grid(ctx, n), 256, 0, ctx->stream>>>(s->pk, s->U, rows, n, q, s->d, s->Lall, s->Kd, s->avail);
   ctx->launches++;
   if (s->nl == 2) {
     dots2_kernel<<<warp_grid(ctx, n), 256, 0, ctx->stream>>>(s->U, s->A, rows, n, s->d, s->dp, nullptr, 0, s->Cd, s->cw);
@@ -650,29 +775,17 @@ static void set_layers(State* s, int nl, int c, int dp, const float* A, const fl
   s->dp = nl == 2 ? dp : 0;
   s->A = nl == 2 ? A : nullptr;
   s->W3 = nl == 2 ? W3 : nullptr;
-  s->nq = c * (c + 1) / 2;
+  s->nq = nl == 2 ? c * (c + 1) / 2 : 0;
   s->cw = nl == 2 ? s->nq + 2 : 1;
 }
 
-}  // namespace fib
-
-int nnal_fi_block_release(nnal_ctx* ctx) {
-  if (!ctx->fi_block_state) return NNAL_OK;
-  fib::State* s = (fib::State*)ctx->fi_block_state;
-  void* ptrs[] = {s->ownP, s->ownU, s->rows, s->Lall, s->Kd, s->avail, s->Scols, s->Kss, s->M, s->Z, s->Lsel, s->red, s->trC,
-                  s->sel, s->blk_loss, s->blk_idx, s->ticket, s->ownA, s->ownW, s->Cd, s->Pw};
-  for (void* p : ptrs) if (p) cudaFree(p);
-  delete s;
-  ctx->fi_block_state = nullptr;
-  return NNAL_OK;
-}
-
-extern "C" int nnal_fi_block_set_candidates_nl(nnal_ctx* ctx, const int64_t* cand, int64_t n_cand, int n_layers) {
+// cap = 0: every class (c <= MAX_C); else the min(cap, c) most probable, 2 <= cap <= MAX_C (one layer)
+static int set_candidates(nnal_ctx* ctx, const int64_t* cand, int64_t n_cand, int n_layers, int cap) {
   if (!ctx || n_cand < 0) return NNAL_ERR_INVALID;
   if (n_layers != 1 && n_layers != 2) NNAL_FAIL(ctx, NNAL_ERR_INVALID, "block FI covers the last 1 or 2 fully-connected layers");
   if (!ctx->pool_post || !ctx->pool_feat || ctx->keep < 1) NNAL_FAIL(ctx, NNAL_ERR_STATE, "pool pass did not keep the feature layer");
   if (n_layers == 2 && (!ctx->pool_prev || ctx->keep < 2)) NNAL_FAIL(ctx, NNAL_ERR_STATE, "pool pass did not keep the previous FC output");
-  if (ctx->n_class < 2 || ctx->n_class > fib::MAX_C) NNAL_FAIL(ctx, NNAL_ERR_UNSUPPORTED, "block FI supports 2 <= c <= 32");
+  if (ctx->n_class < 2 || (!cap && ctx->n_class > MAX_C)) NNAL_FAIL(ctx, NNAL_ERR_UNSUPPORTED, "block FI supports 2 <= c <= 32");
   if (ctx->feature_layer != (int)ctx->layers.size() - 2) NNAL_FAIL(ctx, NNAL_ERR_UNSUPPORTED, "feature layer must feed the last FC layer");
   if (n_layers == 2 && (ctx->feature_layer < 1 || ctx->layers[ctx->feature_layer - 1].type != NNAL_LAYER_FC))
     NNAL_FAIL(ctx, NNAL_ERR_UNSUPPORTED, "two-layer block FI needs an FC layer before the feature layer");
@@ -681,24 +794,47 @@ extern "C" int nnal_fi_block_set_candidates_nl(nnal_ctx* ctx, const int64_t* can
   if (cand)
     for (int64_t i = 0; i < n; ++i)
       if (cand[i] < 0 || cand[i] >= ctx->pool_n) NNAL_FAIL(ctx, NNAL_ERR_INVALID, "candidate position outside the pool");
-  fib::State* s = fib::get(ctx);
+  State* s = get(ctx);
   s->have = false;
-  s->n = n; s->c = ctx->n_class; s->r = ctx->n_class - 1; s->d = ctx->feat_dim;
+  s->n = n; s->c = ctx->n_class; s->q = cap ? std::min(cap, s->c) : s->c; s->r = s->q - 1; s->d = ctx->feat_dim;
   s->post = ctx->pool_post; s->ldp = ctx->pool_n; s->U = ctx->pool_feat;
-  fib::set_layers(s, n_layers, s->c, ctx->prev_dim, ctx->pool_prev, ctx->layers.back().W);
+  set_layers(s, n_layers, s->c, ctx->prev_dim, ctx->pool_prev, ctx->layers.back().W);
   s->use_rows = cand != nullptr;
   if (cand && n) {
-    NNAL_TRY(fib::grow(ctx, s->rows, s->cap_rows, n));
+    NNAL_TRY(grow(ctx, s->rows, s->cap_rows, n));
     CUDA_TRY(ctx, cudaMemcpyAsync(s->rows, cand, (size_t)n * 8, cudaMemcpyHostToDevice, ctx->stream));
   }
-  NNAL_TRY(fib::setup(ctx, s));
+  NNAL_TRY(setup(ctx, s));
   NNAL_SYNC_CHECKED(ctx);                                 // `cand` is caller-owned host memory; fp16 range flag of the pool pass
   s->have = true;
   return NNAL_OK;
 }
 
+}  // namespace fib
+
+int nnal_fi_block_release(nnal_ctx* ctx) {
+  if (!ctx->fi_block_state) return NNAL_OK;
+  fib::State* s = (fib::State*)ctx->fi_block_state;
+  void* ptrs[] = {s->ownP, s->ownU, s->rows, s->cls, s->pk, s->Lall, s->Kd, s->avail, s->Scols, s->Kss, s->M, s->Z, s->Lsel,
+                  s->Csel, s->red, s->trC, s->sel, s->blk_loss, s->blk_idx, s->ticket, s->ownA, s->ownW, s->Cd, s->Pw,
+                  s->tc_rows, s->tc_cls, s->tc_p};
+  for (void* p : ptrs) if (p) cudaFree(p);
+  delete s;
+  ctx->fi_block_state = nullptr;
+  return NNAL_OK;
+}
+
+extern "C" int nnal_fi_block_set_candidates_nl(nnal_ctx* ctx, const int64_t* cand, int64_t n_cand, int n_layers) {
+  return fib::set_candidates(ctx, cand, n_cand, n_layers, 0);
+}
+
 extern "C" int nnal_fi_block_set_candidates(nnal_ctx* ctx, const int64_t* cand, int64_t n_cand) {
-  return nnal_fi_block_set_candidates_nl(ctx, cand, n_cand, 1);
+  return fib::set_candidates(ctx, cand, n_cand, 1, 0);
+}
+
+extern "C" int nnal_fi_block_set_candidates_cls(nnal_ctx* ctx, const int64_t* cand, int64_t n_cand, int r) {
+  if (ctx && (r < 2 || r > fib::MAX_C)) NNAL_FAIL(ctx, NNAL_ERR_INVALID, "block FI keeps 2 to 32 classes per candidate");
+  return fib::set_candidates(ctx, cand, n_cand, 1, r);
 }
 
 extern "C" int nnal_fi_block_set_factors_nl(nnal_ctx* ctx, int64_t n, int c, int d, int d_prev, const float* post, const float* U,
@@ -710,7 +846,7 @@ extern "C" int nnal_fi_block_set_factors_nl(nnal_ctx* ctx, int64_t n, int c, int
   CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   fib::State* s = fib::get(ctx);
   s->have = false;
-  s->n = n; s->c = c; s->r = c - 1; s->d = d;
+  s->n = n; s->c = c; s->q = c; s->r = c - 1; s->d = d;
   NNAL_TRY(fib::grow(ctx, s->ownP, s->cap_p, n * c));
   NNAL_TRY(fib::grow(ctx, s->ownU, s->cap_u, n * d));
   if (n) {
@@ -735,29 +871,88 @@ extern "C" int nnal_fi_block_set_factors(nnal_ctx* ctx, int64_t n, int c, int d,
   return nnal_fi_block_set_factors_nl(ctx, n, c, d, 0, post, U, nullptr, nullptr);
 }
 
+extern "C" int nnal_fi_block_set_factors_cls(nnal_ctx* ctx, int64_t n, int c, int r, int d, const int32_t* cls, const float* p,
+                                             const float* U) {
+  if (!ctx || n < 0 || d <= 0 || (n > 0 && (!cls || !p || !U))) return NNAL_ERR_INVALID;
+  if (c < 2) NNAL_FAIL(ctx, NNAL_ERR_INVALID, "block FI needs c >= 2 classes");
+  if (r < 2 || r > fib::MAX_C || r > c) NNAL_FAIL(ctx, NNAL_ERR_INVALID, "block FI keeps 2 to min(32, c) classes per candidate");
+  for (int64_t i = 0; i < n; ++i)
+    for (int x = 0; x < r; ++x) {
+      const int32_t g = cls[i * r + x];
+      if (g < 0 || g >= c) NNAL_FAIL(ctx, NNAL_ERR_INVALID, "kept class id outside 0..c-1");
+      if (x > 0 && !(g > cls[i * r + x - 1])) NNAL_FAIL(ctx, NNAL_ERR_INVALID, "kept class ids must be strictly ascending");
+    }
+  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  fib::State* s = fib::get(ctx);
+  s->have = false;
+  s->n = n; s->c = c; s->q = r; s->r = r - 1; s->d = d;
+  NNAL_TRY(fib::grow(ctx, s->cls, s->cap_cls, n * r));
+  NNAL_TRY(fib::grow(ctx, s->pk, s->cap_pk, n * r));
+  NNAL_TRY(fib::grow(ctx, s->ownU, s->cap_u, n * d));
+  if (n) {
+    CUDA_TRY(ctx, cudaMemcpyAsync(s->cls, cls, (size_t)n * r * 4, cudaMemcpyHostToDevice, ctx->stream));
+    CUDA_TRY(ctx, cudaMemcpyAsync(s->pk, p, (size_t)n * r * 4, cudaMemcpyHostToDevice, ctx->stream));
+    CUDA_TRY(ctx, cudaMemcpyAsync(s->ownU, U, (size_t)n * d * 4, cudaMemcpyHostToDevice, ctx->stream));
+  }
+  s->post = nullptr; s->ldp = 0; s->U = s->ownU; s->use_rows = false;
+  fib::set_layers(s, 1, c, 0, nullptr, nullptr);
+  NNAL_TRY(fib::setup(ctx, s));
+  CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+  s->have = true;
+  return NNAL_OK;
+}
+
+extern "C" int nnal_pool_top_classes(nnal_ctx* ctx, const int64_t* rows, int64_t n, int r, int32_t* cls_out, float* p_out) {
+  if (!ctx || n < 0 || (n > 0 && (!cls_out || !p_out))) return NNAL_ERR_INVALID;
+  if (r < 2 || r > fib::MAX_C) NNAL_FAIL(ctx, NNAL_ERR_INVALID, "block FI keeps 2 to 32 classes per candidate");
+  if (!ctx->pool_post) NNAL_FAIL(ctx, NNAL_ERR_STATE, "no pool pass");
+  if (!rows && n > ctx->pool_n) NNAL_FAIL(ctx, NNAL_ERR_INVALID, "more rows than the pool holds");
+  if (rows)
+    for (int64_t i = 0; i < n; ++i)
+      if (rows[i] < 0 || rows[i] >= ctx->pool_n) NNAL_FAIL(ctx, NNAL_ERR_INVALID, "row outside the pool");
+  if (n == 0) return NNAL_OK;
+  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  fib::State* s = fib::get(ctx);
+  const int c = ctx->n_class, q = std::min(r, c);
+  NNAL_TRY(fib::grow(ctx, s->tc_cls, s->cap_tc_cls, n * q));
+  NNAL_TRY(fib::grow(ctx, s->tc_p, s->cap_tc_p, n * q));
+  if (rows) {
+    NNAL_TRY(fib::grow(ctx, s->tc_rows, s->cap_tc_rows, n));
+    CUDA_TRY(ctx, cudaMemcpyAsync(s->tc_rows, rows, (size_t)n * 8, cudaMemcpyHostToDevice, ctx->stream));
+  }
+  fib::launch_topc(ctx, ctx->pool_post, ctx->pool_n, rows ? s->tc_rows : nullptr, n, c, q, s->tc_cls, s->tc_p);
+  CUDA_TRY(ctx, cudaGetLastError());
+  CUDA_TRY(ctx, cudaMemcpyAsync(cls_out, s->tc_cls, (size_t)n * q * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  CUDA_TRY(ctx, cudaMemcpyAsync(p_out, s->tc_p, (size_t)n * q * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+  return NNAL_OK;
+}
+
 extern "C" int nnal_fi_block_greedy(nnal_ctx* ctx, int64_t k, double delta, int64_t* sel_out, double* obj_out, double* red_out) {
   if (!ctx || k < 0 || !(delta > 0) || (k > 0 && !sel_out)) return NNAL_ERR_INVALID;
   if (!ctx->fi_block_state || !((fib::State*)ctx->fi_block_state)->have) NNAL_FAIL(ctx, NNAL_ERR_STATE, "block FI candidates not set");
   fib::State* s = (fib::State*)ctx->fi_block_state;
   const int64_t n = s->n;
-  const int c = s->c, r = s->r, cw = s->cw;
+  const int c = s->c, q = s->q, r = s->r, cw = s->cw;
   if (k > n) k = n;
-  if (k * r > fib::MAX_KR) NNAL_FAIL(ctx, NNAL_ERR_UNSUPPORTED, "block FI greedy supports k (c-1) <= 4096");
+  if (k * r > fib::MAX_KR)
+    NNAL_FAIL(ctx, NNAL_ERR_UNSUPPORTED, "block FI greedy supports k (q-1) <= 4096, q = classes kept per candidate (c without a cap)");
   if (k == 0) return NNAL_OK;
   CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   const int64_t mmax = k * r;
   const int npmax = (int)((mmax + 63) / 64 * 64);
-  const int64_t ldk = mmax, ldz = k * c, lds = n * cw;    // column t of candidate j, entry e: Scols[t lds + j cw + e]
+  const int64_t ldk = mmax, ldz = k * q, lds = n * cw;    // column t of candidate j, entry e: Scols[t lds + j cw + e]
   int JC, AT;
   size_t smem;
-  fib::eval_plan(c, r, cw, &JC, &AT, &smem);
+  fib::eval_plan(q, r, cw, &JC, &AT, &smem);
   const int nblk = (int)((n + JC - 1) / JC);
   if (s->nl == 2) NNAL_TRY(fib::check_fits(ctx, 8.0 * k * lds, 8.0 * s->cap_scols, "the winners' columns"));
   NNAL_TRY(fib::grow(ctx, s->Scols, s->cap_scols, k * lds));
   NNAL_TRY(fib::grow(ctx, s->Kss, s->cap_kss, mmax * mmax));
   NNAL_TRY(fib::grow(ctx, s->M, s->cap_m, (int64_t)npmax * npmax));
   NNAL_TRY(fib::grow(ctx, s->Z, s->cap_z, mmax * ldz));
-  NNAL_TRY(fib::grow(ctx, s->Lsel, s->cap_lsel, k * c * r));
+  NNAL_TRY(fib::grow(ctx, s->Lsel, s->cap_lsel, k * q * r));
+  NNAL_TRY(fib::grow(ctx, s->Csel, s->cap_csel, k * q));
   NNAL_TRY(fib::grow(ctx, s->red, s->cap_red, k));
   NNAL_TRY(fib::grow(ctx, s->sel, s->cap_sel, k));
   NNAL_TRY(fib::grow(ctx, s->blk_loss, s->cap_blk, (int64_t)nblk));
@@ -769,16 +964,17 @@ extern "C" int nnal_fi_block_greedy(nnal_ctx* ctx, int64_t k, double delta, int6
   }
   static bool attr = false;
   if (!attr) {
-    CUDA_TRY(ctx, cudaFuncSetAttribute(fib::eval_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fib::EVAL_SMEM_MAX));
-    CUDA_TRY(ctx, cudaFuncSetAttribute(fib::eval_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fib::EVAL_SMEM_MAX));
+    CUDA_TRY(ctx, cudaFuncSetAttribute(fib::eval_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fib::EVAL_SMEM_MAX));
+    CUDA_TRY(ctx, cudaFuncSetAttribute(fib::eval_kernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fib::EVAL_SMEM_MAX));
+    CUDA_TRY(ctx, cudaFuncSetAttribute(fib::eval_kernel<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fib::EVAL_SMEM_MAX));
     attr = true;
   }
   CUDA_TRY(ctx, cudaMemsetAsync(s->avail, 1, (size_t)n, ctx->stream));
   CUDA_TRY(ctx, cudaMemsetAsync(s->trC, 0, sizeof(double), ctx->stream));
   const int64_t* rows = s->use_rows ? s->rows : nullptr;
   fib::EvalArgs ea;
-  ea.Lall = s->Lall; ea.Kd = s->Kd; ea.Z = s->Z; ea.ldz = ldz; ea.Scols = s->Scols; ea.lds = lds;
-  ea.Lsel = s->Lsel; ea.avail = s->avail; ea.n = n; ea.c = c; ea.r = r; ea.JC = JC; ea.AT = AT; ea.cw = cw;
+  ea.Lall = s->Lall; ea.Kd = s->Kd; ea.Z = s->Z; ea.ldz = ldz; ea.Scols = s->Scols; ea.lds = lds; ea.cls = s->cls; ea.Csel = s->Csel;
+  ea.Lsel = s->Lsel; ea.avail = s->avail; ea.n = n; ea.q = q; ea.r = r; ea.JC = JC; ea.AT = AT; ea.cw = cw;
   ea.trC = s->trC; ea.blk_loss = s->blk_loss; ea.blk_idx = s->blk_idx; ea.ticket = s->ticket; ea.sel = s->sel; ea.red = s->red;
   for (int t = 0; t < (int)k; ++t) {
     const double alpha = (double)(t + 1) * delta;
@@ -790,12 +986,12 @@ extern "C" int nnal_fi_block_greedy(nnal_ctx* ctx, int64_t k, double delta, int6
         fib::append2_kernel<<<fib::flat_grid(ctx, (int64_t)t * r * r), 256, 0, ctx->stream>>>(s->Lsel, s->Scols, lds, cw, s->sel,
                                                                                                 t - 1, c, r, s->Kss, ldk);
       else
-        fib::append_kernel<<<fib::flat_grid(ctx, (int64_t)t * r * r), 256, 0, ctx->stream>>>(s->Lsel, s->Scols, lds, s->sel, t - 1,
-                                                                                               c, r, s->Kss, ldk);
+        fib::append_kernel<<<fib::flat_grid(ctx, (int64_t)t * r * r), 256, 0, ctx->stream>>>(s->Lsel, s->Csel, s->Scols, lds, s->sel,
+                                                                                               t - 1, q, r, s->Kss, ldk);
       fib::build_kernel<<<fib::flat_grid(ctx, (int64_t)np * np), 256, 0, ctx->stream>>>(s->Kss, ldk, m, np, alpha, s->M);
       ctx->launches += 2;
       NNAL_TRY(nnal_gj64_invert(ctx, s->M, np));
-      fib::z_kernel<<<fib::flat_grid(ctx, (int64_t)m * t * c), 256, 0, ctx->stream>>>(s->M, np, s->Lsel, t, c, r, s->Z, ldz);
+      fib::z_kernel<<<fib::flat_grid(ctx, (int64_t)m * t * q), 256, 0, ctx->stream>>>(s->M, np, s->Lsel, t, q, r, s->Z, ldz);
       fib::trace_kernel<<<1, 256, 0, ctx->stream>>>(s->M, np, m, s->trC);
       ctx->launches += 2;
       prof_end(ctx);
@@ -803,8 +999,9 @@ extern "C" int nnal_fi_block_greedy(nnal_ctx* ctx, int64_t k, double delta, int6
     prof_begin(ctx, NNAL_PROF_FIB_EVAL);
     ea.t = t;
     ea.alpha = alpha;
-    if (s->nl == 2) fib::eval_kernel<2><<<nblk, fib::EVAL_THREADS, smem, ctx->stream>>>(ea);
-    else fib::eval_kernel<1><<<nblk, fib::EVAL_THREADS, smem, ctx->stream>>>(ea);
+    if (s->nl == 2) fib::eval_kernel<2, true><<<nblk, fib::EVAL_THREADS, smem, ctx->stream>>>(ea);
+    else if (q == c) fib::eval_kernel<1, true><<<nblk, fib::EVAL_THREADS, smem, ctx->stream>>>(ea);
+    else fib::eval_kernel<1, false><<<nblk, fib::EVAL_THREADS, smem, ctx->stream>>>(ea);
     ctx->launches++;
     prof_end(ctx);
     if (t + 1 < (int)k) {

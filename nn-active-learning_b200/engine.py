@@ -576,6 +576,44 @@ class Engine(object):
                                                         None if A_prev is None else _ptr(w_last)))
         self._fi_block_n = n
 
+    def fi_block_set_candidates_cls(self, cand, r):
+        """One-layer block-form FI candidates from the current pool pass (as ``fi_block_set_candidates``), each keeping its
+        ``min(r, c)`` most probable classes, 2 <= r <= 32, renormalised (include/nnal_b200.h); any class count."""
+        if cand is None:
+            self._chk(self.lib.nnal_fi_block_set_candidates_cls(self.h, None, 0, int(r)))
+            self._fi_block_n = self._pool_n
+        else:
+            cand = np.ascontiguousarray(cand, dtype=np.int64).ravel()
+            self.h2d_bytes += cand.nbytes
+            self._chk(self.lib.nnal_fi_block_set_candidates_cls(self.h, _ptr(cand) if cand.size else None, cand.size, int(r)))
+            self._fi_block_n = cand.size
+
+    def fi_block_set_factors_cls(self, cls, p, U, c):
+        """One-layer block-form FI candidates from host factors in kept-class form: ``cls`` [n,r] class ids (strictly
+        ascending per row, < ``c``), ``p`` [n,r] their posteriors, ``U`` [n,d] features."""
+        cls = np.ascontiguousarray(cls, dtype=np.int32)
+        p = np.ascontiguousarray(p, dtype=np.float32)
+        U = np.ascontiguousarray(U, dtype=np.float32)
+        if cls.ndim != 2 or p.shape != cls.shape or U.ndim != 2 or U.shape[0] != cls.shape[0]:
+            raise ValueError('cls and p must be [n,r] and U [n,d] for the same n')
+        n, r = cls.shape
+        self.h2d_bytes += cls.nbytes + p.nbytes + U.nbytes
+        self._chk(self.lib.nnal_fi_block_set_factors_cls(self.h, n, int(c), r, U.shape[1], _ptr(cls), _ptr(p), _ptr(U)))
+        self._fi_block_n = n
+
+    def pool_top_classes(self, rows, r):
+        """The ``min(r, c)`` most probable classes of pool rows ``rows`` of the current pool pass (ties: lower class), as
+        the class-capped block FI keeps them: (ids [n,q] int32 ascending, posteriors [n,q] float32)."""
+        rows = np.ascontiguousarray(rows, dtype=np.int64).ravel()
+        q = min(int(r), self.n_class)
+        cls = np.empty((rows.size, q), dtype=np.int32)
+        p = np.empty((rows.size, q), dtype=np.float32)
+        self.h2d_bytes += rows.nbytes
+        self.d2h_bytes += cls.nbytes + p.nbytes
+        self._chk(self.lib.nnal_pool_top_classes(self.h, _ptr(rows) if rows.size else None, rows.size, int(r), _ptr(cls),
+                                                 _ptr(p)))
+        return cls, p
+
     def fi_block_greedy(self, k, delta):
         """Block-form greedy FI selection.  Returns (candidate indices in selection order, objective per step, reduced
         objective ``tr((delta I + K_SS/s)^-1)`` per step)."""

@@ -595,18 +595,22 @@ def query_whole(model, expr, pool_inds, session):
 def query_whole_block(model, expr, pool_inds, session, return_objective=False):
     """``NNAL.CNN_query(..., 'fi')`` with ``expr.pars['fi_mode'] = 'block-greedy'``: greedy minimisation of the FI
     objective ``tr((sum_{i in S} F_i/|S| + delta I)^-1)`` for 2 <= c <= 32 classes (k (c-1) <= 4096; with more classes the
-    library raises NNAL_ERR_UNSUPPORTED after the pool pass, before it allocates the block system) in
-    the block form of csrc/fi_block.cu.  ``expr.pars['fi_layers']`` (default 1) picks the parameters: 1 = the last FC
+    library raises NNAL_ERR_UNSUPPORTED after the pool pass, before it allocates the block system, unless ``fi_classes`` is
+    set) in the block form of csrc/fi_block.cu.  ``expr.pars['fi_layers']`` (default 1) picks the parameters: 1 = the last FC
     layer, ``F_i = (diag pi_i - pi_i pi_i^T) (x) [u_i;1][u_i;1]^T`` (NN.LLFC_hess, NN.py:891-901); 2 = the last two FC
     layers, as the binary path's default, adding the score ``(M_i W3^T (e_y - pi_i)) (x) [a_i;1]`` of the previous FC
     layer (M_i = diag 1[u_i > 0], a_i its input).  Entropy pre-filter to B exactly as ``query_whole``, then the greedy
     over ``min(k, B)`` steps.  Keys read: ``k``, ``B``, ``fi_diag_load`` (default 1e-5), ``fi_layers`` (1 or 2; anything
-    else raises ValueError).  Returns positions into ``pool_inds`` in selection order (and, with ``return_objective``,
-    the objective and its kernel-dependent part per step).
+    else raises ValueError), ``fi_classes`` (optional, one layer only: an integer 2 <= r <= 32; every candidate keeps its
+    min(r, c) most probable classes, ties to the lower class, renormalised in float64, as the reference's multi-class
+    A-matrices keep at most ten (NNAL.py:379-400); the greedy then runs for any c with k (min(r, c) - 1) <= 4096, and with
+    r >= c it is the uncapped greedy bit for bit).  Returns positions into ``pool_inds`` in selection order (and, with
+    ``return_objective``, the objective and its kernel-dependent part per step).
 
     Several ranks: every rank reads its own candidates' posteriors and feature rows (and, for two layers, the previous FC
     output), the B candidates are all-gathered and put in pre-filter order on every rank, and every rank runs the same
-    deterministic greedy on them."""
+    deterministic greedy on them.  With ``fi_classes`` each rank selects its own candidates' kept classes on the device and
+    the ranks exchange ids and posteriors of the kept classes only."""
     from .NNAL import _posteriors_on_device
     k, B = int(expr.pars['k']), int(expr.pars['B'])
     delta = float(expr.pars.get('fi_diag_load', 1e-5))
@@ -614,6 +618,13 @@ def query_whole_block(model, expr, pool_inds, session, return_objective=False):
     if nl not in (1, 2):
         raise ValueError("fi_layers must be 1 or 2 for fi_mode='block-greedy', got %r" % (nl,))
     nl = int(nl)
+    cap = expr.pars.get('fi_classes')
+    if cap is not None:
+        if isinstance(cap, (bool, np.bool_)) or not isinstance(cap, (int, np.integer)) or not 2 <= cap <= 32:
+            raise ValueError('fi_classes must be an integer from 2 to 32, got %r' % (cap,))
+        if nl == 2:
+            raise ValueError('fi_classes covers the last FC layer only (fi_layers = 1)')
+        cap = int(cap)
     pool_inds = np.asarray(pool_inds)
     n = len(pool_inds)
     eng, lo, hi = _posteriors_on_device(model, expr, pool_inds, session, keep=nl)
@@ -623,7 +634,9 @@ def query_whole_block(model, expr, pool_inds, session, return_objective=False):
     else:
         sel_inds = np.arange(n, dtype=np.int64)
     if not dist.is_dist():
-        if nl == 1:
+        if cap is not None:
+            eng.fi_block_set_candidates_cls(sel_inds - lo, cap)
+        elif nl == 1:
             eng.fi_block_set_candidates(sel_inds - lo)
         else:
             eng.fi_block_set_candidates(sel_inds - lo, nl)
@@ -631,22 +644,28 @@ def query_whole_block(model, expr, pool_inds, session, return_objective=False):
         own = (sel_inds >= lo) & (sel_inds < hi)
         rows = sel_inds[own] - lo
         c = eng.n_class
-        post = eng.pool_posteriors()[:, rows] if len(rows) else np.zeros((c, 0), dtype=np.float32)
         F = eng.pool_feature_rows(rows)
         d = F.shape[1]
         gpos = dist.allgather_concat(sel_inds[own].astype(np.int64))
-        P = dist.allgather_concat(np.ascontiguousarray(post.T, dtype=np.float32).ravel()).reshape(-1, c)
         Fg = dist.allgather_concat(np.ascontiguousarray(F, dtype=np.float32).ravel()).reshape(-1, d)
         order = np.argsort(gpos, kind='stable')
         perm = order[np.searchsorted(gpos[order], sel_inds)]          # gathered row of every candidate, pre-filter order
-        if nl == 1:
-            eng.fi_block_set_factors(P[perm].T, Fg[perm])
+        if cap is not None:
+            cls, p = eng.pool_top_classes(rows, cap)
+            Cg = dist.allgather_concat(cls.ravel()).reshape(-1, cls.shape[1])
+            Pg = dist.allgather_concat(p.ravel()).reshape(-1, cls.shape[1])
+            eng.fi_block_set_factors_cls(Cg[perm], Pg[perm], Fg[perm], c)
         else:
-            A = eng.pool_prev_rows(rows)
-            Ag = dist.allgather_concat(np.ascontiguousarray(A, dtype=np.float32).ravel()).reshape(-1, A.shape[1])
-            layers = list(model.layer_dict.items()) if isinstance(model.layer_dict, dict) else list(model.layer_dict)
-            W3 = np.asarray(model.get_weights(session)[layers[-1][0]][0], dtype=np.float32)     # [c, d]
-            eng.fi_block_set_factors(P[perm].T, Fg[perm], Ag[perm], W3)
+            post = eng.pool_posteriors()[:, rows] if len(rows) else np.zeros((c, 0), dtype=np.float32)
+            P = dist.allgather_concat(np.ascontiguousarray(post.T, dtype=np.float32).ravel()).reshape(-1, c)
+            if nl == 1:
+                eng.fi_block_set_factors(P[perm].T, Fg[perm])
+            else:
+                A = eng.pool_prev_rows(rows)
+                Ag = dist.allgather_concat(np.ascontiguousarray(A, dtype=np.float32).ravel()).reshape(-1, A.shape[1])
+                layers = list(model.layer_dict.items()) if isinstance(model.layer_dict, dict) else list(model.layer_dict)
+                W3 = np.asarray(model.get_weights(session)[layers[-1][0]][0], dtype=np.float32)     # [c, d]
+                eng.fi_block_set_factors(P[perm].T, Fg[perm], Ag[perm], W3)
     chosen, obj, red = eng.fi_block_greedy(min(k, len(sel_inds)), delta)
     q = sel_inds[chosen]
     if return_objective == 'reduced':
